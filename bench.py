@@ -2,7 +2,7 @@
 """bench.py — captions/sec of the role-shift decoder's beam search on synthetic COCO-Entities-shaped
 batches (BASELINE.json metric), on N GPUs of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is ONE full beam-search decode of one 100-caption batch: the once-per-batch prologue, the 20 decoder
@@ -21,6 +21,10 @@ What the keys of the JSON line measure (all on the same K timed steps, after W >
   e2e             host buffers -> H2D -> beam_search_v -> D2H -> host read through vsrdec.DecodePipeline (same stacking
                   and lanes), every copy inside the timed region
   parity_check    one timed-workload decode verified against the CPU oracle inside this run (see parity_check())
+
+`--dump-outputs DIR` writes what the headline's last timed decode call returned for its last batch (timed step K):
+words.npy and gates.npy (ids as float64), log_probs_words.npy and log_probs_gates.npy (float32), each (100, T).
+Weights and inputs come from fixed seeds, so two builds run with the same arguments can be compared output for output.
 
 `--impl reference` times the CPU port of the reference's algorithm (oracle/vsr_oracle.py, torch CPU
 ops, all host threads) on the SAME workload (100 captions per step); the reference itself is Python and is not
@@ -239,6 +243,17 @@ def bind_to_gpu_cpus(gpu_index):
         return "unavailable: " + repr(e)[:80]
 
 
+def dump_outputs(out_dir, outputs):
+    """Writes what beam_search_v returned for one batch, (words, gates, lp_words, lp_gates) each (b, T), as
+    <out_dir>/<name>.npy: token and gate ids as float64, log-probabilities as float32."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in zip(("words", "gates", "log_probs_words", "log_probs_gates"), outputs):
+        t = t.detach().cpu()
+        t = t.float() if t.is_floating_point() else t.double()
+        np.save(os.path.join(out_dir, name + ".npy"), t.numpy())
+
+
 def main_ours(args, rank, world, local_rank):
     import torch.distributed as dist
     from models import ControllableCaptioningModel
@@ -340,6 +355,7 @@ def main_ours(args, rank, world, local_rank):
                 statics = tuple(t[:n * b] for t in sset)
                 (words, gates), (lpw, lpg) = lane_models[ln].beam_search_v(statics, w["eos"], w["beam"], 1, gt=w["gt"])
                 last["words"], last["set"], last["n"] = gather(words), (ln + n_lanes * (gi // n_lanes)) % len(dev_stacked), n
+                last["outputs"] = (words, gates, lpw, lpg)
         for ln in lanes:
             ev = torch.cuda.Event()
             ev.record(ln)
@@ -597,6 +613,9 @@ def main_ours(args, rank, world, local_rank):
             line["parity_check"]["ok"] = line["parity_check"]["ok"] and ok
         dist.barrier()
     if rank == 0:
+        if args.dump_outputs:
+            # the last timed step is the last 100-caption batch of the last timed decode call
+            dump_outputs(args.dump_outputs, [t[-b:] for t in last["outputs"]])
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -614,7 +633,11 @@ def main():
     ap.add_argument("--idx-stack", type=int, default=5, help="batches per decode call of the index-form e2e loop")
     ap.add_argument("--e2e-stack", type=int, default=1, help="batches per decode call of the e2e loop (materialised inputs)")
     ap.add_argument("--lanes", type=int, default=2, help="decode calls in flight per GPU (engines on their own streams)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the run, write the outputs of the last timed step "
+                    "(the words, gates and log-probs the headline's decode call returned for its last batch) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -50,8 +50,15 @@ def synth_seq(b: int = 6, N: int = 10, seed: int = 77) -> torch.Tensor:
 
 
 def checksum(t: torch.Tensor) -> float:
+    """sum_i t_i * ((i + 1) mod 97) in float64, summed pairwise with elementwise adds.  Each add is one IEEE rounding, so
+    the value is the same on every host; torch.sum's order, and with it the last bits, depends on the CPU's vector width."""
     t = t.double().flatten()
-    return float((t * torch.arange(1, t.numel() + 1, dtype=torch.float64).remainder(97.0)).sum())
+    x = t * torch.arange(1, t.numel() + 1, dtype=torch.float64).remainder(97.0)
+    while x.numel() > 1:
+        if x.numel() % 2:
+            x = torch.cat([x, x.new_zeros(1)])
+        x = x[0::2] + x[1::2]
+    return float(x.sum())
 
 
 def logits(W, seq: torch.Tensor) -> torch.Tensor:

@@ -4,6 +4,7 @@ import os
 import torch
 
 from oracle import vsr_oracle as O
+from oracle.ssp_oracle import checksum  # noqa: F401  (the golden fixtures' checksum)
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
@@ -20,11 +21,6 @@ def load_golden(name):
             ctrl[:, t] = ds[:, min(t // 2, L - 1)]
         fx["ctrl"] = ctrl
     return fx
-
-
-def checksum(t: torch.Tensor) -> float:
-    t = t.double().flatten()
-    return float((t * torch.arange(1, t.numel() + 1, dtype=torch.float64).remainder(97.0)).sum())
 
 
 def rel_close(a, b, rel=1e-3, abs_floor=1e-4):

@@ -1,8 +1,8 @@
-"""Generate golden vectors from the UNMODIFIED reference (build container only).
+"""Generate golden vectors from the UNMODIFIED reference (a checkout of the original project).
 
-    python tests/golden/make_golden.py
+    VSR_REFERENCE_ROOT=<checkout> python tests/golden/make_golden.py
 
-Imports /root/reference/models, runs the reference's own ``beam_search_v`` /
+Imports $VSR_REFERENCE_ROOT/models, runs the reference's own ``beam_search_v`` /
 ``beam_search`` / ``forward`` / ``test`` / ``step_v`` on seeded synthetic inputs and
 stores inputs + outputs as small ``.pt`` fixtures beside this script:
 
@@ -27,11 +27,7 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 import refload  # noqa: E402
 from oracle import vsr_oracle as O  # noqa: E402
-
-
-def checksum(t: torch.Tensor) -> float:
-    t = t.double().flatten()
-    return float((t * torch.arange(1, t.numel() + 1, dtype=torch.float64).remainder(97.0)).sum())
+from oracle.ssp_oracle import checksum  # noqa: E402
 
 
 def run_small(path, dims: O.Dims, seed_w, seed_x):
@@ -104,7 +100,7 @@ def run_full_cfg1(path):
 
 
 if __name__ == "__main__":
-    assert refload.available(), "needs /root/reference"
+    assert refload.available(), "set VSR_REFERENCE_ROOT to a checkout of the original project"
     small = dict(seq_len=20, vocab_size=157, bos_idx=2, det_feat_size=96, input_encoding_size=36,
                  rnn_size=50, att_size=20)
     run_small(os.path.join(HERE, "small_a.pt"), O.Dims(**small), seed_w=1234, seed_x=1001)

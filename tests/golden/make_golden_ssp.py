@@ -41,9 +41,14 @@ def main():
         la = rnd.sample(pool, rnd.randint(1, n))
         lb = rnd.sample(pool, rnd.randint(1, n))
         merges.append((list(la), list(lb), tools.verb_rank_merge(list(la), list(lb))))
+    # the oracle's matrix for a second input, computed where these vectors are made: a test host that reproduces it
+    # bit for bit rounds float32 like this one (tests/test_oracle_ssp.py then demands the reference's matrix bit for bit)
+    with torch.no_grad():
+        probe = {"seed_x": 78, "matrix": S.forward(S.init_weights(10, 1234), S.synth_seq(6, 10, 78))}
     # weights and inputs are reproducible from their seeds (oracle: init_weights / synth_seq): only checksums are stored
     torch.save({"weight_checksums": {k: S.checksum(v) for k, v in net.state_dict().items()}, "seq_checksum": S.checksum(seq),
-                "matrix": out, "seed_w": 1234, "seed_x": 77, "merges": merges}, os.path.join(HERE, "ssp_small.pt"))
+                "matrix": out, "seed_w": 1234, "seed_x": 77, "merges": merges, "probe": probe},
+               os.path.join(HERE, "ssp_small.pt"))
     print("wrote ssp_small.pt", tuple(out.shape), len(merges), "merges")
 
 

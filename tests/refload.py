@@ -1,9 +1,10 @@
-"""Import the UNMODIFIED reference model from /root/reference (build container only).
+"""Import the UNMODIFIED reference model from the checkout of the original project that
+VSR_REFERENCE_ROOT names.  The original is not part of this repository: without that variable
+``available()`` is False and its callers skip (the stored golden vectors keep the comparison).
 
 The reference constructor opens four JSON files relative to the CWD
 (models/controllable_captioning.py:25-34), so it is constructed from a temp
-directory holding those fixture files.  Never used at GPU-box run time:
-/root/reference does not exist there (callers must check ``available()``).
+directory holding those fixture files.
 """
 import contextlib
 import importlib
@@ -12,11 +13,11 @@ import os
 import sys
 import tempfile
 
-REFERENCE_ROOT = os.environ.get("VSR_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("VSR_REFERENCE_ROOT", "")
 
 
 def available() -> bool:
-    return os.path.isfile(os.path.join(REFERENCE_ROOT, "models", "controllable_captioning.py"))
+    return bool(REFERENCE_ROOT) and os.path.isfile(os.path.join(REFERENCE_ROOT, "models", "controllable_captioning.py"))
 
 
 @contextlib.contextmanager

@@ -17,7 +17,14 @@ def test_sinkhorn_oracle_matches_reference_golden():
     assert S.checksum(seq) == fx["seq_checksum"]
     with torch.no_grad():
         out = S.forward(W, seq)
-    assert torch.equal(out, fx["matrix"])                   # bit for bit
+        probe = S.forward(W, S.synth_seq(6, 10, fx["probe"]["seed_x"]))
+    if torch.equal(probe, fx["probe"]["matrix"]):
+        # this host's float32 CPU kernels round like those of the host that made the golden vectors
+        assert torch.equal(out, fx["matrix"])               # bit for bit
+    else:
+        # other BLAS / vector-width paths reorder the sums; exp(x / 0.1) and 20 normalisation rounds amplify that to
+        # ~110 ulps (1.3e-5 relative) at most over the code paths measured
+        assert torch.allclose(out, fx["matrix"], rtol=5e-5, atol=0)
     # the matrix is (nearly) doubly stochastic and its optimal assignment is a permutation
     assert torch.allclose(out.sum(-1), torch.ones(6, 10), atol=1e-4)
     for i in range(6):

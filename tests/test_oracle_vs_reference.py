@@ -1,12 +1,14 @@
-"""Live check of the oracle against the UNMODIFIED reference (only where /root/reference exists,
-i.e. in the build container; skipped on the GPU box)."""
+"""Live check of the oracle against the UNMODIFIED reference (only where VSR_REFERENCE_ROOT names a
+checkout of the original project; skipped elsewhere).  test_oracle_golden.py keeps the comparison
+against vectors the reference produced, without it."""
 import pytest
 import torch
 
 import refload
 from oracle import vsr_oracle as O
 
-pytestmark = pytest.mark.skipif(not refload.available(), reason="/root/reference not present")
+pytestmark = pytest.mark.skipif(not refload.available(),
+                                reason="the original project is not present (set VSR_REFERENCE_ROOT to its checkout)")
 
 
 @pytest.mark.parametrize("flags", [(True, False), (False, False), (True, True)])

@@ -178,6 +178,25 @@ int vsr_greedy(vsr_handle h, int64_t* out_words, int64_t* out_gates, void* strea
 int vsr_sample(vsr_handle h, uint64_t seed, int64_t* out_words, int64_t* out_gates,
                float* lp_words, float* lp_gates, void* stream);
 
+/* Attention capture: where the decoder looks for every generated word.
+ * vsr_set_attention_capture: while enabled, the decode drivers (vsr_beam_search, vsr_greedy, vsr_sample,
+ *   vsr_forward_teacher) record, at every step and for every row, the R+1 attention weights of the slot attention
+ *   (controllable_captioning.py:167-169) and the slot the row read, in a grow-only workspace of [T][rows][R+1] fp32 +
+ *   [T][rows] int32 (8.4 MB at 1000 captions x beam 5 x R = 20).  Off by default; when off nothing is recorded and no
+ *   launch or output changes.  Captured decodes replay from their own CUDA graphs.
+ * vsr_get_attention: the attention of the last decode on the handle, enqueued on `stream` (no host synchronisation).
+ *   vsr_beam_search:  alpha (b,out_size,T,R+1) fp32, slot (b,out_size,T) int32, following the back-pointer path of each
+ *                     returned beam (the row whose distributions produced token t).  Note that lp_words / lp_gates are
+ *                     NOT back-tracked (slot order, as in the reference), the attention is.
+ *   other drivers:    alpha (b,T,R+1), slot (b,T): one row per caption (T = the captions' length for teacher forcing).
+ *   alpha[..., 0] is the sentinel weight and alpha[..., r+1] the weight of region r of the slot read at that step; the
+ *   weights are exactly the ones that form the attended feature: 0 at padding regions and at an all-zero sentinel, the
+ *   rest sums to 1.  Verb forcing does not change them.  After a caption's EOS the frozen beam keeps decoding and its
+ *   weights are returned as computed, not masked.  R is the prologue's R at decode time.
+ *   Returns VSR_ESTATE when the last decode ran without capture (or none has run). */
+int vsr_set_attention_capture(vsr_handle h, int32_t enabled);
+int vsr_get_attention(vsr_handle h, float* alpha, int32_t* slot, void* stream);
+
 /* Number of kernels this handle has launched so far (bench.py's gpu_launches). */
 int64_t vsr_launch_count(vsr_handle h);
 

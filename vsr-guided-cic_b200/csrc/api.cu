@@ -181,6 +181,43 @@ int ensure_beam_ws(Ctx* c, int caps, int T) {
   return VSR_OK;
 }
 
+// grow-only capture buffers for a decode of T steps with up to step_rows rows per step (and a back-tracked path of
+// path entries); clears what the previous decode left.  Nothing is allocated while capture is off.
+static int attn_begin(Ctx* c, int64_t step_rows, int T, size_t path) {
+  c->attn_ready = false;
+  if (!c->attn_capture) return VSR_OK;
+  const size_t n_slot = (size_t)step_rows * T, n_alpha = n_slot * (c->R + 1);
+  if (n_alpha > c->cap_attn_alpha) {
+    dev_free(c, c->attn_alpha); c->attn_alpha = nullptr; c->cap_attn_alpha = 0;
+    ALLOC_F(c->attn_alpha, n_alpha);
+    c->cap_attn_alpha = n_alpha;
+  }
+  if (n_slot > c->cap_attn_slot) {
+    dev_free(c, c->attn_slot); c->attn_slot = nullptr; c->cap_attn_slot = 0;
+    VSR_TRY(dev_alloc(c, (void**)&c->attn_slot, sizeof(int32_t) * n_slot));
+    c->cap_attn_slot = n_slot;
+  }
+  if (path > c->cap_attn_path) {
+    dev_free(c, c->attn_path); c->attn_path = nullptr; c->cap_attn_path = 0;
+    VSR_TRY(dev_alloc(c, (void**)&c->attn_path, sizeof(int32_t) * path));
+    c->cap_attn_path = path;
+  }
+  return VSR_OK;
+}
+
+// capture outputs of step t: rows of step t start at t * step_rows (null pointers when capture is off)
+static void attn_step_io(const Ctx* c, StepIO& io, int t, int64_t step_rows) {
+  if (!c->attn_capture) return;
+  io.attn_alpha = c->attn_alpha + (size_t)t * step_rows * (c->R + 1);
+  io.attn_slot = c->attn_slot + (size_t)t * step_rows;
+}
+
+// after a successful decode: what vsr_get_attention returns (n_out rows per step, back-tracked when beam)
+static void attn_done(Ctx* c, bool beam, int T, int n_out, int64_t step_rows) {
+  c->attn_ready = c->attn_capture;
+  c->attn_beam = beam; c->attn_T = T; c->attn_R = c->R; c->attn_n_out = n_out; c->attn_step_rows = step_rows;
+}
+
 static int create_impl(const VsrDims* d, const float* const* w, Ctx** out) {
   VSR_REQUIRE(d != nullptr && w != nullptr && out != nullptr, VSR_EINVAL, "vsr_create: null argument");
   VSR_REQUIRE(d->vocab_size > 0 && d->rnn_size > 0 && d->att_size > 0 && d->input_encoding_size > 0 &&
@@ -484,6 +521,7 @@ static int enqueue_beam_steps(Ctx* c, int k, const int64_t* eos, int use_verbs, 
     io.zero_state = t == 0 && c->zero_state_opt;
     if (tr && tr->step_out) { io.out_logp = tr->step_out + (size_t)t * b * k * c->V; io.out_stride = c->V; }
     if (tr && tr->step_gate) { io.gate_out = tr->step_gate + (size_t)t * b * k * 2; io.gate_stride = 2; }
+    attn_step_io(c, io, t, (int64_t)b * k);
     VSR_TRY(run_step(c, io, st));
     const size_t fo = (size_t)t * b * k;
     VSR_TRY(launch_beam_step(c, t, b, cur, k, eos[0], eos[1], have_forced ? tr->forced_beam + fo : nullptr,
@@ -501,7 +539,7 @@ static int enqueue_beam_steps(Ctx* c, int k, const int64_t* eos, int use_verbs, 
 static int beam_steps_graphed(Ctx* c, int k, const int64_t* eos, int use_verbs, int gt, cudaStream_t st) {
   Ctx::GraphKey key = graph_key(c, 0);
   key.eos0 = eos[0]; key.eos1 = eos[1];
-  key.k = k; key.use_verbs = use_verbs; key.gt = gt; key.T = c->d.seq_len;
+  key.k = k; key.use_verbs = use_verbs; key.gt = gt; key.T = c->d.seq_len; key.attn = c->attn_capture;
   return run_graphed(c, key, st, [&](cudaStream_t s) { return enqueue_beam_steps(c, k, eos, use_verbs, gt, nullptr, s); });
 }
 
@@ -520,13 +558,16 @@ static int beam_search_impl(Ctx* c, int k, int out_size, const int64_t* eos, int
   const int b = c->b, T = c->d.seq_len;
   VSR_TRY(ensure_rows(c, b * k));
   VSR_TRY(ensure_beam_ws(c, b, T));
+  VSR_TRY(attn_begin(c, (int64_t)b * k, T, (size_t)b * out_size * T));
   c->hist_T = T; c->hist_b = b; c->hist_k = k;
   // graph replay unless a trace is requested, the phase profiler is on, or the caller is capturing itself
   if (tr == nullptr && graphs_usable(c, st))
     VSR_TRY(beam_steps_graphed(c, k, eos, use_verbs, gt, st));
   else
     VSR_TRY(enqueue_beam_steps(c, k, eos, use_verbs, gt, tr, st));
-  VSR_TRY(launch_backtrack(c, b, k, T, out_size, out_words, out_gates, lp_words, lp_gates, st));
+  VSR_TRY(launch_backtrack(c, b, k, T, out_size, out_words, out_gates, lp_words, lp_gates,
+                           c->attn_capture ? c->attn_path : nullptr, st));
+  attn_done(c, true, T, b * out_size, (int64_t)b * k);
   return VSR_OK;
 }
 
@@ -558,6 +599,7 @@ static int enqueue_forward_steps(Ctx* c, const int64_t* captions, int T, bool ba
     StepIO io{};
     io.rows = b; io.cur_beam = 1; io.use_verbs = false; io.gt = false; io.topk = 0;
     io.zero_state = t == 0 && c->zero_state_opt;
+    attn_step_io(c, io, t, b);
     if (batched) {
       io.skip_vocab = true;
       VSR_TRY(run_step(c, io, st));
@@ -580,12 +622,17 @@ static int forward_impl(Ctx* c, const int64_t* captions, int T, float* out, floa
   VSR_REQUIRE(T >= 1 && T <= c->L, VSR_EINVAL, "vsr_forward_teacher: T=%d exceeds the prologue's slot count L=%d", T, c->L);
   const int b = c->b;
   VSR_TRY(ensure_rows(c, b));
+  VSR_TRY(attn_begin(c, b, T, 0));
   const bool batched = c->use_tc;        // (the FFMA twin keeps the plain per-step unroll)
-  if (!batched) return enqueue_forward_steps(c, captions, T, false, out, gate, st);
+  if (!batched) {
+    VSR_TRY(enqueue_forward_steps(c, captions, T, false, out, gate, st));
+    attn_done(c, false, T, b, b);
+    return VSR_OK;
+  }
   VSR_TRY(ensure_fwd_ws(c, b * T));
   if (graphs_usable(c, st)) {            // the loop + the batched vocabulary GEMM replay from the graph cache (kind 2)
     Ctx::GraphKey key = graph_key(c, 2);
-    key.captions = captions; key.T = T;
+    key.captions = captions; key.T = T; key.attn = c->attn_capture;
     VSR_TRY(run_graphed(c, key, st, [&](cudaStream_t s) { return enqueue_forward_steps(c, captions, T, true, nullptr, nullptr, s); }));
   } else {
     VSR_TRY(enqueue_forward_steps(c, captions, T, true, nullptr, nullptr, st));
@@ -593,6 +640,7 @@ static int forward_impl(Ctx* c, const int64_t* captions, int T, float* out, floa
   // caller-owned outputs are written outside the graph: log-softmax of the b*T vocabulary rows, and the gate rows
   VSR_TRY(run_vocab_rows(c, c->h2all_b, c->logits_all, b * T, out, st, true));
   VSR_CHECK_CUDA(cudaMemcpyAsync(gate, c->gate_all, sizeof(float) * (size_t)b * T * 2, cudaMemcpyDeviceToDevice, st));
+  attn_done(c, false, T, b, b);
   return VSR_OK;
 }
 
@@ -602,15 +650,18 @@ static int greedy_impl(Ctx* c, int64_t* out_words, int64_t* out_gates, cudaStrea
   const int b = c->b, T = c->d.seq_len;
   VSR_TRY(ensure_rows(c, b));
   VSR_TRY(ensure_beam_ws(c, b, T));
+  VSR_TRY(attn_begin(c, b, T, 0));
   VSR_TRY(launch_state_init(c, b, st));
   for (int t = 0; t < T; ++t) {
     StepIO io{};
     io.rows = b; io.cur_beam = 1; io.use_verbs = false; io.gt = false; io.topk = 1;
     io.zero_state = t == 0 && c->zero_state_opt;
+    attn_step_io(c, io, t, b);
     VSR_TRY(run_step(c, io, st));
     VSR_TRY(launch_greedy_pick(c, b, t, T, out_words, out_gates, st));
     if (t + 1 < T) VSR_TRY(launch_commit_identity(c, b, nullptr, 0, -1, st));
   }
+  attn_done(c, false, T, b, b);
   return VSR_OK;
 }
 
@@ -622,15 +673,18 @@ static int sample_impl(Ctx* c, uint64_t seed, int64_t* out_words, int64_t* out_g
   const int b = c->b, T = c->d.seq_len;
   VSR_TRY(ensure_rows(c, b));
   VSR_TRY(ensure_beam_ws(c, b, T));
+  VSR_TRY(attn_begin(c, b, T, 0));
   VSR_TRY(launch_state_init(c, b, st));
   for (int t = 0; t < T; ++t) {
     StepIO io{};
     io.rows = b; io.cur_beam = 1; io.use_verbs = false; io.gt = false; io.topk = 0;     // statistics + gate head only
     io.zero_state = t == 0 && c->zero_state_opt;
+    attn_step_io(c, io, t, b);
     VSR_TRY(run_step(c, io, st));
     VSR_TRY(launch_sample_pick(c, b, t, T, seed, out_words, out_gates, lp_words, lp_gates, st));
     if (t + 1 < T) VSR_TRY(launch_commit_identity(c, b, nullptr, 0, -1, st));
   }
+  attn_done(c, false, T, b, b);
   return VSR_OK;
 }
 
@@ -759,6 +813,23 @@ int vsr_get_history(vsr_handle h, int32_t* parent, int32_t* word, int32_t* gate,
   if (gate) VSR_CHECK_CUDA(cudaMemcpyAsync(gate, c->hist_gate, n * 4, cudaMemcpyDeviceToDevice, st));
   if (score) VSR_CHECK_CUDA(cudaMemcpyAsync(score, c->hist_score, n * 4, cudaMemcpyDeviceToDevice, st));
   return VSR_OK;
+}
+
+int vsr_set_attention_capture(vsr_handle h, int32_t enabled) {
+  if (!h) { vsr::set_error("vsr_set_attention_capture: null handle"); return VSR_EINVAL; }
+  ((Ctx*)h)->attn_capture = enabled != 0;
+  return VSR_OK;
+}
+
+int vsr_get_attention(vsr_handle h, float* alpha, int32_t* slot, void* stream) {
+  if (!h) { vsr::set_error("vsr_get_attention: null handle"); return VSR_EINVAL; }
+  DeviceGuard dg((const vsr::Ctx*)h);
+  Ctx* c = (Ctx*)h;
+  VSR_REQUIRE(c->attn_ready, VSR_ESTATE,
+              "vsr_get_attention: the last decode on this handle ran without attention capture (vsr_set_attention_capture)");
+  VSR_REQUIRE(alpha && slot, VSR_EINVAL, "vsr_get_attention: null argument");
+  return vsr::launch_attn_gather(c, c->attn_beam ? c->attn_path : nullptr, c->attn_n_out, c->attn_T, alpha, slot,
+                                 (cudaStream_t)stream);
 }
 
 int vsr_forward_teacher(vsr_handle h, const int64_t* captions, int32_t T, float* out, float* gate, void* stream) {

@@ -312,10 +312,12 @@ __global__ void __launch_bounds__(256) k_sample_pick(const float* __restrict__ l
 // final ordering of the beams by accumulated score (stable, descending) and unroll of the
 // back-pointers (CaptioningModel.py:182-194 / 279-293).  One CTA per caption: the caption's [T][k] history is
 // staged in shared memory with coalesced loads, so the serial pointer chase never waits on global memory.
+// path_row (optional, [b][out_size][T]): the step-t row whose distributions produced token t of the returned beam.
 __global__ void __launch_bounds__(64) k_backtrack(int b, int k, int T, int out_size, const float* seq_lp,
                                                   const int32_t* hist_parent, const int32_t* hist_word,
                                                   const int32_t* hist_gate, const float* hist_lpw, const float* hist_lpg,
-                                                  int64_t* out_words, int64_t* out_gates, float* lp_words, float* lp_gates) {
+                                                  int64_t* out_words, int64_t* out_gates, float* lp_words, float* lp_gates,
+                                                  int32_t* path_row) {
   extern __shared__ __align__(16) unsigned char bt_smem[];      // 5 arrays of T*k 4-byte entries (<= 40 KB)
   int32_t* s_par = reinterpret_cast<int32_t*>(bt_smem);
   int32_t* s_wrd = s_par + T * k;
@@ -353,7 +355,25 @@ __global__ void __launch_bounds__(64) k_backtrack(int b, int k, int T, int out_s
     lp_words[ob + t] = s_lpw[t * k + final_slot];
     lp_gates[ob + t] = s_lpg[t * k + final_slot];
     slot = s_par[t * k + slot];
+    // the attention, unlike the log-probs, follows the back-pointers: rows of step t are c * cur_t + parent slot
+    if (path_row != nullptr) path_row[ob + t] = c * (t == 0 ? 1 : k) + slot;
   }
+}
+
+// attention of the returned sequences from the per-step capture: out row i (caption * out_size + beam) at step t reads
+// captured row path_row[i][t] of step t, or row i itself when path_row is null (one row per caption: greedy, sampling,
+// teacher forcing).  One warp per (i, t).
+__global__ void __launch_bounds__(128) k_attn_gather(const float* __restrict__ alpha_ws, const int32_t* __restrict__ slot_ws,
+                                                     int64_t step_rows, const int32_t* __restrict__ path_row, int n_out, int T,
+                                                     int W, float* __restrict__ alpha, int32_t* __restrict__ slot) {
+  const int lane = threadIdx.x & 31;
+  const int item = blockIdx.x * 4 + (threadIdx.x >> 5);
+  if (item >= n_out * T) return;
+  const int i = item / T, t = item - i * T;
+  const int64_t row = path_row != nullptr ? path_row[item] : i;
+  const int64_t src = (int64_t)t * step_rows + row;
+  for (int j = lane; j < W; j += 32) alpha[(size_t)item * W + j] = alpha_ws[(size_t)src * W + j];
+  if (lane == 0) slot[item] = slot_ws[src];
 }
 
 }  // namespace
@@ -464,14 +484,22 @@ int launch_sample_pick(Ctx* c, int rows, int t, int T, uint64_t seed, int64_t* o
 }
 
 int launch_backtrack(Ctx* c, int b, int k, int T, int out_size, int64_t* out_words,
-                     int64_t* out_gates, float* lp_words, float* lp_gates, cudaStream_t st) {
+                     int64_t* out_gates, float* lp_words, float* lp_gates, int32_t* path_row, cudaStream_t st) {
   PhaseScope ps(c, PH_FINAL, st);
   VSR_REQUIRE(T <= VSR_MAX_SEQ_LEN, VSR_EINVAL, "seq_len=%d > %d unsupported by the back-track kernel", T, VSR_MAX_SEQ_LEN);
   // final scores come from the history slice of the last step, NOT from the ping-pong buffer c->seq_lp: a replayed
   // CUDA graph bakes in the ping-pong parity of its capture, which need not be the host's current one (odd seq_len)
   k_backtrack<<<b, 64, (size_t)T * k * 20, st>>>(b, k, T, out_size, c->hist_score + (size_t)(T - 1) * b * k, c->hist_parent, c->hist_word,
                                             c->hist_gate, c->hist_lpw, c->hist_lpg, out_words, out_gates,
-                                            lp_words, lp_gates);
+                                            lp_words, lp_gates, path_row);
+  VSR_CHECK_CUDA(cudaGetLastError()); c->launches++;
+  return VSR_OK;
+}
+
+int launch_attn_gather(Ctx* c, const int32_t* path_row, int n_out, int T, float* alpha, int32_t* slot, cudaStream_t st) {
+  const int items = n_out * T;
+  k_attn_gather<<<(items + 3) / 4, 128, 0, st>>>(c->attn_alpha, c->attn_slot, c->attn_step_rows, path_row, n_out, T,
+                                                 c->attn_R + 1, alpha, slot);
   VSR_CHECK_CUDA(cudaGetLastError()); c->launches++;
   return VSR_OK;
 }

@@ -341,6 +341,15 @@ struct Ctx {
   float *hist_score, *hist_lpw, *hist_lpg;       // [T][caps][beam]
   int hist_T = 0, hist_b = 0, hist_k = 0;
   int64_t* word_in = nullptr;        // [rows] scratch (teacher forcing / step)
+  // attention capture (vsr_set_attention_capture): per step t, rows t * attn_step_rows .. of [R+1] weights and the
+  // slot each row read; attn_path = the back-tracked rows of the returned beams [b][out_size][T]
+  bool attn_capture = false;
+  float* attn_alpha = nullptr; int32_t* attn_slot = nullptr; int32_t* attn_path = nullptr;
+  size_t cap_attn_alpha = 0, cap_attn_slot = 0, cap_attn_path = 0;   // capacities in elements
+  // what the last decode left for vsr_get_attention: captured (attn_ready), shape, and whether rows follow attn_path
+  bool attn_ready = false, attn_beam = false;
+  int attn_T = 0, attn_R = 0, attn_n_out = 0;
+  int64_t attn_step_rows = 0;
   // bookkeeping
   int64_t launches = 0;
   bool profiling = false;
@@ -356,7 +365,7 @@ struct Ctx {
     const void* captions;
     const void *det, *det_seqs, *slot_index, *verbs;
     int64_t det_stride, eos0, eos1;
-    int32_t b, D, L, R, n_img, verbs_dtype, k, use_verbs, gt, T;
+    int32_t b, D, L, R, n_img, verbs_dtype, k, use_verbs, gt, T, attn;
   };
   struct GraphEntry { GraphKey key; cudaGraphExec_t exec; int64_t launches; uint64_t last_use; };
   std::vector<GraphEntry> graphs;
@@ -401,6 +410,8 @@ struct StepIO {
   bool zero_state;   // h1 = h2 = 0 on entry (first step after init_state): their GEMM contributions are skipped
   bool skip_vocab;   // stop after LSTM cell 2 (batched teacher-forced forward: out_fc + log-softmax run once after the loop)
   bool need_h32;     // the caller reads the fp32 h1'/h2' (vsr_step); the tensor-core path itself only needs the fp16 twins
+  float* attn_alpha;    // optional [rows][R+1] attention weights of the step (capture), with ...
+  int32_t* attn_slot;   // ... [rows] the slot each row read; both null when capture is off
 };
 int run_step(Ctx* c, const StepIO& io, cudaStream_t st);
 
@@ -410,7 +421,8 @@ int launch_beam_step(Ctx* c, int t, int b, int cur, int k, int64_t eos0, int64_t
                      const int32_t* f_beam, const int32_t* f_word, const int32_t* f_gate, bool advance,
                      cudaStream_t st);
 int launch_backtrack(Ctx* c, int b, int k, int T, int out_size, int64_t* out_words,
-                     int64_t* out_gates, float* lp_words, float* lp_gates, cudaStream_t st);
+                     int64_t* out_gates, float* lp_words, float* lp_gates, int32_t* path_row, cudaStream_t st);
+int launch_attn_gather(Ctx* c, const int32_t* path_row, int n_out, int T, float* alpha, int32_t* slot, cudaStream_t st);
 int launch_commit_identity(Ctx* c, int rows, const int64_t* next_words, int64_t word_stride,
                            int next_slot, cudaStream_t st);
 int launch_greedy_pick(Ctx* c, int rows, int t, int T, int64_t* out_words, int64_t* out_gates,

@@ -115,6 +115,9 @@ struct AttendArgs {
   float* att; int ld_att;
   PairOut att_b;
   float* shift;            // [rows] sum of the valid region scores = the "shift" gate logit (:187)
+  // attention capture (null = off): the row's R+1 weights after the masked renormalisation, column 0 = sentinel,
+  // column r+1 = region r of the slot it reads ([rows][R+1]), and that slot ([rows])
+  float* alpha_out; int32_t* slot_out;
   int rows, cur_beam, L, R, F, A, H, ldP;
 };
 
@@ -280,9 +283,13 @@ __global__ void __launch_bounds__(ATT_THREADS) k_attend(const AttendArgs a) {
       const float T = warp_sum(w);
       w = w / T;
       const float shift = warp_sum(region ? ev : 0.f);
+      if (a.alpha_out != nullptr && in) a.alpha_out[(size_t)n * (a.R + 1) + lane] = w;
       const unsigned msk = __ballot_sync(0xffffffffu, region);
       if (region) { const int pos = __popc(msk & ((1u << lane) - 1u)); s_rows[pos] = lane - 1; s_w[pos] = w; }
-      if (lane == 0) { e[0] = w; s_nv = __popc(msk); a.shift[n] = shift; }
+      if (lane == 0) {
+        e[0] = w; s_nv = __popc(msk); a.shift[n] = shift;
+        if (a.slot_out != nullptr) a.slot_out[n] = slot;
+      }
     } else if (lane == 0) {
       const float e_pad = s_pad;
       float m = e[0];
@@ -306,6 +313,10 @@ __global__ void __launch_bounds__(ATT_THREADS) k_attend(const AttendArgs a) {
       }
       s_nv = nv;
       a.shift[n] = shift;    // the gate head is finished in k_softmax_topk (needs the att_ga projection)
+      if (a.alpha_out != nullptr) {
+        for (int r = 0; r <= a.R; ++r) a.alpha_out[(size_t)n * (a.R + 1) + r] = e[r];
+        a.slot_out[n] = slot;
+      }
     }
   }
   __syncthreads();
@@ -781,6 +792,7 @@ int run_step(Ctx* c, const StepIO& io, cudaStream_t st) {
     a.att = fused ? nullptr : c->att; a.ld_att = c->Fp; a.att_b = pair_out(c, c->att_b); a.shift = c->shift;
     a.rows = rows; a.cur_beam = io.cur_beam; a.L = c->L; a.R = c->R; a.F = c->F; a.A = c->A; a.H = H;
     a.ldP = c->NVA;
+    a.alpha_out = io.attn_alpha; a.slot_out = io.attn_slot;
     const size_t smem = sizeof(float) * ((size_t)c->A + (size_t)c->R * c->A + c->R + 1);
     if (!c->attend_attr_set) {     // per device, hence per handle
       VSR_CHECK_CUDA(cudaFuncSetAttribute(k_attend, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));

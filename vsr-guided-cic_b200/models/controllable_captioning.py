@@ -3,7 +3,8 @@
 Keeps the reference's class surface (models/controllable_captioning.py:10-303): constructor
 signature, the 28-tensor state_dict (same names, shapes, dtypes, registration order),
 `init_state`, `step`, `step_v`, `test`, `sample_rl`, and the inherited `forward` /
-`beam_search` / `beam_search_v`.  The parameters live in ordinary torch modules so that
+`beam_search` / `beam_search_v`.  Every decode driver also returns the per-word attention on request
+(`return_attention=True`, see models/CaptioningModel.py), which the reference only exposes as a local of `step_v`.  The parameters live in ordinary torch modules so that
 `.to()`, `.eval()`, `load_state_dict()` work unchanged; all arithmetic of the hot path runs in
 libvsrdec's sm_100a kernels on a packed copy of the weights that is rebuilt whenever the
 parameters change.  CPU tensors raise: this path has no fallback.
@@ -194,8 +195,8 @@ class ControllableCaptioningModel(_CaptioningModel):
             (reference controllable_captioning.py:192-297) '''
         return self._step_impl(t, state, prev_outputs, statics, seqs, mode, True, gt)
 
-    def test(self, detections, ctrl_det_seqs_test):
-        return super().test((detections, ctrl_det_seqs_test))
+    def test(self, detections, ctrl_det_seqs_test, return_attention=False):
+        return super().test((detections, ctrl_det_seqs_test), return_attention=return_attention)
 
-    def sample_rl(self, detections, ctrl_det_seqs_test, seed=None):
-        return super().sample_rl((detections, ctrl_det_seqs_test), seed=seed)
+    def sample_rl(self, detections, ctrl_det_seqs_test, seed=None, return_attention=False):
+        return super().sample_rl((detections, ctrl_det_seqs_test), seed=seed, return_attention=return_attention)

@@ -46,6 +46,8 @@ EXPORTED_SYMBOLS = {
     "vsr_forward_teacher": (ctypes.c_int, [c_vp, c_vp, c_i32, c_vp, c_vp, c_vp]),
     "vsr_greedy": (ctypes.c_int, [c_vp, c_vp, c_vp, c_vp]),
     "vsr_sample": (ctypes.c_int, [c_vp, ctypes.c_uint64, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "vsr_set_attention_capture": (ctypes.c_int, [c_vp, c_i32]),
+    "vsr_get_attention": (ctypes.c_int, [c_vp, c_vp, c_vp, c_vp]),
     "vsr_launch_count": (c_i64, [c_vp]),
     "vsr_gemm_kind": (ctypes.c_char_p, [c_vp]),
     "vsr_set_profiling": (ctypes.c_int, [c_vp, c_i32]),

@@ -42,6 +42,7 @@ class DecoderEngine:
         self.device = weights[0].device
         self._keep = None
         self._weights = None
+        self._attn_shape = None
         self.handle = c_vp()
         d = VsrDims(*(int(self.dims[k]) for k in ("seq_len", "vocab_size", "bos_idx", "det_feat_size",
                                                    "input_encoding_size", "rnn_size", "att_size",
@@ -219,6 +220,7 @@ class DecoderEngine:
                 words.data_ptr(), gates.data_ptr(), lpw.data_ptr(), lpg.data_ptr(), tr_ref,
                 _stream_ptr(dev)))
         self._last = (T, b, beam_size)
+        self._attn_shape = (b, out_size, T, self.R)
         return (words, gates), (lpw, lpg), extra
 
     def history(self):
@@ -243,6 +245,7 @@ class DecoderEngine:
         with torch.cuda.device(self.device):
             _lib.check(self.lib, self.lib.vsr_forward_teacher(self.handle, cap.data_ptr(), T, out.data_ptr(),
                                                               gate.data_ptr(), _stream_ptr(self.device)))
+        self._attn_shape = (b, None, T, self.R)
         return out, gate
 
     def greedy(self):
@@ -252,6 +255,7 @@ class DecoderEngine:
         with torch.cuda.device(self.device):
             _lib.check(self.lib, self.lib.vsr_greedy(self.handle, words.data_ptr(), gates.data_ptr(),
                                                      _stream_ptr(self.device)))
+        self._attn_shape = (b, None, T, self.R)
         return words, gates
 
     def sample(self, seed: int):
@@ -265,7 +269,29 @@ class DecoderEngine:
             _lib.check(self.lib, self.lib.vsr_sample(self.handle, int(seed) & 0xFFFFFFFFFFFFFFFF, words.data_ptr(),
                                                      gates.data_ptr(), lpw.data_ptr(), lpg.data_ptr(),
                                                      _stream_ptr(self.device)))
+        self._attn_shape = (b, None, T, self.R)
         return (words, gates), (lpw, lpg)
+
+    # ------------------------------------------------------------------ attention capture
+    def set_attention_capture(self, on: bool):
+        """Record the per-step attention of the following decodes (vsr_set_attention_capture); off by default."""
+        _lib.check(self.lib, self.lib.vsr_set_attention_capture(self.handle, int(bool(on))))
+
+    def attention(self):
+        """Attention of the last decode (vsr_get_attention): {"alpha": float32, "slot": int64}, shaped
+        (b, out_size, T, R+1) / (b, out_size, T) after a beam search (following each returned beam's back-pointer
+        path), (b, T, R+1) / (b, T) after the other drivers.  alpha[..., 0] is the sentinel, alpha[..., r+1] region r
+        of the slot read at that step.  Raises VsrError when that decode ran without capture."""
+        if self._attn_shape is None:
+            raise VsrError("attention(): no decode has run on this engine")
+        b, out_size, T, R = self._attn_shape
+        lead = (b, T) if out_size is None else (b, out_size, T)
+        alpha = torch.empty(lead + (R + 1,), device=self.device, dtype=torch.float32)
+        slot = torch.empty(lead, device=self.device, dtype=torch.int32)
+        with torch.cuda.device(self.device):
+            _lib.check(self.lib, self.lib.vsr_get_attention(self.handle, alpha.data_ptr(), slot.data_ptr(),
+                                                            _stream_ptr(self.device)))
+        return {"alpha": alpha, "slot": slot.long()}
 
     # ------------------------------------------------------------------ instrumentation
     def launch_count(self) -> int:

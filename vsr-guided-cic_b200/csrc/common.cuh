@@ -233,6 +233,10 @@ int make_pair_maps(F16Pair* b, int pair_rows);   // tensor maps of a weight for 
 // x -> pair (fp16 hi + fp16 lo and/or e4m3 hi8/lo8, whichever arrays the pair has); scale = device {s, 1/s} computed
 // here from max|x| (weights), or null: x is multiplied by p.act_scale (activations)
 int launch_split_pair(const float* x, const F16Pair& p, size_t n, cudaStream_t st, bool weight_scale = false);
+#ifdef VSR_DBG_CLK
+// debug builds only: prints the per-tile clock64 phases recorded by the last k_gemm_pair launch, then clears them
+void tc_dbg_clk_report(const char* label);
+#endif
 
 // ---------------------------------------------------------------- context
 struct Phase {

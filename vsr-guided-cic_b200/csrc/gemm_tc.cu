@@ -26,6 +26,8 @@
 #include <string.h>
 #include <cuda_fp16.h>
 
+#include <algorithm>
+
 #include "common.cuh"
 
 namespace vsr {
@@ -209,6 +211,21 @@ struct TcParams {
 // swizzled) in shared memory and lets all eight epilogue warps work on it with lanes running ALONG a row:
 // every global load / store of a warp is then 128 contiguous bytes per row.
 __device__ __forceinline__ void epi_bar(int id) { asm volatile("bar.sync %0, %1;" ::"r"(id), "n"(TC_EPI_THREADS) : "memory"); }
+
+#ifdef VSR_DBG_CLK
+// k_gemm_pair's clock64 record of one tile of one CTA (tc_dbg_clk_report): absolute clocks of the CTA's SM, except the
+// durations in DBG_MFULL and the per-quarter [dump, epi_bar(3), process, epi_bar(4)] block of epilogue warp 2 at DBG_Q
+enum {
+  DBG_M0, DBG_M1, DBG_M2, DBG_MFULL,            // MMA issuer (leader): tmem_empty wait from M0 to M1, k-loop M1..M2, sum of full waits
+  DBG_E0, DBG_E1, DBG_E2, DBG_E3, DBG_E4,       // epilogue: start, bias + epi_bar(1) done, tmem_full done, accumulator released, end
+  DBG_Q, DBG_F = DBG_Q + 16
+};
+constexpr int DBG_CTAS = 160, DBG_TILES = 48;
+__device__ long long g_dbg_clk[DBG_CTAS * DBG_TILES * DBG_F];
+__device__ __forceinline__ long long* dbg_rec(int ti) {
+  return (blockIdx.x < DBG_CTAS && ti < DBG_TILES) ? g_dbg_clk + ((size_t)blockIdx.x * DBG_TILES + ti) * DBG_F : nullptr;
+}
+#endif
 __device__ __forceinline__ void add4(float4& a, const float4 b) { a.x += b.x; a.y += b.y; a.z += b.z; a.w += b.w; }
 
 // float offset of 16-byte piece c4 of tile row r (XOR swizzle inside aligned groups of 8 pieces: conflict-free both for
@@ -248,8 +265,27 @@ __device__ __forceinline__ void tile_dump(uint32_t tlane, float* tile, int hsel,
 template <int BN>
 __device__ __forceinline__ void tile_plain(const TcProblem& p, const float* tile, const float* s_bias, int rowq, int n0, int te) {
   constexpr int P4 = BN / 4, ITEMS = 32 * P4 / TC_EPI_THREADS;     // 16-byte pieces per row, pieces per thread
-  float4 acc[ITEMS], x0[ITEMS], x1[ITEMS], x2[ITEMS];
   const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
+  // Tiles with nothing but the bias to add (GEMM-B, the h1' projection outside the g_t columns): the general loop below
+  // spends ~6 k cycles per lane quarter in per-piece tests and parameter reloads, more than the 32 KB of stores it
+  // issues.  Same sums in the same order (the zero addends included: x + 0 turns -0 into +0), so the results are
+  // bit-identical.
+  if (n0 >= p.gt_cols && p.rowadd == nullptr && p.cadd == nullptr && p.gather == nullptr) {
+    float* const c = p.c;
+    const int ldc = p.ldc, live = p.M - rowq;
+#pragma unroll
+    for (int k = 0; k < ITEMS; ++k) {
+      const int idx = te + k * TC_EPI_THREADS;
+      const int r = idx / P4, c4 = idx - r * P4;
+      if (r >= live) break;                // rows grow with k
+      float4 o = *reinterpret_cast<const float4*>(tile + tile_slot<BN>(r, c4));
+      add4(o, *reinterpret_cast<const float4*>(s_bias + 4 * c4));
+      add4(o, zero); add4(o, zero); add4(o, zero);
+      *reinterpret_cast<float4*>(c + (size_t)(rowq + r) * ldc + n0 + 4 * c4) = o;
+    }
+    return;
+  }
+  float4 acc[ITEMS], x0[ITEMS], x1[ITEMS], x2[ITEMS];
 #pragma unroll
   for (int k = 0; k < ITEMS; ++k) {        // all loads first: one round trip for the thread's pieces
     const int idx = te + k * TC_EPI_THREADS;
@@ -362,13 +398,10 @@ __device__ __forceinline__ void tile_cell(const TcProblem& p, const float* tile,
 // all eight epilogue warps: quarter by quarter, dump -> barrier -> cooperative pass -> barrier
 template <int BN>
 __device__ __forceinline__ void tile_epilogue(const TcProblem& p, uint32_t tmem_base, int m0, int n0, int n_tile, int warp, int lane,
-                                              const float* s_bias, float* tile) {
+                                              const float* s_bias, float* tile, long long* clk = nullptr) {
   const int q = warp & 3, hsel = (warp - 2) >> 2, te = (warp - 2) * 32 + lane;
   const uint32_t tlane = tmem_base + ((uint32_t)(q * 32) << 16);
   const float sc = (p.acc_scale != nullptr ? __ldg(p.acc_scale) : 1.f) * p.act_inv;
-#ifdef VSR_DBG_CLK
-  long long td = 0, tb1 = 0, tp = 0, tb2 = 0;
-#endif
 #pragma unroll 1
   for (int qq = 0; qq < 4; ++qq) {
     if (m0 + qq * 32 >= p.M) break;                 // no live row in this or any later quarter (uniform)
@@ -395,13 +428,12 @@ __device__ __forceinline__ void tile_epilogue(const TcProblem& p, uint32_t tmem_
 #endif
     epi_bar(4);
 #ifdef VSR_DBG_CLK
-    td += c1 - c0; tb1 += c2 - c1; tp += c3 - c2; tb2 += clock64() - c3;
+    if (clk != nullptr && warp == 2 && lane == 0) {    // warp 2 dumps quarter 2; in the others its bar(3) wait is the dump
+      long long* q4 = clk + DBG_Q + 4 * qq;
+      q4[0] = c1 - c0; q4[1] = c2 - c1; q4[2] = c3 - c2; q4[3] = clock64() - c3;
+    }
 #endif
   }
-#ifdef VSR_DBG_CLK
-  if (lane == 0 && (warp == 2 || warp == 4 || warp == 9) && blockIdx.x == 5 && p.M > 200)
-    printf("epi BN=%d mode=%d warp=%d: dump %lld bar1 %lld process %lld bar2 %lld\n", BN, p.mode, warp, td, tb1, tp, tb2);
-#endif
 }
 
 // Vocabulary-head epilogue: besides storing the logits (acc + bias) the thread that owns a row reduces every 16-column
@@ -942,7 +974,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1) k_gem
   const int mp0 = (params.pr[0].m_tiles + 1) >> 1;
   const int tiles0 = params.pr[0].n_tiles * mp0;
   const int total_tiles = tiles0 + (params.nprob > 1 ? params.pr[1].n_tiles * ((params.pr[1].m_tiles + 1) >> 1) : 0);
-  uint8_t* smem = reinterpret_cast<uint8_t*>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
+  // 1 KB-aligned by pointer arithmetic on smem_raw (not through an integer): the epilogue's staging-tile accesses then
+  // compile to shared-memory loads / stores instead of generic ones
+  uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
 
   pdl_trigger();
   pdl_wait();                       // (no early weight prefetch here: multi-wave launches hide the set-up anyway)
@@ -1016,12 +1050,26 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1) k_gem
     } else if (warp == 1) {
       if (lane == 0 && rank == 0) {
         constexpr uint32_t idesc = make_idesc_pair<BN>();
+#ifdef VSR_DBG_CLK
+        long long* clk = dbg_rec(ti);
+        const long long m0c = clock64();
+        long long mfull = 0;
+#endif
         mbar_wait(&tmem_empty_bar[acc], aph ^ 1);       // both CTAs' epilogues have drained this accumulator
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+#ifdef VSR_DBG_CLK
+        const long long m1c = clock64();
+#endif
         for (int kb = 0; kb < total_kb; ++kb) {
           const int st = (it + kb) % Cfg::kStages;
           const uint32_t ph = ((it + kb) / Cfg::kStages) & 1;
+#ifdef VSR_DBG_CLK
+          const long long f0 = clock64();
+#endif
           mbar_wait(&full_bar[st], ph);
+#ifdef VSR_DBG_CLK
+          mfull += clock64() - f0;
+#endif
           asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
           const uint32_t base = smem_u32(smem + st * Cfg::kStageBytes);
           const uint32_t wbase = base + 2 * Cfg::kABytes;
@@ -1053,26 +1101,44 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1) k_gem
           umma_commit_pair(&empty_bar[st]);     // frees this stage in BOTH CTAs
         }
         umma_commit_pair(&tmem_full_bar[acc]);  // accumulators complete in both CTAs -> epilogues
+#ifdef VSR_DBG_CLK
+        if (clk != nullptr) { clk[DBG_M0] = m0c; clk[DBG_M1] = m1c; clk[DBG_M2] = clock64(); clk[DBG_MFULL] = mfull; }
+#endif
       }
       __syncwarp();
     } else {
       // bias of the tile -> shared memory behind the main loop
+#ifdef VSR_DBG_CLK
+      long long* clk = (warp == 2 && lane == 0) ? dbg_rec(ti) : nullptr;
+      const long long e0c = clock64();
+#endif
       if (ti != 0) epi_bar(1);                  // previous tile's readers are done
       for (int i = (warp - 2) * 32 + lane; i < BN; i += TC_EPI_THREADS) s_bias[i] = p.bias != nullptr ? __ldg(p.bias + n0 + i) : 0.f;
       epi_bar(1);
+#ifdef VSR_DBG_CLK
+      const long long e1c = clock64();
+#endif
       mbar_wait(&tmem_full_bar[acc], aph);
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+#ifdef VSR_DBG_CLK
+      const long long e2c = clock64();
+#else
+      long long* clk = nullptr;
+#endif
       if constexpr (VOCAB) {
         const int q = warp & 3, row = m0 + q * 32 + lane;
         vocab_epilogue<BN>(p, tmem_acc + ((uint32_t)(q * 32) << 16), row, row < p.M, n0, s_bias, (warp - 2) >> 2);
       } else {
-        tile_epilogue<BN>(p, tmem_acc, m0, n0, n_tile, warp, lane, s_bias, reinterpret_cast<float*>(smem + Cfg::kRingBytes));
+        tile_epilogue<BN>(p, tmem_acc, m0, n0, n_tile, warp, lane, s_bias, reinterpret_cast<float*>(smem + Cfg::kRingBytes), clk);
       }
       asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
       __syncwarp();
       if (lane == 0) {                          // every epilogue warp of both CTAs -> the leader's barrier
         if (rank == 0) mbar_arrive(&tmem_empty_bar[acc]); else mbar_arrive_cluster(&tmem_empty_bar[acc], 0);
       }
+#ifdef VSR_DBG_CLK
+      if (clk != nullptr) { clk[DBG_E0] = e0c; clk[DBG_E1] = e1c; clk[DBG_E2] = e2c; clk[DBG_E3] = clk[DBG_E4] = clock64(); }
+#endif
     }
     it += total_kb;
     ++ti;
@@ -1213,6 +1279,77 @@ int tc_gemm_init() {
   if (dev < 64) done_mask |= 1ull << dev;
   return VSR_OK;
 }
+
+#ifdef VSR_DBG_CLK
+void tc_dbg_clk_report(const char* label) {
+  std::vector<long long> r((size_t)DBG_CTAS * DBG_TILES * DBG_F);
+  void* sym = nullptr;
+  if (cudaDeviceSynchronize() != cudaSuccess || cudaGetSymbolAddress(&sym, g_dbg_clk) != cudaSuccess ||
+      cudaMemcpy(r.data(), sym, r.size() * sizeof(long long), cudaMemcpyDeviceToHost) != cudaSuccess) {
+    printf("clk %s: no records\n", label);
+    return;
+  }
+  cudaMemset(sym, 0, r.size() * sizeof(long long));
+  int khz = 1;
+  cudaDeviceGetAttribute(&khz, cudaDevAttrClockRate, 0);
+  enum { S_MWAIT, S_MLOOP, S_MFULL, S_BIAS, S_EWAIT, S_RELEASE, S_BODY, S_DUMP, S_BAR3, S_PROC, S_BAR4, S_N };
+  static const char* names[S_N] = {"mma: wait tmem_empty", "mma: k-loop span", "mma:   of it waiting full_bar", "epi: bias + epi_bar(1)",
+                                   "epi: wait tmem_full", "epi: full -> accumulator released", "epi: full -> tile done",
+                                   "epi: dump (4 quarters)", "epi: epi_bar(3) (4 quarters)", "epi: process (4 quarters)",
+                                   "epi: epi_bar(4) (4 quarters)"};
+  std::vector<double> v[S_N];
+  double span = 0, mma_busy = 0, epi_busy = 0, overlap = 0;
+  int ctas = 0, max_tiles = 0;
+  for (int b = 0; b < DBG_CTAS; ++b) {
+    const long long* c = r.data() + (size_t)b * DBG_TILES * DBG_F;
+    int nt = 0;
+    while (nt < DBG_TILES && c[nt * DBG_F + DBG_E4] != 0) ++nt;
+    if (nt == 0) continue;
+    max_tiles = nt > max_tiles ? nt : max_tiles;
+    const bool leader = c[DBG_M2] != 0;
+    for (int t = 0; t < nt; ++t) {
+      const long long* x = c + t * DBG_F;
+      if (leader) { v[S_MWAIT].push_back(x[DBG_M1] - x[DBG_M0]); v[S_MLOOP].push_back(x[DBG_M2] - x[DBG_M1]); v[S_MFULL].push_back(x[DBG_MFULL]); }
+      v[S_BIAS].push_back(x[DBG_E1] - x[DBG_E0]); v[S_EWAIT].push_back(x[DBG_E2] - x[DBG_E1]);
+      v[S_RELEASE].push_back(x[DBG_E3] - x[DBG_E2]); v[S_BODY].push_back(x[DBG_E4] - x[DBG_E2]);
+      for (int ph = 0; ph < 4; ++ph) {
+        long long sum = 0;
+        for (int q = 0; q < 4; ++q) sum += x[DBG_Q + 4 * q + ph];
+        v[S_DUMP + ph].push_back(sum);
+      }
+    }
+    if (!leader) continue;
+    // the leader's MMA issuer and epilogue share the SM clock: how much of the epilogue ran under a k-loop
+    ++ctas;
+    span += c[(nt - 1) * DBG_F + DBG_E4] - c[DBG_M0];
+    for (int t = 0; t < nt; ++t) {
+      const long long* e = c + t * DBG_F;
+      mma_busy += e[DBG_M2] - e[DBG_M1];
+      epi_busy += e[DBG_E4] - e[DBG_E2];
+      for (int u = 0; u < nt; ++u) {
+        const long long* m = c + u * DBG_F;
+        const long long lo = m[DBG_M1] > e[DBG_E2] ? m[DBG_M1] : e[DBG_E2], hi = m[DBG_M2] < e[DBG_E4] ? m[DBG_M2] : e[DBG_E4];
+        if (hi > lo) overlap += hi - lo;
+      }
+    }
+  }
+  const double us = 1e3 / khz;
+  printf("clk %s: %d leader CTAs, up to %d tiles per CTA, cycles per tile (us at %d MHz): mean / median / p90\n", label, ctas,
+         max_tiles, khz / 1000);
+  for (int k = 0; k < S_N; ++k) {
+    std::vector<double>& x = v[k];
+    if (x.empty()) continue;
+    std::sort(x.begin(), x.end());
+    double m = 0;
+    for (double y : x) m += y;
+    m /= x.size();
+    printf("  %-36s %8.0f %8.0f %8.0f  (%.2f us)\n", names[k], m, x[x.size() / 2], x[x.size() * 9 / 10], m * us);
+  }
+  if (ctas > 0)
+    printf("  per leader CTA: span %.1f us, k-loops %.1f us, epilogues %.1f us, epilogue under a k-loop %.1f us (%.0f %% of the epilogue)\n",
+           span / ctas * us, mma_busy / ctas * us, epi_busy / ctas * us, overlap / ctas * us, 100.0 * overlap / (epi_busy > 0 ? epi_busy : 1));
+}
+#endif
 
 static int fill_problem(TcProblem* p, const GemmArgs& g, int BN, int kb = 64, bool pair = false) {
   VSR_REQUIRE(g.M > 0 && g.N >= round_up(g.wb->n_valid, BN), VSR_EINVAL, "launch_gemm_tc: N=%d too small for N tile %d", g.N, BN);

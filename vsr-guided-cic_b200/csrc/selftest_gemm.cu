@@ -47,6 +47,7 @@ static void make_pair(F16Pair* b, const float* f, int rows, int ld, int box, boo
 static bool g_time = true;
 static bool g_f8 = false;
 static bool g_pair = false;      // CTA-pair kernel (needs M >= 1024; BN = pair tile width)
+static bool g_vocab = false;     // vocabulary-head epilogue (logits + chunk records; the logits are checked)
 static int run_case(int M, int N, int nseg, const int* ks, bool extras, int BN, float wscale = 0.05f) {
   const int Mp = (M + 127) / 128 * 128;
   int K = 0; for (int s = 0; s < nseg; ++s) K += ks[s];
@@ -68,11 +69,17 @@ static int run_case(int M, int N, int nseg, const int* ks, bool extras, int BN, 
     bias = dev_rand(N, 1.f, 5); radd = dev_rand((size_t)(Mp / 5 + 1) * N, 1.f, 6); cadd = dev_rand((size_t)Mp * (N + 64), 1.f, 7);
     g.bias = bias; g.rowadd = radd; g.ld_rowadd = N; g.row_div = 5; g.rowadd_mul = 1; g.cadd = cadd + 64; g.ld_cadd = N + 64;
   }
+  float* vpart = nullptr;
+  if (g_vocab) {
+    bias = dev_rand(N, 1.f, 5); g.bias = bias;
+    CK(cudaMalloc(&vpart, (size_t)Mp * (N / 16) * 2 * sizeof(float)));
+  }
   float *C1, *C2;
   CK(cudaMalloc(&C1, (size_t)Mp * N * 4)); CK(cudaMalloc(&C2, (size_t)Mp * N * 4));
   CK(cudaMemset(C1, 0, (size_t)Mp * N * 4)); CK(cudaMemset(C2, 0, (size_t)Mp * N * 4));
   g.M = M; g.N = N; g.ldc = N;
   g.c = C1; VK(launch_gemm_simt(g, 0));
+  if (g_vocab) { g.cell.mode = 3; g.cell.vocab_part = vpart; }
   g.c = C2; VK(launch_gemm_tc(g, nullptr, 0));
   CK(cudaDeviceSynchronize());
   std::vector<float> h1((size_t)M * N), h2((size_t)M * N);
@@ -92,6 +99,13 @@ static int run_case(int M, int N, int nseg, const int* ks, bool extras, int BN, 
     cudaEventRecord(e0); for (int i = 0; i < 10; ++i) { g.c = C2; VK(launch_gemm_tc(g, nullptr, 0)); } cudaEventRecord(e1); CK(cudaEventSynchronize(e1));
     cudaEventElapsedTime(&ms_tc, e0, e1);
   }
+#ifdef VSR_DBG_CLK
+  if (g_pair) {
+    char label[96];
+    snprintf(label, sizeof(label), "M=%d N=%d K=%d BN=%d%s", M, N, K, BN, g_vocab ? " vocab" : "");
+    tc_dbg_clk_report(label);
+  }
+#endif
   cudaEventRecord(e0); for (int i = 0; i < 3; ++i) { g.c = C1; VK(launch_gemm_simt(g, 0)); } cudaEventRecord(e1); CK(cudaEventSynchronize(e1));
   cudaEventElapsedTime(&ms_simt, e0, e1);
   const double flops = 2.0 * M * N * K;
@@ -117,11 +131,13 @@ int main(int argc, char** argv) {
     return 0;
   }
   const int k1[] = {64}, k2[] = {1024}, k3[] = {1024, 1024, 1024}, k4[] = {2048, 1024}, k5[] = {64, 64, 64};
-  if (argc > 1 && strcmp(argv[1], "epi") == 0) {   // CTA-pair kernel at the 1000-caption step shapes (B-, D-like): timing; with
-    g_pair = true; g_f8 = true;                     // -DVSR_DBG_CLK the epilogue's cycle breakdown is printed by the kernel
+  if (argc > 1 && strcmp(argv[1], "epi") == 0) {   // CTA-pair kernel at the 1000-caption step shapes (B-, D-, vocabulary-like):
+    g_pair = true; g_f8 = true;                     // timing; with -DVSR_DBG_CLK also the per-tile clock64 phases of the last launch
     const int k6[] = {2048, 1024, 1024};
     bad += run_case(5000, 4096, 1, k2, false, 256);
     bad += run_case(5000, 4096, 3, k6, false, 256);
+    g_vocab = true;
+    bad += run_case(5000, 10368, 1, k2, false, 192);
     return bad ? 1 : 0;
   }
   if (argc > 1 && strcmp(argv[1], "quick") == 0) {   // one launch per kernel variant, no timing loops (compute-sanitizer)

@@ -44,10 +44,13 @@ extern "C" {
 #define VSR_MAX_SEQ_LEN 256 /* largest seq_len of the beam-search back-track kernel  */
 #define VSR_NUM_WEIGHTS 28
 
-/* dtype tags for the `verbs` tensor (eval_coco.py:240 hands float64 from numpy) */
+/* dtype tags: the `verbs` tensor takes F64 / F32 / I64 (eval_coco.py:240 hands float64 from numpy);
+ * the region features of vsr_prologue_ex / vsr_prologue_indexed_ex take F32 / F16 / BF16 */
 #define VSR_DT_F64 0
 #define VSR_DT_F32 1
 #define VSR_DT_I64 2
+#define VSR_DT_F16 3   /* IEEE binary16 (__half)      */
+#define VSR_DT_BF16 4  /* bfloat16 (__nv_bfloat16)    */
 
 typedef struct VsrHandle_* vsr_handle;
 
@@ -56,7 +59,7 @@ typedef struct VsrDims {
   int32_t seq_len;
   int32_t vocab_size;
   int32_t bos_idx;
-  int32_t det_feat_size;       /* must be a multiple of 4 (128-bit feature loads) */
+  int32_t det_feat_size;       /* must be a multiple of 4 (four-element feature loads) */
   int32_t input_encoding_size;
   int32_t rnn_size;
   int32_t att_size;
@@ -111,9 +114,9 @@ int vsr_set_verb_table(vsr_handle h, const int64_t* keys, const int32_t* offsets
  * (controllable_captioning.py:126-128 / 203-205 image descriptor; :159/:240 validity of the
  * region rows; :161/:242 att_va projection of every slot tile; the img columns of
  * W1_is / lstm_cell_1.weight_ih / W1_ig (:151-152,181) and of lstm_cell_2.weight_ih (:174)).
- *   det       (b, D, F) fp32; det_batch_stride in elements, 0 when the caller expanded one
+ *   det       (b, D, F) fp32 (fp16 / bf16 through vsr_prologue_ex); det_batch_stride in elements, 0 when the caller expanded one
  *             image over all captions (eval_coco.py:243)
- *   det_seqs  (b, L, R, F) fp32 slot tiles (feedback: statics[1]; teacher forcing: seqs[1], L=T)
+ *   det_seqs  (b, L, R, F) fp32 slot tiles, same dtype as det (feedback: statics[1]; teacher forcing: seqs[1], L=T)
  *   verbs     (b, L) or NULL; verbs_dtype one of VSR_DT_*; value -1 = no verb in that slot */
 int vsr_prologue(vsr_handle h, const float* det, int64_t det_batch_stride, int32_t D,
                  const float* det_seqs, int32_t b, int32_t L, int32_t R,
@@ -130,6 +133,26 @@ int vsr_prologue(vsr_handle h, const float* det, int64_t det_batch_stride, int32
 int vsr_prologue_indexed(vsr_handle h, const float* det, int64_t det_batch_stride, int32_t D,
                          const int32_t* slot_index, int32_t b, int32_t L, int32_t R,
                          const void* verbs, int32_t verbs_dtype, void* stream);
+
+/* Both prologues with the element type of the region features as an argument: feat_dtype is VSR_DT_F32, VSR_DT_F16
+ * or VSR_DT_BF16 and applies to det and det_seqs alike (anything else is VSR_EINVAL).  det_batch_stride stays in
+ * elements.  Feature pointers must be aligned to four elements (16 bytes in fp32, 8 bytes in half precision).
+ * vsr_prologue / vsr_prologue_indexed are these calls with VSR_DT_F32.
+ *   - Every kernel that reads features widens each value to fp32 as it loads it (exact) and then does the fp32
+ *     arithmetic of the fp32 path in the same order, so a decode of half-precision features x is bit-identical to
+ *     a decode of their fp32 upcast.  Only the bytes read change: half the copy and DRAM traffic of the features.
+ *   - The index form's -2 rows (the image mean) stay fp32: the mean is computed in fp32 and never rounded.
+ *   - The magnitude limit of the tensor-core operands (|feature| < 255 in the default f16+f8x2 mode) is unchanged;
+ *     it bounds the activation scale, not the input format.
+ *   - VSRDEC_GEMM=simt (the fp32 FFMA twin, a verification mode that reads det_seqs in place) takes fp32 features
+ *     only: half precision returns VSR_EINVAL.
+ * Every decode entry point works unchanged after either prologue, in any feature dtype. */
+int vsr_prologue_ex(vsr_handle h, const void* det, int64_t det_batch_stride, int32_t D, const void* det_seqs,
+                    int32_t b, int32_t L, int32_t R, int32_t feat_dtype, const void* verbs, int32_t verbs_dtype,
+                    void* stream);
+int vsr_prologue_indexed_ex(vsr_handle h, const void* det, int64_t det_batch_stride, int32_t D,
+                            const int32_t* slot_index, int32_t b, int32_t L, int32_t R, int32_t feat_dtype,
+                            const void* verbs, int32_t verbs_dtype, void* stream);
 
 /* One decoder step for the b prologue captions, one row per caption
  * (ControllableCaptioningModel.step / step_v, controllable_captioning.py:117-190 / 192-297).

@@ -370,6 +370,7 @@ static Ctx::GraphKey graph_key(const Ctx* c, int kind) {
   key.epoch = c->epoch; key.det = c->det; key.det_seqs = c->det_seqs; key.slot_index = c->slot_index; key.verbs = c->verbs;
   key.det_stride = c->det_stride;
   key.b = c->b; key.D = c->D; key.L = c->L; key.R = c->R; key.n_img = c->n_img; key.verbs_dtype = c->verbs_dtype;
+  key.feat_dtype = c->feat_dtype;   // the same addresses and shapes in another dtype run other kernels
   return key;
 }
 
@@ -379,9 +380,9 @@ static bool graphs_usable(Ctx* c, cudaStream_t st) {
   return c->use_graphs && !c->profiling && cap == cudaStreamCaptureStatusNone;
 }
 
-static int prologue_impl(Ctx* c, const float* det, int64_t det_stride, int D, const float* det_seqs,
-                         const int32_t* slot_index, int b, int L, int R, const void* verbs, int verbs_dtype,
-                         cudaStream_t st) {
+static int prologue_impl(Ctx* c, const void* det, int64_t det_stride, int D, const void* det_seqs,
+                         const int32_t* slot_index, int b, int L, int R, int feat_dtype, const void* verbs,
+                         int verbs_dtype, cudaStream_t st) {
   VSR_REQUIRE(det != nullptr && (det_seqs != nullptr || slot_index != nullptr), VSR_EINVAL, "vsr_prologue: null input");
   VSR_REQUIRE(b > 0 && D > 0 && L > 0 && R > 0, VSR_EINVAL, "vsr_prologue: bad shape b=%d D=%d L=%d R=%d", b, D, L, R);
   VSR_REQUIRE(R <= 64, VSR_EINVAL, "vsr_prologue: R=%d regions per slot > 64 unsupported", R);
@@ -389,13 +390,20 @@ static int prologue_impl(Ctx* c, const float* det, int64_t det_stride, int D, co
   VSR_REQUIRE(verbs == nullptr || (verbs_dtype >= 0 && verbs_dtype <= 2), VSR_EINVAL, "vsr_prologue: bad verbs dtype");
   VSR_REQUIRE(slot_index == nullptr || det_stride == 0 || det_stride == (int64_t)D * c->F, VSR_EINVAL,
               "vsr_prologue_indexed: detections must be dense (b, D, F) or one shared image");
-  VSR_REQUIRE(((uintptr_t)det % 16) == 0 && ((uintptr_t)det_seqs % 16) == 0 && (det_stride % 4) == 0, VSR_EINVAL,
-              "vsr_prologue: feature tensors must be 16-byte aligned");
+  const int esz = feat_elem_size(feat_dtype);
+  VSR_REQUIRE(esz != 0, VSR_EINVAL, "vsr_prologue: feat_dtype=%d is not VSR_DT_F32, VSR_DT_F16 or VSR_DT_BF16", feat_dtype);
+  VSR_REQUIRE(feat_dtype == VSR_DT_F32 || c->use_tc, VSR_EINVAL,
+              "vsr_prologue: half-precision features need the tensor-core GEMMs; the fp32 FFMA twin (VSRDEC_GEMM=simt) "
+              "reads features in place and takes fp32 only");
+  // feature loads are four elements wide: 16 bytes in fp32, 8 in half precision
+  VSR_REQUIRE(((uintptr_t)det % (4 * esz)) == 0 && ((uintptr_t)det_seqs % (4 * esz)) == 0 && (det_stride % 4) == 0,
+              VSR_EINVAL, "vsr_prologue: feature tensors must be %d-byte aligned", 4 * esz);
   c->have_prologue = false;
   if (c->profiling) reset_phases(c);   // a decode job starts here
   c->b = b; c->D = D; c->L = L; c->R = R;
   c->n_img = det_stride == 0 ? 1 : b;
   c->det_seqs = det_seqs; c->slot_index = slot_index; c->det = det; c->det_stride = det_stride;
+  c->feat_dtype = feat_dtype;
   c->verbs = verbs; c->verbs_dtype = verbs_dtype;
   const size_t n_img_pad = round_up(c->n_img, MPAD);
   if (n_img_pad > c->cap_img) {
@@ -766,21 +774,34 @@ int vsr_set_verb_table(vsr_handle h, const int64_t* keys, const int32_t* offsets
   return VSR_OK;
 }
 
-int vsr_prologue(vsr_handle h, const float* det, int64_t det_batch_stride, int32_t D, const float* det_seqs,
-                 int32_t b, int32_t L, int32_t R, const void* verbs, int32_t verbs_dtype, void* stream) {
+int vsr_prologue_ex(vsr_handle h, const void* det, int64_t det_batch_stride, int32_t D, const void* det_seqs,
+                    int32_t b, int32_t L, int32_t R, int32_t feat_dtype, const void* verbs, int32_t verbs_dtype,
+                    void* stream) {
   if (!h) { vsr::set_error("vsr_prologue: null handle"); return VSR_EINVAL; }
   DeviceGuard dg((const vsr::Ctx*)h);
-  return vsr::prologue_impl((Ctx*)h, det, det_batch_stride, D, det_seqs, nullptr, b, L, R, verbs, verbs_dtype,
-                            (cudaStream_t)stream);
+  return vsr::prologue_impl((Ctx*)h, det, det_batch_stride, D, det_seqs, nullptr, b, L, R, feat_dtype, verbs,
+                            verbs_dtype, (cudaStream_t)stream);
+}
+
+int vsr_prologue_indexed_ex(vsr_handle h, const void* det, int64_t det_batch_stride, int32_t D,
+                            const int32_t* slot_index, int32_t b, int32_t L, int32_t R, int32_t feat_dtype,
+                            const void* verbs, int32_t verbs_dtype, void* stream) {
+  if (!h || !slot_index) { vsr::set_error("vsr_prologue_indexed: null argument"); return VSR_EINVAL; }
+  DeviceGuard dg((const vsr::Ctx*)h);
+  return vsr::prologue_impl((Ctx*)h, det, det_batch_stride, D, nullptr, slot_index, b, L, R, feat_dtype, verbs,
+                            verbs_dtype, (cudaStream_t)stream);
+}
+
+int vsr_prologue(vsr_handle h, const float* det, int64_t det_batch_stride, int32_t D, const float* det_seqs,
+                 int32_t b, int32_t L, int32_t R, const void* verbs, int32_t verbs_dtype, void* stream) {
+  return vsr_prologue_ex(h, det, det_batch_stride, D, det_seqs, b, L, R, VSR_DT_F32, verbs, verbs_dtype, stream);
 }
 
 int vsr_prologue_indexed(vsr_handle h, const float* det, int64_t det_batch_stride, int32_t D,
                          const int32_t* slot_index, int32_t b, int32_t L, int32_t R, const void* verbs,
                          int32_t verbs_dtype, void* stream) {
-  if (!h || !slot_index) { vsr::set_error("vsr_prologue_indexed: null argument"); return VSR_EINVAL; }
-  DeviceGuard dg((const vsr::Ctx*)h);
-  return vsr::prologue_impl((Ctx*)h, det, det_batch_stride, D, nullptr, slot_index, b, L, R, verbs, verbs_dtype,
-                            (cudaStream_t)stream);
+  return vsr_prologue_indexed_ex(h, det, det_batch_stride, D, slot_index, b, L, R, VSR_DT_F32, verbs, verbs_dtype,
+                                 stream);
 }
 
 int vsr_step(vsr_handle h, const float* h1, const float* c1, const float* h2, const float* c2,

@@ -38,6 +38,7 @@ static inline int round_up(int x, int m) { return (x + m - 1) / m * m; }
 
 #ifdef __CUDACC__
 }  // namespace vsr
+#include <cuda_bf16.h>
 #include <cuda_fp16.h>
 #include <cuda_fp8.h>
 namespace vsr {
@@ -47,7 +48,28 @@ namespace vsr {
 // the attention scores / LSTM cells need (checked by the parity tests against the fp32 oracle).
 __device__ __forceinline__ float fast_sigmoid(float x) { return __fdividef(1.f, 1.f + __expf(-x)); }
 __device__ __forceinline__ float fast_tanh(float x) { return 1.f - __fdividef(2.f, __expf(2.f * x) + 1.f); }
+
+// Caller features (det, det_seqs) are fp32, fp16 or bf16 (vsr_prologue_ex).  Four consecutive elements, widened to
+// fp32 as they are loaded: exact, so every kernel that reads features does the same fp32 arithmetic in the same order
+// whatever the storage type.  fp32 is one 16-byte load, half precision one 8-byte load (a row of F % 8 == 4 half
+// elements is only 8-byte aligned).
+__device__ __forceinline__ float4 ldg_feat4(const float* p) { return __ldg(reinterpret_cast<const float4*>(p)); }
+__device__ __forceinline__ float4 ldg_feat4(const __half* p) {
+  const uint2 u = __ldg(reinterpret_cast<const uint2*>(p));
+  const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&u.x));
+  const float2 b = __half22float2(*reinterpret_cast<const __half2*>(&u.y));
+  return make_float4(a.x, a.y, b.x, b.y);
+}
+__device__ __forceinline__ float4 ldg_feat4(const __nv_bfloat16* p) {
+  const uint2 u = __ldg(reinterpret_cast<const uint2*>(p));
+  const float2 a = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&u.x));
+  const float2 b = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&u.y));
+  return make_float4(a.x, a.y, b.x, b.y);
+}
 #endif
+
+// element size in bytes of a feature dtype tag (VSR_DT_F32 / F16 / BF16), 0 for any other tag
+static inline int feat_elem_size(int dt) { return dt == VSR_DT_F32 ? 4 : (dt == VSR_DT_F16 || dt == VSR_DT_BF16) ? 2 : 0; }
 
 // K (reduction) dims are padded to KPAD floats (one 128-byte swizzle row of fp32), output-feature
 // dims to NPAD rows, activation row counts to MPAD rows; pads are zero so they never contribute.
@@ -296,9 +318,11 @@ struct Ctx {
   // prologue products (per batch)
   bool have_prologue = false;
   int b = 0, D = 0, L = 0, R = 0, n_img = 0;
-  const float* det_seqs = nullptr;       // materialised slot tiles (b,L,R,F), or null in index form
+  // caller features, element type feat_dtype (VSR_DT_F32 / F16 / BF16) for det and det_seqs alike
+  const void* det_seqs = nullptr;        // materialised slot tiles (b,L,R,F), or null in index form
   const int32_t* slot_index = nullptr;   // index form: (b,L,R) detection row / -2 mean row / -1 padding
-  const float* det = nullptr; int64_t det_stride = 0;   // index form: detections (n_img, D, F)
+  const void* det = nullptr; int64_t det_stride = 0;   // index form: detections (n_img, D, F); stride in elements
+  int feat_dtype = VSR_DT_F32;
   float* Pmean = nullptr;                // index form: att_va projection of the image mean rows [n_img][NVA]
   const void* verbs = nullptr; int verbs_dtype = 0;
   float* img = nullptr;        // [n_img_alloc][Fp]
@@ -369,7 +393,7 @@ struct Ctx {
     const void* captions;
     const void *det, *det_seqs, *slot_index, *verbs;
     int64_t det_stride, eos0, eos1;
-    int32_t b, D, L, R, n_img, verbs_dtype, k, use_verbs, gt, T, attn;
+    int32_t b, D, L, R, n_img, verbs_dtype, k, use_verbs, gt, T, attn, feat_dtype;
   };
   struct GraphEntry { GraphKey key; cudaGraphExec_t exec; int64_t launches; uint64_t last_use; };
   std::vector<GraphEntry> graphs;
@@ -397,8 +421,8 @@ struct PhaseScope {  // records start/stop events around a phase when profiling 
 
 // ---------------------------------------------------------------- kernels (defined in *.cu)
 int pack_weights(Ctx* c, const float* const* w, cudaStream_t st);
-int run_prologue(Ctx* c, const float* det, int64_t det_stride, cudaStream_t st);
-int run_prologue_indexed(Ctx* c, const float* det, int64_t det_stride, cudaStream_t st);
+int run_prologue(Ctx* c, const void* det, int64_t det_stride, cudaStream_t st);
+int run_prologue_indexed(Ctx* c, const void* det, int64_t det_stride, cudaStream_t st);
 int ensure_rows(Ctx* c, int rows);
 int ensure_beam_ws(Ctx* c, int caps, int T);
 

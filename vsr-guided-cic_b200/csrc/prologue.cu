@@ -48,18 +48,22 @@ __global__ void k_pack_bias(float* __restrict__ dst, int o0, const float* __rest
   if (i < n) dst[o0 + i] = a[i] + (b != nullptr ? b[i] : 0.f);
 }
 
+// The kernels that read caller features are templates on their element type T (float, __half, __nv_bfloat16):
+// each value is widened to fp32 as it is loaded (ldg_feat4), after which the arithmetic is T-independent.
+
 // one warp per row: flag[row] = (sum_f x[row][f] != 0).  Row r of image/caption g lives at
 // base + g*group_stride + (r % rows_per_group)*F.
 // Optionally also writes the row's fp16 hi/lo split (operand of the tcgen05 att_va projection).
-__global__ void k_row_valid(const float* __restrict__ x, int64_t group_stride, int rows_per_group,
+template <typename T>
+__global__ void k_row_valid(const T* __restrict__ x, int64_t group_stride, int rows_per_group,
                             int total_rows, int F, uint8_t* __restrict__ flag, PairOut split) {
   const int row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (row >= total_rows) return;
-  const float* p = x + (size_t)(row / rows_per_group) * group_stride + (size_t)(row % rows_per_group) * F;
+  const T* p = x + (size_t)(row / rows_per_group) * group_stride + (size_t)(row % rows_per_group) * F;
   float s = 0.f;
   for (int f = lane * 4; f < F; f += 128) {
-    const float4 v = __ldg(reinterpret_cast<const float4*>(p + f));
+    const float4 v = ldg_feat4(p + f);
     s += (v.x + v.y) + (v.z + v.w);
     if (split.on()) store_pair4(split, (size_t)row * split.ld + f, v);
   }
@@ -106,7 +110,8 @@ __global__ void __launch_bounds__(1024) k_slot_scan(const unsigned long long* __
 }
 
 // one warp per source row: valid rows are split to fp16 hi/lo at their compact position
-__global__ void k_split_compact(const float* __restrict__ x, int R, int total_rows, int F,
+template <typename T>
+__global__ void k_split_compact(const T* __restrict__ x, int R, int total_rows, int F,
                                 const unsigned long long* __restrict__ mask, const int32_t* __restrict__ slot_base,
                                 PairOut split) {
   const int row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -116,9 +121,9 @@ __global__ void k_split_compact(const float* __restrict__ x, int R, int total_ro
   const unsigned long long m = mask[s];
   if (!((m >> r) & 1ull)) return;
   const int dst = slot_base[s] + __popcll(m & ((1ull << r) - 1ull));
-  const float* p = x + (size_t)row * F;
+  const T* p = x + (size_t)row * F;
   for (int f = lane * 4; f < F; f += 128)
-    store_pair4(split, (size_t)dst * split.ld + f, __ldg(reinterpret_cast<const float4*>(p + f)));
+    store_pair4(split, (size_t)dst * split.ld + f, ldg_feat4(p + f));
 }
 
 // index form: validity mask of a slot from its detection indices (-2 = image mean row, valid iff the image
@@ -142,7 +147,8 @@ __global__ void k_slot_masks_indexed(const int32_t* __restrict__ slot_index, con
 // img[g][f] = sum_d det[g][d][f] / count(valid rows of g).  Block (128, POOL_Y): thread (x, y) sums the rows
 // d = y, y + POOL_Y, ... of float4 column x; the POOL_Y partial sums are combined in a fixed order (deterministic).
 constexpr int POOL_Y = 4;
-__global__ void __launch_bounds__(128 * POOL_Y) k_pool(const float* __restrict__ det, int64_t img_stride, int D, int F,
+template <typename T>
+__global__ void __launch_bounds__(128 * POOL_Y) k_pool(const T* __restrict__ det, int64_t img_stride, int D, int F,
                        const uint8_t* __restrict__ valid, float* __restrict__ img, int ld_img, PairOut split) {
   __shared__ float4 s_part[POOL_Y][128];
   __shared__ int s_cnt;
@@ -159,13 +165,13 @@ __global__ void __launch_bounds__(128 * POOL_Y) k_pool(const float* __restrict__
   }
   float4 s = make_float4(0.f, 0.f, 0.f, 0.f);
   if (f < F) {
-    const float* p = det + (size_t)g * img_stride + f;
+    const T* p = det + (size_t)g * img_stride + f;
     for (int d0 = ty; d0 < D; d0 += 8 * POOL_Y) {     // 8 independent row loads in flight
       float4 v[8];
 #pragma unroll
       for (int u = 0; u < 8; ++u) {
         const int d = d0 + u * POOL_Y;
-        v[u] = d < D ? __ldg(reinterpret_cast<const float4*>(p + (size_t)d * F)) : make_float4(0.f, 0.f, 0.f, 0.f);
+        v[u] = d < D ? ldg_feat4(p + (size_t)d * F) : make_float4(0.f, 0.f, 0.f, 0.f);
       }
 #pragma unroll
       for (int u = 0; u < 8; ++u) { s.x += v[u].x; s.y += v[u].y; s.z += v[u].z; s.w += v[u].w; }
@@ -317,9 +323,19 @@ int pack_weights(Ctx* c, const float* const* w, cudaStream_t st) {
   return VSR_OK;
 }
 
-int run_prologue(Ctx* c, const float* det, int64_t det_stride, cudaStream_t st) {
+// calls fn(T()) with T the element type of feature dtype tag dt (validated by prologue_impl)
+template <typename Fn>
+static int with_feat_type(int dt, Fn&& fn) {
+  if (dt == VSR_DT_F16) return fn(__half());
+  if (dt == VSR_DT_BF16) return fn(__nv_bfloat16());
+  return fn(float());
+}
+
+template <typename T>
+static int run_prologue_t(Ctx* c, const T* det, int64_t det_stride, cudaStream_t st) {
   PhaseScope ps(c, PH_PROLOGUE, st);
   const int F = c->F, D = c->D, b = c->b, L = c->L, R = c->R;
+  const T* det_seqs = static_cast<const T*>(c->det_seqs);
   const int n_img = c->n_img;
   // validity of detection rows and slot rows
   {
@@ -328,7 +344,7 @@ int run_prologue(Ctx* c, const float* det, int64_t det_stride, cudaStream_t st) 
     k_row_valid<<<(rows * 32 + 255) / 256, 256, 0, st>>>(det, det_stride, D, rows, F, c->det_valid, none);
     VSR_CHECK_CUDA(cudaGetLastError());
     const int srows = b * L * R;
-    k_row_valid<<<(int)(((size_t)srows * 32 + 255) / 256), 256, 0, st>>>(c->det_seqs, (int64_t)L * R * F, L * R,
+    k_row_valid<<<(int)(((size_t)srows * 32 + 255) / 256), 256, 0, st>>>(det_seqs, (int64_t)L * R * F, L * R,
                                                                           srows, F, c->seq_valid, none);
     VSR_CHECK_CUDA(cudaGetLastError());
     k_slot_masks<<<(b * L + 127) / 128, 128, 0, st>>>(c->seq_valid, R, b * L, c->slot_mask);
@@ -339,7 +355,7 @@ int run_prologue(Ctx* c, const float* det, int64_t det_stride, cudaStream_t st) 
       const PairOut dsp{twin_out(&c->ds_b), c->Fp};
       k_slot_scan<<<1, 1024, 0, st>>>(c->slot_mask, b * L, c->slot_base, c->comp_valid, round_up(srows, MPAD));
       VSR_CHECK_CUDA(cudaGetLastError());
-      k_split_compact<<<(int)(((size_t)srows * 32 + 255) / 256), 256, 0, st>>>(c->det_seqs, R, srows, F, c->slot_mask,
+      k_split_compact<<<(int)(((size_t)srows * 32 + 255) / 256), 256, 0, st>>>(det_seqs, R, srows, F, c->slot_mask,
                                                                                c->slot_base, dsp);
       VSR_CHECK_CUDA(cudaGetLastError());
       c->launches += 2;
@@ -370,10 +386,11 @@ int run_prologue(Ctx* c, const float* det, int64_t det_stride, cudaStream_t st) 
       c->launches++;
     }
   }
-  // P = att_va . det_seqs rows (tiles of padding rows are skipped)
+  // P = att_va . det_seqs rows (tiles of padding rows are skipped).  The tensor-core path reads the fp16 twins
+  // written above; the fp32 FFMA twin reads det_seqs in place, which prologue_impl allows only for fp32 features.
   {
     GemmArgs g{};
-    g.nseg = 1; g.seg[0] = {c->det_seqs, F, c->Fp, F, &c->ds_b};
+    g.nseg = 1; g.seg[0] = {reinterpret_cast<const float*>(det_seqs), F, c->Fp, F, &c->ds_b};
     g.w = c->Wva; g.ldw = c->Fp; g.wb = &c->Wva_b;
     g.c = c->P; g.ldc = c->NVA; g.M = b * L * R; g.N = c->NVA;
     g.row_skip = c->p_compact ? c->comp_valid : c->seq_valid;     // compact: the tiles past the last valid row are skipped
@@ -383,9 +400,16 @@ int run_prologue(Ctx* c, const float* det, int64_t det_stride, cudaStream_t st) 
   return VSR_OK;
 }
 
+int run_prologue(Ctx* c, const void* det, int64_t det_stride, cudaStream_t st) {
+  return with_feat_type(c->feat_dtype, [&](auto t) {
+    return run_prologue_t(c, static_cast<const decltype(t)*>(det), det_stride, st);
+  });
+}
+
 // Index form (vsr_prologue_indexed): projections per DETECTION row + one per image mean row; slot tiles are
 // never materialised.
-int run_prologue_indexed(Ctx* c, const float* det, int64_t det_stride, cudaStream_t st) {
+template <typename T>
+static int run_prologue_indexed_t(Ctx* c, const T* det, int64_t det_stride, cudaStream_t st) {
   PhaseScope ps(c, PH_PROLOGUE, st);
   const int F = c->F, D = c->D, b = c->b, L = c->L, R = c->R;
   const int n_img = c->n_img;
@@ -421,8 +445,9 @@ int run_prologue_indexed(Ctx* c, const float* det, int64_t det_stride, cudaStrea
   }
   {  // P per detection row, and per image mean row
     GemmArgs g{};
-    // the fp32 FFMA twin reads the detections in place; their rows are contiguous only when images are dense
-    g.nseg = 1; g.seg[0] = {det, F, c->Fp, F, &c->ds_b};
+    // the fp32 FFMA twin reads the detections in place (fp32 features only); their rows are contiguous only when
+    // images are dense
+    g.nseg = 1; g.seg[0] = {reinterpret_cast<const float*>(det), F, c->Fp, F, &c->ds_b};
     g.w = c->Wva; g.ldw = c->Fp; g.wb = &c->Wva_b;
     g.c = c->P; g.ldc = c->NVA; g.M = rows; g.N = c->NVA;
     g.row_skip = c->det_valid;
@@ -435,6 +460,12 @@ int run_prologue_indexed(Ctx* c, const float* det, int64_t det_stride, cudaStrea
     c->launches += 2;
   }
   return VSR_OK;
+}
+
+int run_prologue_indexed(Ctx* c, const void* det, int64_t det_stride, cudaStream_t st) {
+  return with_feat_type(c->feat_dtype, [&](auto t) {
+    return run_prologue_indexed_t(c, static_cast<const decltype(t)*>(det), det_stride, st);
+  });
 }
 
 }  // namespace vsr

@@ -9,6 +9,7 @@
 
 #include <cstdlib>
 #include <cstring>
+#include <type_traits>
 #include "common.cuh"
 #include "vocab_head.cuh"
 
@@ -101,10 +102,12 @@ constexpr int ATT_THREADS = 256;
 constexpr int ATT_MAX_R = 64;
 
 struct AttendArgs {
-  const float* det_seqs;   // (b, L, R, F) materialised slot tiles, or null in index form
+  // caller features det_seqs / det: element type feat_dtype (VSR_DT_F32 / F16 / BF16), the Elem of k_attend<Elem>
+  const void* det_seqs;    // (b, L, R, F) materialised slot tiles, or null in index form
   const float* P;          // materialised: [b*L*R][ldP]; index form: [n_img*D][ldP] (per detection row)
-  // index form (vsr_prologue_indexed): region = det[img][idx] (idx >= 0) or the image mean row (idx == -2)
-  const int32_t* slot_index; const float* det; int64_t det_stride; int D;
+  // index form (vsr_prologue_indexed): region = det[img][idx] (idx >= 0) or the image mean row (idx == -2, fp32
+  // whatever Elem is: the mean is computed in fp32 by k_pool)
+  const int32_t* slot_index; const void* det; int64_t det_stride; int D;
   const float* img; int ld_img; const float* Pmean; int img_mul;
   const unsigned long long* slot_mask;  // [b*L] validity bits of each slot tile
   const int32_t* slot_base;             // [b*L] first P row of the slot when only valid rows were projected, or null
@@ -119,9 +122,12 @@ struct AttendArgs {
   // column r+1 = region r of the slot it reads ([rows][R+1]), and that slot ([rows])
   float* alpha_out; int32_t* slot_out;
   int rows, cur_beam, L, R, F, A, H, ldP;
+  int feat_dtype;
 };
 
+template <typename Elem>
 __global__ void __launch_bounds__(ATT_THREADS) k_attend(const AttendArgs a) {
+  constexpr bool f32 = std::is_same<Elem, float>::value;
   extern __shared__ __align__(16) float sm[];
   float* ha = sm;                       // [A]
   float* Ps = ha + a.A;                 // [R][A] att_va projections of the slot's valid regions (cp.async)
@@ -131,7 +137,9 @@ __global__ void __launch_bounds__(ATT_THREADS) k_attend(const AttendArgs a) {
   __shared__ int s_rows[ATT_MAX_R];     // compacted valid region rows and their weights
   __shared__ float s_w[ATT_MAX_R];
   __shared__ int s_nv;
-  __shared__ const float* s_feat[ATT_MAX_R];   // feature row of every region of the slot
+  __shared__ const void* s_feat[ATT_MAX_R];    // feature row of every region of the slot
+  // half-precision features: 1 = the row is fp32 (the index form's image mean row), 0 = a row of Elem
+  __shared__ uint8_t s_row_f32[f32 ? 1 : ATT_MAX_R];
 
   const int n = blockIdx.x;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -184,27 +192,40 @@ __global__ void __launch_bounds__(ATT_THREADS) k_attend(const AttendArgs a) {
   for (int r = warp; r < a.R; r += nwarp) {
     if (!((vmask >> r) & 1ull)) continue;
     const float* prow;
-    const float* frow;
+    const void* frow;
+    bool row_f32 = f32;
     if (a.slot_index == nullptr) {
       prow = a.P + (pbase >= 0 ? (size_t)(pbase + __popcll(vmask & ((1ull << r) - 1ull))) : tile_row0 + r) * a.ldP;
-      frow = a.det_seqs + (tile_row0 + r) * a.F;
+      frow = static_cast<const Elem*>(a.det_seqs) + (tile_row0 + r) * a.F;
     } else {
       const int idx = a.slot_index[tile_row0 + r];
       if (idx >= 0) {
         prow = a.P + ((size_t)imgi * a.D + idx) * a.ldP;
-        frow = a.det + (size_t)imgi * a.det_stride + (size_t)idx * a.F;
+        frow = static_cast<const Elem*>(a.det) + (size_t)imgi * a.det_stride + (size_t)idx * a.F;
       } else {
         prow = a.Pmean + (size_t)imgi * a.ldP;
         frow = a.img + (size_t)imgi * a.ld_img;
+        row_f32 = true;
       }
     }
-    if (lane == 0) s_feat[r] = frow;
+    if (lane == 0) {
+      s_feat[r] = frow;
+      if constexpr (!f32) s_row_f32[r] = row_f32 ? 1 : 0;
+    }
     float* pdst = Ps + (size_t)r * a.A;
     for (int ch = lane * 4; ch < a.A; ch += 128) {
       const unsigned dst = (unsigned)__cvta_generic_to_shared(pdst + ch);
       asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(prow + ch) : "memory");
     }
-    for (int f = lane * 32; f < a.F; f += 32 * 32) asm volatile("prefetch.global.L2 [%0];" ::"l"(frow + f));
+    // one 128-byte line per lane: the row is F * sizeof(element) bytes
+    if constexpr (f32) {
+      for (int f = lane * 32; f < a.F; f += 32 * 32)
+        asm volatile("prefetch.global.L2 [%0];" ::"l"(static_cast<const float*>(frow) + f));
+    } else {
+      const int bytes = a.F * (row_f32 ? (int)sizeof(float) : (int)sizeof(Elem));
+      for (int o = lane * 128; o < bytes; o += 32 * 128)
+        asm volatile("prefetch.global.L2 [%0];" ::"l"(static_cast<const char*>(frow) + o));
+    }
   }
   asm volatile("cp.async.commit_group;" ::: "memory");
 #pragma unroll
@@ -338,9 +359,16 @@ __global__ void __launch_bounds__(ATT_THREADS) k_attend(const AttendArgs a) {
       float4 v0[4], v1[4];
 #pragma unroll
       for (int u = 0; u < 4; ++u) {
-        const float* rp = s_feat[s_rows[min(i + u, nv - 1)]];
-        v0[u] = __ldg(reinterpret_cast<const float4*>(rp + f0));
-        v1[u] = two ? __ldg(reinterpret_cast<const float4*>(rp + f1)) : make_float4(0.f, 0.f, 0.f, 0.f);
+        const int row = s_rows[min(i + u, nv - 1)];
+        if (f32 || s_row_f32[row]) {
+          const float* rp = static_cast<const float*>(s_feat[row]);
+          v0[u] = __ldg(reinterpret_cast<const float4*>(rp + f0));
+          v1[u] = two ? __ldg(reinterpret_cast<const float4*>(rp + f1)) : make_float4(0.f, 0.f, 0.f, 0.f);
+        } else {
+          const Elem* rp = static_cast<const Elem*>(s_feat[row]);
+          v0[u] = ldg_feat4(rp + f0);
+          v1[u] = two ? ldg_feat4(rp + f1) : make_float4(0.f, 0.f, 0.f, 0.f);
+        }
       }
 #pragma unroll
       for (int u = 0; u < 4; ++u) {
@@ -782,7 +810,7 @@ int run_step(Ctx* c, const StepIO& io, cudaStream_t st) {
   {
     PhaseScope ps(c, PH_ATTEND, st);
     AttendArgs a{};
-    a.det_seqs = c->det_seqs; a.P = c->P; a.slot_mask = c->slot_mask; a.ptr = c->ptr;
+    a.det_seqs = c->det_seqs; a.feat_dtype = c->feat_dtype; a.P = c->P; a.slot_mask = c->slot_mask; a.ptr = c->ptr;
     a.slot_base = c->p_compact ? c->slot_base : nullptr;
     a.slot_index = c->slot_index; a.det = c->det; a.det_stride = c->det_stride; a.D = c->D;
     a.img = c->img; a.ld_img = c->Fp; a.Pmean = c->Pmean; a.img_mul = (c->n_img == 1 ? 0 : 1);
@@ -794,12 +822,14 @@ int run_step(Ctx* c, const StepIO& io, cudaStream_t st) {
     a.ldP = c->NVA;
     a.alpha_out = io.attn_alpha; a.slot_out = io.attn_slot;
     const size_t smem = sizeof(float) * ((size_t)c->A + (size_t)c->R * c->A + c->R + 1);
+    void (*const kern[3])(const AttendArgs) = {k_attend<float>, k_attend<__half>, k_attend<__nv_bfloat16>};
     if (!c->attend_attr_set) {     // per device, hence per handle
-      VSR_CHECK_CUDA(cudaFuncSetAttribute(k_attend, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+      for (auto k : kern) VSR_CHECK_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
       c->attend_attr_set = true;
     }
     VSR_REQUIRE(smem <= 200 * 1024, VSR_EINVAL, "attention tile (R=%d x A=%d) does not fit shared memory", c->R, c->A);
-    VSR_CHECK_CUDA(launch_k(k_attend, dim3(rows), dim3(ATT_THREADS), smem, st, c->use_pdl && (c->pdl_mode & 2), a));
+    const int ki = c->feat_dtype == VSR_DT_F16 ? 1 : c->feat_dtype == VSR_DT_BF16 ? 2 : 0;
+    VSR_CHECK_CUDA(launch_k(kern[ki], dim3(rows), dim3(ATT_THREADS), smem, st, c->use_pdl && (c->pdl_mode & 2), a));
     VSR_CHECK_CUDA(cudaGetLastError()); c->launches++;
   }
   {  // D: pre2 = WD . [att | h2_old | h1'] + b (+ U2[img]);  C: ga = att_ga . g_t rides in the same launch

@@ -11,6 +11,11 @@ Every driver takes `return_attention=False`.  When True the usual return value g
 slot read at that step) and `slot` (int64, the token outputs' shape: that slot).  The weights are the ones that form the
 attended feature (0 at padding regions), untouched by verb forcing and not masked after a caption's EOS.  For beam search
 they follow each returned beam's back-pointer path, unlike the log-probs, which are in slot order as in the reference.
+
+Every driver (`beam_search`, `beam_search_v`, `beam_search_v_indexed`, `forward`, `test`, `sample_rl`, and `step` /
+`step_v` of the sub-class) takes region features in float32, float16 or bfloat16, one dtype for the detections and the
+slot tiles.  The kernels widen half-precision values to fp32 as they load them, so every output is bit-identical to that
+of the same call on the features' float32 upcast; only the bytes read and copied halve.
 """
 import torch
 from torch import nn

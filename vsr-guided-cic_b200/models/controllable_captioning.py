@@ -4,7 +4,9 @@ Keeps the reference's class surface (models/controllable_captioning.py:10-303): 
 signature, the 28-tensor state_dict (same names, shapes, dtypes, registration order),
 `init_state`, `step`, `step_v`, `test`, `sample_rl`, and the inherited `forward` /
 `beam_search` / `beam_search_v`.  Every decode driver also returns the per-word attention on request
-(`return_attention=True`, see models/CaptioningModel.py), which the reference only exposes as a local of `step_v`.  The parameters live in ordinary torch modules so that
+(`return_attention=True`, see models/CaptioningModel.py), which the reference only exposes as a local of `step_v`.
+Region features (detections, det_seqs / ctrl_det_seqs) may be float16 or bfloat16 as well as float32: a decode of
+half-precision features is bit-identical to the decode of their float32 upcast, and reads half the bytes.  The parameters live in ordinary torch modules so that
 `.to()`, `.eval()`, `load_state_dict()` work unchanged; all arithmetic of the hot path runs in
 libvsrdec's sm_100a kernels on a packed copy of the weights that is rebuilt whenever the
 parameters change.  CPU tensors raise: this path has no fallback.
@@ -17,7 +19,10 @@ LIMITS the reference does not have (each raises VsrError with a message, never a
   * seq_len <= 256 for beam search (back-track kernel's shared-memory history);
   * tensor-core operands are carried as fp16 (+ fp16 / e4m3 residuals): weights are rescaled per tensor by a power of
     two, activations are not — hidden states are in [-1, 1] by construction, region features must stay below 255 in
-    magnitude in the default "f16+f8x2" GEMM mode (65504 with VSRDEC_GEMM=f16x3); larger values saturate.
+    magnitude in the default "f16+f8x2" GEMM mode (65504 with VSRDEC_GEMM=f16x3); larger values saturate.  The bound is
+    on the activation scale, not the input format: it is the same for float32, float16 and bfloat16 features;
+  * region features are float32, float16 or bfloat16, one dtype for the detections and the slot tiles (a mismatch or
+    any other dtype raises); half precision is refused under VSRDEC_GEMM=simt (the fp32 FFMA verification twin).
 Among candidates whose fp32 scores tie EXACTLY the order is (score desc, flat index asc); torch.sort leaves it unspecified.
 """
 import json

@@ -39,6 +39,9 @@ EXPORTED_SYMBOLS = {
                                           ctypes.POINTER(c_i32), c_i32]),
     "vsr_prologue": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i32, c_vp, c_i32, c_i32, c_i32, c_vp, c_i32, c_vp]),
     "vsr_prologue_indexed": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i32, c_vp, c_i32, c_i32, c_i32, c_vp, c_i32, c_vp]),
+    "vsr_prologue_ex": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i32, c_vp, c_i32, c_i32, c_i32, c_i32, c_vp, c_i32, c_vp]),
+    "vsr_prologue_indexed_ex": (ctypes.c_int, [c_vp, c_vp, c_i64, c_i32, c_vp, c_i32, c_i32, c_i32, c_i32, c_vp, c_i32,
+                                               c_vp]),
     "vsr_step": (ctypes.c_int, [c_vp] + [c_vp] * 6 + [c_i32, c_i32] + [c_vp] * 6 + [c_vp]),
     "vsr_beam_search": (ctypes.c_int, [c_vp, c_i32, c_i32, ctypes.POINTER(c_i64), c_i32, c_i32,
                                        c_vp, c_vp, c_vp, c_vp, ctypes.POINTER(VsrTrace), c_vp]),

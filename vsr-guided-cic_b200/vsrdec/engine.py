@@ -21,10 +21,24 @@ PARAM_NAMES = (
     "W1_hg.weight", "W1_hg.bias", "att_ga.weight", "att_g.weight")
 
 _VERB_DT = {torch.float64: 0, torch.float32: 1, torch.int64: 2}
+# element types of the region features (VSR_DT_F32 / F16 / BF16): a half-precision decode is bit-identical to the
+# decode of its fp32 upcast (the kernels widen every value as they load it)
+_FEAT_DT = {torch.float32: 1, torch.float16: 3, torch.bfloat16: 4}
 
 
 def _stream_ptr(device) -> int:
     return torch.cuda.current_stream(device).cuda_stream
+
+
+def _feat_dtype(*feats):
+    """dtype tag of the feature tensors, which must share one of float32 / float16 / bfloat16."""
+    dt = feats[0][0].dtype
+    for t, name in feats:
+        if t.dtype not in _FEAT_DT:
+            raise VsrError(f"{name} must be torch.float32, torch.float16 or torch.bfloat16, got {t.dtype}")
+        if t.dtype != dt:
+            raise VsrError(f"detections and det_seqs must share one dtype, got {dt} and {t.dtype}")
+    return _FEAT_DT[dt]
 
 
 def _req_cuda(t: torch.Tensor, name: str, dtype=None):
@@ -107,8 +121,10 @@ class DecoderEngine:
 
     # ------------------------------------------------------------------ prologue
     def prologue(self, det: torch.Tensor, det_seqs: torch.Tensor, verbs: Optional[torch.Tensor] = None):
-        _req_cuda(det, "detections", torch.float32)
-        _req_cuda(det_seqs, "det_seqs", torch.float32)
+        """det (b, D, F) and det_seqs (b, L, R, F) in one of float32 / float16 / bfloat16."""
+        _req_cuda(det, "detections")
+        _req_cuda(det_seqs, "det_seqs")
+        fdt = _feat_dtype((det, "detections"), (det_seqs, "det_seqs"))
         if det.dim() != 3 or det_seqs.dim() != 4 or det.size(0) != det_seqs.size(0):
             raise VsrError(f"bad static shapes {tuple(det.shape)} / {tuple(det_seqs.shape)}")
         F = self.dims["det_feat_size"]
@@ -133,14 +149,16 @@ class DecoderEngine:
         self._keep = (det_k, ds, vb)
         self.b, self.L, self.R = b, ds.size(1), ds.size(2)
         with torch.cuda.device(self.device):
-            _lib.check(self.lib, self.lib.vsr_prologue(
-                self.handle, det_k.data_ptr(), stride, D, ds.data_ptr(), b, self.L, self.R,
+            _lib.check(self.lib, self.lib.vsr_prologue_ex(
+                self.handle, det_k.data_ptr(), stride, D, ds.data_ptr(), b, self.L, self.R, fdt,
                 vb.data_ptr() if vb is not None else None, vdt, _stream_ptr(self.device)))
 
     def prologue_indexed(self, det: torch.Tensor, slot_index: torch.Tensor, verbs: Optional[torch.Tensor] = None):
         """Index form of the prologue (vsr_prologue_indexed): slot_index (b, L, R) holds, per region, a
-        detection row of the caption's image (>= 0), -2 for the image's mean row, or -1 for padding."""
-        _req_cuda(det, "detections", torch.float32)
+        detection row of the caption's image (>= 0), -2 for the image's mean row, or -1 for padding.  det is
+        float32, float16 or bfloat16; the mean rows are computed and read in fp32 whatever its dtype."""
+        _req_cuda(det, "detections")
+        fdt = _feat_dtype((det, "detections"))
         _req_cuda(slot_index, "slot_index")
         if det.dim() != 3 or slot_index.dim() != 3 or det.size(0) != slot_index.size(0):
             raise VsrError(f"bad static shapes {tuple(det.shape)} / {tuple(slot_index.shape)}")
@@ -166,8 +184,8 @@ class DecoderEngine:
         self._keep = (det_k, idx, vb)
         self.b, self.L, self.R = b, idx.size(1), idx.size(2)
         with torch.cuda.device(self.device):
-            _lib.check(self.lib, self.lib.vsr_prologue_indexed(
-                self.handle, det_k.data_ptr(), stride, D, idx.data_ptr(), b, self.L, self.R,
+            _lib.check(self.lib, self.lib.vsr_prologue_indexed_ex(
+                self.handle, det_k.data_ptr(), stride, D, idx.data_ptr(), b, self.L, self.R, fdt,
                 vb.data_ptr() if vb is not None else None, vdt, _stream_ptr(self.device)))
 
     # ------------------------------------------------------------------ single step

@@ -197,12 +197,50 @@ int vsr_greedy(vsr_handle h, int64_t* out_words, int64_t* out_gates, void* strea
  * coco_scripts/train.py:151): at every step both heads are sampled from the step's distributions (word: Gumbel-max
  * over the vocabulary row with a Philox4x32-10 stream keyed by `seed`; gate: one uniform draw), the picks are fed
  * back, and the log-probs of the picks are returned.  The whole loop runs on the device.
- *   out_words,out_gates (b,T) int64;  lp_words,lp_gates (b,T) fp32.  The same seed reproduces the same draws. */
+ *   out_words,out_gates (b,T) int64;  lp_words,lp_gates (b,T) fp32.  The same seed reproduces the same draws.
+ * Equal to vsr_sample_ex with {seed, 1, 1.f, 0, 1.f, 0, 0}. */
 int vsr_sample(vsr_handle h, uint64_t seed, int64_t* out_words, int64_t* out_gates,
                float* lp_words, float* lp_gates, void* stream);
 
+/* Sampling decode with several draws per caption, temperature, top-k / top-p truncation and verb forcing.
+ * A call decodes the prologue's b captions with n >= 1 independent draws per caption.  Rows are caption-major:
+ * row r = caption c = r / n, draw j = r % n.  Every row starts as init_state does; statics are read by c (no copy per
+ * draw).  All T = seq_len steps run (no EOS stop).
+ * At each step an UNFORCED row with vocabulary logits x (fp32), temperature tau, top_k and top_p:
+ *   1. z_v = x_v / tau in fp32 (tau = 1 leaves x untouched).
+ *   2. The vocabulary is ordered by (x desc, index asc): on x, not z, so that division rounding creates no new ties.
+ *   3. Top-k: K = the first min(top_k, V) entries of that order; top_k = 0 means all V.
+ *   4. Top-p: q_v = exp(z_v - max z) / sum_{u in K} exp(z_u - max z) over K; P = the shortest prefix of K, in the same
+ *      order, whose mass is >= top_p.  top_p = 1 means P = K.  P always holds at least one word.
+ *   5. word = argmax_{v in P} (z_v + G_v), ties by (value desc, index asc), G_v = -log(-log u_v) with u_v from the
+ *      Philox4x32-10 counter (v >> 2, c, t, 2j), lane v & 3 (for j = 0 the numbers vsr_sample uses).  The gate is drawn
+ *      from the step's gate log-probs with counter (0, c, t, 2j + 1); temperature and truncation apply to the word
+ *      head only.
+ *   6. lp_words = the MODEL's log-prob of the draw, (x_w - row max) - row log-sum-exp, unaffected by tau, top_k and
+ *      top_p (what a scorer needs); lp_gates = the gate's log-prob, as vsr_sample returns them.
+ * With use_verbs (vsr_step's use_verbs / gt semantics, gt as in vsr_beam_search; the prologue must have a verbs tensor)
+ * a FORCED row (its current slot has a verb) takes the forced word with lp_word = 0 and gate 1 with lp_gate = 0.
+ * Draw j of caption c is bit-identical for every n > j, and does not depend on b or on the other captions.  Masses
+ * are summed in fixed point, so the top-p boundary does not depend on launch shape either.
+ *   out_words,out_gates (b,n,T) int64;  lp_words,lp_gates (b,n,T) fp32.
+ * z is clamped to +-FLT_MAX, so a tau small enough for x / tau to overflow float32 still gives a finite row: the
+ * overflowing entries tie at FLT_MAX and are resolved in index order like any other tie.
+ * VSR_EINVAL: n < 1, b * n > 2^30, tau not finite or <= 0, top_k < 0, top_p not in (0, 1], a null pointer, use_verbs
+ * without a verbs tensor. */
+typedef struct VsrSampleParams {
+  uint64_t seed;
+  int32_t n;            /* draws per caption, >= 1 */
+  float temperature;    /* finite, > 0 */
+  int32_t top_k;        /* >= 0, 0 = off */
+  float top_p;          /* (0, 1], 1 = off */
+  int32_t use_verbs;    /* step_v semantics: verb forcing (needs a prologue with verbs) */
+  int32_t gt;
+} VsrSampleParams;
+int vsr_sample_ex(vsr_handle h, const VsrSampleParams* p, int64_t* out_words, int64_t* out_gates,
+                  float* lp_words, float* lp_gates, void* stream);
+
 /* Attention capture: where the decoder looks for every generated word.
- * vsr_set_attention_capture: while enabled, the decode drivers (vsr_beam_search, vsr_greedy, vsr_sample,
+ * vsr_set_attention_capture: while enabled, the decode drivers (vsr_beam_search, vsr_greedy, vsr_sample(_ex),
  *   vsr_forward_teacher) record, at every step and for every row, the R+1 attention weights of the slot attention
  *   (controllable_captioning.py:167-169) and the slot the row read, in a grow-only workspace of [T][rows][R+1] fp32 +
  *   [T][rows] int32 (8.4 MB at 1000 captions x beam 5 x R = 20).  Off by default; when off nothing is recorded and no
@@ -211,6 +249,7 @@ int vsr_sample(vsr_handle h, uint64_t seed, int64_t* out_words, int64_t* out_gat
  *   vsr_beam_search:  alpha (b,out_size,T,R+1) fp32, slot (b,out_size,T) int32, following the back-pointer path of each
  *                     returned beam (the row whose distributions produced token t).  Note that lp_words / lp_gates are
  *                     NOT back-tracked (slot order, as in the reference), the attention is.
+ *   vsr_sample_ex:    alpha (b,n,T,R+1), slot (b,n,T): draw j of caption c is row c*n + j.
  *   other drivers:    alpha (b,T,R+1), slot (b,T): one row per caption (T = the captions' length for teacher forcing).
  *   alpha[..., 0] is the sentinel weight and alpha[..., r+1] the weight of region r of the slot read at that step; the
  *   weights are exactly the ones that form the attended feature: 0 at padding regions and at an all-zero sentinel, the

@@ -1,5 +1,6 @@
 // C-ABI entry points of libvsrdec (include/vsrdec.h): context life-cycle, workspace
 // management and the decode drivers (beam search, teacher-forced forward, greedy, single step).
+#include <math.h>
 #include <stdarg.h>
 #include <stdlib.h>
 #include <string.h>
@@ -156,24 +157,29 @@ int ensure_rows(Ctx* c, int rows) {
   return VSR_OK;
 }
 
+// per-row selection buffers (beam search: caps * VSR_MAX_BEAM slots; greedy and sampling: one per decoded row)
+int ensure_sel(Ctx* c, int rows) {
+  if (rows <= c->cap_sel) return VSR_OK;
+  int32_t** ib[] = {&c->sel_beam, &c->sel_word, &c->sel_gate, &c->sel_beam_n, &c->sel_word_n, &c->sel_gate_n};
+  for (int32_t** p : ib) { dev_free(c, *p); *p = nullptr; }
+  c->cap_sel = 0;
+  for (int32_t** p : ib) VSR_TRY(dev_alloc(c, (void**)p, sizeof(int32_t) * (size_t)rows));
+  c->cap_sel = rows;
+  return VSR_OK;
+}
+
 int ensure_beam_ws(Ctx* c, int caps, int T) {
+  VSR_TRY(ensure_sel(c, caps * VSR_MAX_BEAM));
   if (caps <= c->cap_caps && T <= c->cap_T) return VSR_OK;
   caps = std::max(caps, c->cap_caps); T = std::max(T, c->cap_T);
   float** fb[] = {&c->seq_lp, &c->seq_lp_n, &c->m0, &c->m1, &c->m0n, &c->m1n, &c->hist_score, &c->hist_lpw, &c->hist_lpg};
-  int32_t** ib[] = {&c->sel_beam, &c->sel_word, &c->sel_gate, &c->sel_beam_n, &c->sel_word_n, &c->sel_gate_n,
-                    &c->hist_parent, &c->hist_word, &c->hist_gate};
+  int32_t** ib[] = {&c->hist_parent, &c->hist_word, &c->hist_gate};
   for (float** p : fb) { dev_free(c, *p); *p = nullptr; }
   for (int32_t** p : ib) { dev_free(c, *p); *p = nullptr; }
   c->cap_caps = 0; c->cap_T = 0;
   const size_t s = (size_t)caps * VSR_MAX_BEAM, hs = s * T;
   ALLOC_F(c->seq_lp, s); ALLOC_F(c->seq_lp_n, s); ALLOC_F(c->m0, s); ALLOC_F(c->m1, s); ALLOC_F(c->m0n, s); ALLOC_F(c->m1n, s);
   ALLOC_F(c->hist_score, hs); ALLOC_F(c->hist_lpw, hs); ALLOC_F(c->hist_lpg, hs);
-  VSR_TRY(dev_alloc(c, (void**)&c->sel_beam, sizeof(int32_t) * s));
-  VSR_TRY(dev_alloc(c, (void**)&c->sel_word, sizeof(int32_t) * s));
-  VSR_TRY(dev_alloc(c, (void**)&c->sel_gate, sizeof(int32_t) * s));
-  VSR_TRY(dev_alloc(c, (void**)&c->sel_beam_n, sizeof(int32_t) * s));
-  VSR_TRY(dev_alloc(c, (void**)&c->sel_word_n, sizeof(int32_t) * s));
-  VSR_TRY(dev_alloc(c, (void**)&c->sel_gate_n, sizeof(int32_t) * s));
   VSR_TRY(dev_alloc(c, (void**)&c->hist_parent, sizeof(int32_t) * hs));
   VSR_TRY(dev_alloc(c, (void**)&c->hist_word, sizeof(int32_t) * hs));
   VSR_TRY(dev_alloc(c, (void**)&c->hist_gate, sizeof(int32_t) * hs));
@@ -673,26 +679,38 @@ static int greedy_impl(Ctx* c, int64_t* out_words, int64_t* out_gates, cudaStrea
   return VSR_OK;
 }
 
-// multinomial sampling decode: the whole loop on the device, one pick kernel per step, no host work in between
-static int sample_impl(Ctx* c, uint64_t seed, int64_t* out_words, int64_t* out_gates, float* lp_words, float* lp_gates,
-                       cudaStream_t st) {
+// multinomial sampling decode: the whole loop on the device, one pick kernel per step, no host work in between.
+// p.n draws per caption run as rows = b * p.n with cur_beam = p.n: every row starts from init_state, statics are read by
+// caption = row / p.n, and the draws of a row depend on (seed, caption, draw, step) only (vsr_sample_ex in vsrdec.h).
+static int sample_impl(Ctx* c, const VsrSampleParams& p, int64_t* out_words, int64_t* out_gates, float* lp_words,
+                       float* lp_gates, cudaStream_t st) {
   VSR_REQUIRE(c->have_prologue, VSR_ESTATE, "vsr_sample: call vsr_prologue first");
   VSR_REQUIRE(out_words && out_gates && lp_words && lp_gates, VSR_EINVAL, "vsr_sample: null argument");
+  VSR_REQUIRE(p.n >= 1, VSR_EINVAL, "vsr_sample_ex: n=%d draws per caption, must be >= 1", p.n);
+  VSR_REQUIRE(isfinite(p.temperature) && p.temperature > 0.f, VSR_EINVAL,
+              "vsr_sample_ex: temperature=%g must be finite and > 0", (double)p.temperature);
+  VSR_REQUIRE(p.top_k >= 0, VSR_EINVAL, "vsr_sample_ex: top_k=%d must be >= 0 (0 = off)", p.top_k);
+  VSR_REQUIRE(p.top_p > 0.f && p.top_p <= 1.f, VSR_EINVAL, "vsr_sample_ex: top_p=%g not in (0, 1]", (double)p.top_p);
+  VSR_REQUIRE(!p.use_verbs || c->verbs != nullptr, VSR_EINVAL, "vsr_sample_ex: use_verbs without a verbs tensor");
   const int b = c->b, T = c->d.seq_len;
-  VSR_TRY(ensure_rows(c, b));
-  VSR_TRY(ensure_beam_ws(c, b, T));
-  VSR_TRY(attn_begin(c, b, T, 0));
-  VSR_TRY(launch_state_init(c, b, st));
+  VSR_REQUIRE((int64_t)b * p.n <= (int64_t)1 << 30, VSR_EINVAL, "vsr_sample_ex: b*n = %lld rows > 2^30 unsupported",
+              (long long)b * p.n);
+  const int rows = b * p.n;
+  VSR_TRY(ensure_rows(c, rows));
+  VSR_TRY(ensure_sel(c, rows));
+  VSR_TRY(attn_begin(c, rows, T, 0));
+  VSR_TRY(launch_state_init(c, rows, st));
   for (int t = 0; t < T; ++t) {
     StepIO io{};
-    io.rows = b; io.cur_beam = 1; io.use_verbs = false; io.gt = false; io.topk = 0;     // statistics + gate head only
+    io.rows = rows; io.cur_beam = p.n; io.use_verbs = p.use_verbs != 0; io.gt = p.gt != 0;
+    io.topk = 0;     // statistics + gate head (+ forced word) only
     io.zero_state = t == 0 && c->zero_state_opt;
-    attn_step_io(c, io, t, b);
+    attn_step_io(c, io, t, rows);
     VSR_TRY(run_step(c, io, st));
-    VSR_TRY(launch_sample_pick(c, b, t, T, seed, out_words, out_gates, lp_words, lp_gates, st));
-    if (t + 1 < T) VSR_TRY(launch_commit_identity(c, b, nullptr, 0, -1, st));
+    VSR_TRY(launch_sample_pick(c, rows, t, T, p, out_words, out_gates, lp_words, lp_gates, st));
+    if (t + 1 < T) VSR_TRY(launch_commit_identity(c, rows, nullptr, 0, -1, st));
   }
-  attn_done(c, false, T, b, b);
+  attn_done(c, false, T, rows, rows);
   return VSR_OK;
 }
 
@@ -865,11 +883,17 @@ int vsr_greedy(vsr_handle h, int64_t* out_words, int64_t* out_gates, void* strea
   return vsr::greedy_impl((Ctx*)h, out_words, out_gates, (cudaStream_t)stream);
 }
 
+int vsr_sample_ex(vsr_handle h, const VsrSampleParams* p, int64_t* out_words, int64_t* out_gates, float* lp_words,
+                  float* lp_gates, void* stream) {
+  if (!h || !p) { vsr::set_error("vsr_sample_ex: null argument"); return VSR_EINVAL; }
+  DeviceGuard dg((const vsr::Ctx*)h);
+  return vsr::sample_impl((Ctx*)h, *p, out_words, out_gates, lp_words, lp_gates, (cudaStream_t)stream);
+}
+
 int vsr_sample(vsr_handle h, uint64_t seed, int64_t* out_words, int64_t* out_gates, float* lp_words, float* lp_gates,
                void* stream) {
-  if (!h) { vsr::set_error("vsr_sample: null handle"); return VSR_EINVAL; }
-  DeviceGuard dg((const vsr::Ctx*)h);
-  return vsr::sample_impl((Ctx*)h, seed, out_words, out_gates, lp_words, lp_gates, (cudaStream_t)stream);
+  const VsrSampleParams p = {seed, 1, 1.f, 0, 1.f, 0, 0};
+  return vsr_sample_ex(h, &p, out_words, out_gates, lp_words, lp_gates, stream);
 }
 
 int64_t vsr_launch_count(vsr_handle h) { return h ? ((Ctx*)h)->launches : -1; }

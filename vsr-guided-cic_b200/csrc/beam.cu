@@ -4,18 +4,18 @@
 // Reference: models/CaptioningModel.py:116-195 (beam_search), :197-294 (beam_search_v),
 // :78-114 (_select_beam).  Statics are never copied per beam (SURVEY.md §2.1 k15): rows index
 // them by caption = row / beam.
+#include <cooperative_groups.h>
+#include <cooperative_groups/reduce.h>
 #include <cuda_fp16.h>
+#include <float.h>
 #include <math.h>
 
 #include "common.cuh"
+#include "vocab_head.cuh"
 
 namespace vsr {
 
 namespace {
-
-__device__ __forceinline__ bool before(float v1, int i1, float v2, int i2) {
-  return v1 > v2 || (v1 == v2 && i1 < i2);
-}
 
 // log-prob of vocabulary entry `word` in row `row` as returned by the step (post verb forcing)
 __device__ __forceinline__ float row_logp(const float* logits, int ld, const float* row_max,
@@ -248,7 +248,8 @@ __global__ void k_greedy_pick(const int32_t* cand, const float* gate_lp, int32_t
 }
 
 // ---------------------------------------------------------------- multinomial sampling (CaptioningModel.sample_rl)
-// Philox4x32-10 counter-based generator: the draw of (seed, row, step, vocabulary entry) never depends on launch shape.
+// Philox4x32-10 counter-based generator: the draw of (seed, caption, step, draw, vocabulary entry) never depends on
+// launch shape.
 __device__ __forceinline__ uint4 philox4x32_10(uint4 ctr, uint2 key) {
 #pragma unroll
   for (int r = 0; r < 10; ++r) {
@@ -261,51 +262,249 @@ __device__ __forceinline__ uint4 philox4x32_10(uint4 ctr, uint2 key) {
 }
 __device__ __forceinline__ float u01(unsigned x) { return ((float)(x >> 8) + 0.5f) * (1.f / 16777216.f); }   // (0, 1)
 
-// One CTA per row: word ~ Categorical(softmax(logits)) by the Gumbel-max trick (argmax of logit + G, G = -log(-log u),
-// which draws index v with probability exp(logit_v) / sum exp), gate ~ Categorical(exp(gate_lp)); log-probs of the
-// draws as torch.distributions.Categorical(logits=out).log_prob(sample) returns them (CaptioningModel.py:66-70).
-__global__ void __launch_bounds__(256) k_sample_pick(const float* __restrict__ logits, int ld, int V, const float* __restrict__ row_max,
-                                                     const float* __restrict__ row_lsum, const float* __restrict__ gate_lp,
-                                                     unsigned long long seed, int t, int T, int32_t* sel_word, int32_t* sel_gate,
-                                                     int64_t* out_words, int64_t* out_gates, float* lp_words, float* lp_gates) {
-  __shared__ float s_v[8];
-  __shared__ int s_i[8];
+struct SampleArgs {
+  const float* logits; int ld, V;
+  const float* row_max; const float* row_lsum; const float* gate_lp;
+  const int32_t* forced;          // [rows] forced word or -1 (verb forcing), or null
+  unsigned long long seed;
+  int t, T, n;                    // step, steps, draws per caption (row = caption * n + draw)
+  float tau; int top_k; float top_p;
+  int32_t *sel_word, *sel_gate;
+  int64_t *out_words, *out_gates; float *lp_words, *lp_gates;
+};
+
+constexpr int SP_THREADS = 256;
+// masses of the top-p select as fixed point (x 2^47): integer sums are exact, so the shared-memory histograms and the
+// totals do not depend on the order the atomics land in, and a draw depends on (seed, caption, draw, step, row) alone
+constexpr float SP_FIX = 140737488355328.f;   // 2^47; a row of <= 49152 masses <= 1 sums below 2^63
+
+// z = x / tau (x itself at tau = 1), kept finite: at a tiny tau the quotient would overflow to inf and z - max z to NaN
+__device__ __forceinline__ float sp_z(float x, float tau) {
+  return tau == 1.f ? x : fminf(fmaxf(__fdiv_rn(x, tau), -FLT_MAX), FLT_MAX);
+}
+
+// the vocabulary entry of this row whose key is `key`, at 1-based rank r (1 <= r <= number of such entries) among the
+// entries of that key in index order.  Tiles of SP_THREADS consecutive entries (conflict-free shared loads), a ballot
+// per warp and one barrier per tile; stops at the tile that holds the entry.
+__device__ int sp_nth_tie(const float* s_x, int V, unsigned key, unsigned r, unsigned (*s_cnt)[SP_THREADS / 32],
+                          int* s_res) {
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  if (tid == 0) *s_res = V - 1;
+  unsigned base = 0;
+  for (int v0 = 0, it = 0; v0 < V; v0 += SP_THREADS, ++it) {
+    const int v = v0 + tid;
+    const bool hit = v < V && orderable(s_x[v]) == key;
+    const unsigned bal = __ballot_sync(0xffffffffu, hit);
+    if (lane == 0) s_cnt[it & 1][warp] = __popc(bal);
+    __syncthreads();           // (double-buffered counts: the next tile's writes follow this barrier)
+    unsigned before_warp = 0, tile = 0;
+#pragma unroll
+    for (int w = 0; w < SP_THREADS / 32; ++w) {
+      const unsigned cw = s_cnt[it & 1][w];
+      before_warp += w < warp ? cw : 0u;
+      tile += cw;
+    }
+    if (hit && base + before_warp + __popc(bal & ((1u << lane) - 1u)) + 1u == r) *s_res = v;
+    base += tile;
+    if (base >= r) break;      // block-uniform
+  }
+  __syncthreads();
+  const int res = *s_res;
+  __syncthreads();
+  return res;
+}
+
+// hist[bin] += val, summed first over the active lanes of the warp that hit the same bin: logits of one row share
+// their high key bits, so plain per-lane atomics would serialise on one or two bins.  Integer sums: exact in any order.
+template <typename T>
+__device__ __forceinline__ void sp_hist_add(T* hist, unsigned bin, T val) {
+  namespace cg = cooperative_groups;
+  const cg::coalesced_group g = cg::labeled_partition(cg::coalesced_threads(), bin);
+  const T sum = cg::reduce(g, val, cg::plus<T>());
+  if (g.thread_rank() == 0) atomicAdd(&hist[bin], sum);
+}
+
+// Warp 0 walks a 256-bin histogram from the highest digit down and finds the bin in which the running total reaches
+// `need` (1 <= need <= total).  Returns the digit; `need` becomes what is still needed inside that bin.
+template <typename T>
+__device__ __forceinline__ int sp_pick_digit(const T* hist, T& need) {
+  const int lane = threadIdx.x & 31;
+  T part = 0;
+#pragma unroll
+  for (int i = 0; i < 8; ++i) part += hist[255 - (lane * 8 + i)];
+  T incl = part;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) { const T y = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += y; }
+  const T excl = incl - part;
+  const unsigned hit = __ballot_sync(0xffffffffu, excl < need && need <= incl);
+  const int src = __ffs(hit) - 1;
+  int digit = 0;
+  T left = need - excl;
+  if (lane == src) {
+    for (int i = 0; i < 8; ++i) {
+      const T h = hist[255 - (lane * 8 + i)];
+      if (left <= h) { digit = 255 - (lane * 8 + i); break; }
+      left -= h;
+    }
+  }
+  digit = __shfl_sync(0xffffffffu, digit, src);
+  need = __shfl_sync(0xffffffffu, left, src);
+  return digit;
+}
+
+// Truncated draws: stage row n in s_x and find the (key, index) bound of P.  K (top-k) and P (top-p) are prefixes of
+// the order (x desc, index asc), found without sorting: radix selects on orderable(x) in 8-bit digits, 256-bin
+// histograms of counts (K) and of exp masses (P), the entries of the boundary value taken in index order.
+__device__ void sp_bounds(const SampleArgs& a, int n, const float* x, float* s_x, unsigned& pkey, int& pidx) {
+  __shared__ unsigned s_hc[256], s_cnt[2][SP_THREADS / 32];
+  __shared__ unsigned long long s_hm[256], s_need;
+  __shared__ int s_res;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, V = a.V;
+  const float tau = a.tau;
+  for (int v = tid * 4; v < V; v += SP_THREADS * 4)
+    *reinterpret_cast<float4*>(s_x + v) = *reinterpret_cast<const float4*>(x + v);   // rows are padded to 4 columns
+  __syncthreads();
+  // ---- K: the first min(top_k, V) entries
+  if (a.top_k > 0 && a.top_k < V) {
+    unsigned need = (unsigned)a.top_k, prefix = 0u;
+    for (int shift = 24; shift >= 0; shift -= 8) {
+      const unsigned hmask = shift == 24 ? 0u : 0xffffffffu << (shift + 8);
+      s_hc[tid] = 0u;
+      __syncthreads();
+      for (int v = tid; v < V; v += SP_THREADS) {
+        const unsigned k = orderable(s_x[v]);
+        if ((k & hmask) == prefix) sp_hist_add(s_hc, (k >> shift) & 255u, 1u);
+      }
+      __syncthreads();
+      if (warp == 0) {
+        const int d = sp_pick_digit(s_hc, need);
+        if (lane == 0) { s_cnt[0][0] = prefix | ((unsigned)d << shift); s_cnt[0][1] = need; }
+      }
+      __syncthreads();
+      prefix = s_cnt[0][0]; need = s_cnt[0][1];
+      __syncthreads();
+    }
+    pkey = prefix;
+    pidx = sp_nth_tie(s_x, V, prefix, need, s_cnt, &s_res);
+  }
+  // ---- P: the shortest prefix of K whose mass exp(z - max z) reaches top_p of K's
+  if (a.top_p < 1.f) {
+    const unsigned kkey = pkey; const int kidx = pidx;
+    const float zmax = sp_z(a.row_max[n], tau);
+    auto mass = [&](float xv) { return (unsigned long long)__float2ull_rz(expf(sp_z(xv, tau) - zmax) * SP_FIX); };
+    unsigned long long need = 0ull;
+    unsigned pre = 0u;
+    for (int shift = 24; shift >= 0; shift -= 8) {
+      const unsigned hmask = shift == 24 ? 0u : 0xffffffffu << (shift + 8);
+      s_hm[tid] = 0ull;
+      __syncthreads();
+      for (int v = tid; v < V; v += SP_THREADS) {
+        const float xv = s_x[v];
+        const unsigned k = orderable(xv);
+        if ((k & hmask) == pre && (k > kkey || (k == kkey && v <= kidx))) sp_hist_add(s_hm, (k >> shift) & 255u, mass(xv));
+      }
+      __syncthreads();
+      if (warp == 0) {
+        if (shift == 24) {     // the first histogram holds all of K: need = ceil(top_p * mass(K)) >= 1 (max z has 2^47)
+          unsigned long long tot = 0ull;
+#pragma unroll
+          for (int i = 0; i < 8; ++i) tot += s_hm[lane * 8 + i];
+#pragma unroll
+          for (int o = 16; o > 0; o >>= 1) tot += __shfl_xor_sync(0xffffffffu, tot, o);
+          need = (unsigned long long)ceil((double)a.top_p * (double)tot);
+        }
+        const int d = sp_pick_digit(s_hm, need);
+        if (lane == 0) { s_cnt[0][0] = pre | ((unsigned)d << shift); s_need = need; }
+      }
+      __syncthreads();
+      pre = s_cnt[0][0]; need = s_need;
+      __syncthreads();
+    }
+    // every entry of the boundary value has the same mass: take as many of them, in index order, as `need` asks
+    const float xb = __uint_as_float((pre & 0x80000000u) ? (pre & 0x7fffffffu) : ~pre);
+    const unsigned long long mb = mass(xb);
+    pkey = pre;
+    pidx = sp_nth_tie(s_x, V, pre, (unsigned)((need + mb - 1) / mb), s_cnt, &s_res);
+  }
+}
+
+// One CTA per row: word ~ Categorical(softmax(z)), z = logits / tau, restricted to the top-k / top-p set P, by the
+// Gumbel-max trick (argmax over P of z + G, G = -log(-log u), draws v with probability exp(z_v) / sum_P exp), gate ~
+// Categorical(exp(gate_lp)); log-probs of the draws under the model's untempered distributions, as
+// torch.distributions.Categorical(logits=out).log_prob(sample) returns them (CaptioningModel.py:66-70).  A forced row
+// (verb forcing, step_v) takes its forced word and gate 1, both with log-prob 0.
+// TRUNC = false (no top-k / top-p): the row is read once from global memory (L2: the vocabulary GEMM just wrote it), with
+// no shared-memory staging or select state.  TRUNC = true: sp_bounds stages the row in dynamic shared memory and finds
+// P; v is in P when orderable(x_v) > key, or == key and v <= index.  Register bounds: 40 for the untruncated pick (6 CTAs
+// per SM, as before truncation existed), 64 for the truncated one.
+template <bool TRUNC>
+__global__ void __launch_bounds__(SP_THREADS, TRUNC ? 4 : 6) k_sample_pick(const SampleArgs a) {
+  __shared__ float s_v[SP_THREADS / 32];
+  __shared__ int s_i[SP_THREADS / 32];
   const int n = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const float* x = logits + (size_t)n * ld;
-  const uint2 key = make_uint2((unsigned)seed, (unsigned)(seed >> 32));
+  const int c = n / a.n, j = n - c * a.n, V = a.V;
+  const float* x = a.logits + (size_t)n * a.ld;
+  const uint2 key = make_uint2((unsigned)a.seed, (unsigned)(a.seed >> 32));
+  const size_t o = (size_t)n * a.T + a.t;
+  const int forced = a.forced != nullptr ? a.forced[n] : -1;
+  if (forced >= 0) {        // step_v: out = 0 at the forced word, gate = [-1e3, 0]
+    if (tid == 0) {
+      a.sel_word[n] = forced; a.sel_gate[n] = 1;
+      a.out_words[o] = forced; a.out_gates[o] = 1; a.lp_words[o] = 0.f; a.lp_gates[o] = 0.f;
+    }
+    return;
+  }
+  const float tau = a.tau;
+  const float* src = x;
+  unsigned pk = 0u; int pi = 0x7fffffff;           // bound of P
+  if constexpr (TRUNC) {
+    extern __shared__ __align__(16) float s_x[];
+    sp_bounds(a, n, x, s_x, pk, pi);
+    src = s_x;
+  }
+  // ---- draw: Gumbel-max over P, lanes of one Philox block = 4 consecutive vocabulary entries
   float bv = -INFINITY; int bi = 0x7fffffff;
-  for (int v0 = tid * 4; v0 < V; v0 += 256 * 4) {
-    const uint4 r = philox4x32_10(make_uint4((unsigned)(v0 >> 2), (unsigned)n, (unsigned)t, 0u), key);
-    const float4 q = *reinterpret_cast<const float4*>(x + v0);        // rows are padded to a multiple of 4 columns
+  for (int v0 = tid * 4; v0 < V; v0 += SP_THREADS * 4) {
+    const float4 q = *reinterpret_cast<const float4*>(src + v0);
     const float xs[4] = {q.x, q.y, q.z, q.w};
+    bool in[4];
+    bool any = false;
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+      const unsigned k = orderable(xs[e]);
+      in[e] = v0 + e < V && (!TRUNC || k > pk || (k == pk && v0 + e <= pi));
+      any |= in[e];
+    }
+    if (!any) continue;
+    const uint4 r = philox4x32_10(make_uint4((unsigned)(v0 >> 2), (unsigned)c, (unsigned)a.t, 2u * (unsigned)j), key);
     const unsigned rs[4] = {r.x, r.y, r.z, r.w};
 #pragma unroll
     for (int e = 0; e < 4; ++e) {
-      if (v0 + e >= V) break;
+      if (!in[e]) continue;
       const float g = -logf(-logf(u01(rs[e])));
-      const float sc = xs[e] + g;
+      const float sc = sp_z(xs[e], tau) + g;
       if (sc > bv) { bv = sc; bi = v0 + e; }
     }
   }
 #pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
-    const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
+  for (int off = 16; off > 0; off >>= 1) {
+    const float ov = __shfl_xor_sync(0xffffffffu, bv, off);
+    const int oi = __shfl_xor_sync(0xffffffffu, bi, off);
     if (before(ov, oi, bv, bi)) { bv = ov; bi = oi; }
   }
   if (lane == 0) { s_v[warp] = bv; s_i[warp] = bi; }
   __syncthreads();
   if (tid == 0) {
-    for (int w = 1; w < 8; ++w) if (before(s_v[w], s_i[w], bv, bi)) { bv = s_v[w]; bi = s_i[w]; }
+    for (int w = 1; w < SP_THREADS / 32; ++w) if (before(s_v[w], s_i[w], bv, bi)) { bv = s_v[w]; bi = s_i[w]; }
     const int word = bi < V ? bi : V - 1;
-    const float lw = (x[word] - row_max[n]) - row_lsum[n];
-    // gate: two categories with log-probs gate_lp[n]; counter word 1 keeps this draw apart from the vocabulary's
-    const uint4 r = philox4x32_10(make_uint4(0u, (unsigned)n, (unsigned)t, 1u), key);
-    const float g0 = gate_lp[(size_t)n * 2], g1 = gate_lp[(size_t)n * 2 + 1];
+    const float lw = (x[word] - a.row_max[n]) - a.row_lsum[n];
+    // gate: two categories with log-probs gate_lp[n]; counter word 2j + 1 keeps this draw apart from the vocabulary's
+    const uint4 r = philox4x32_10(make_uint4(0u, (unsigned)c, (unsigned)a.t, 2u * (unsigned)j + 1u), key);
+    const float g0 = a.gate_lp[(size_t)n * 2], g1 = a.gate_lp[(size_t)n * 2 + 1];
     const int gate = u01(r.x) < expf(g0) ? 0 : 1;
-    sel_word[n] = word; sel_gate[n] = gate;
-    out_words[(size_t)n * T + t] = word; out_gates[(size_t)n * T + t] = gate;
-    lp_words[(size_t)n * T + t] = lw; lp_gates[(size_t)n * T + t] = gate == 0 ? g0 : g1;
+    a.sel_word[n] = word; a.sel_gate[n] = gate;
+    a.out_words[o] = word; a.out_gates[o] = gate;
+    a.lp_words[o] = lw; a.lp_gates[o] = gate == 0 ? g0 : g1;
   }
 }
 
@@ -474,11 +673,27 @@ int launch_greedy_pick(Ctx* c, int rows, int t, int T, int64_t* out_words, int64
   return VSR_OK;
 }
 
-int launch_sample_pick(Ctx* c, int rows, int t, int T, uint64_t seed, int64_t* out_words, int64_t* out_gates,
-                       float* lp_words, float* lp_gates, cudaStream_t st) {
+int launch_sample_pick(Ctx* c, int rows, int t, int T, const VsrSampleParams& p, int64_t* out_words,
+                       int64_t* out_gates, float* lp_words, float* lp_gates, cudaStream_t st) {
   PhaseScope ps(c, PH_BEAM, st);
-  k_sample_pick<<<rows, 256, 0, st>>>(c->logits, c->NE, c->V, c->row_max, c->row_lsum, c->gate_lp, (unsigned long long)seed, t, T,
-                                      c->sel_word, c->sel_gate, out_words, out_gates, lp_words, lp_gates);
+  SampleArgs a{};
+  a.logits = c->logits; a.ld = c->NE; a.V = c->V;
+  a.row_max = c->row_max; a.row_lsum = c->row_lsum; a.gate_lp = c->gate_lp;
+  a.forced = p.use_verbs ? c->forced : nullptr;
+  a.seed = (unsigned long long)p.seed; a.t = t; a.T = T; a.n = p.n;
+  a.tau = p.temperature; a.top_k = p.top_k; a.top_p = p.top_p;
+  const bool trunc = (p.top_k > 0 && p.top_k < c->V) || p.top_p < 1.f;
+  a.sel_word = c->sel_word; a.sel_gate = c->sel_gate;
+  a.out_words = out_words; a.out_gates = out_gates; a.lp_words = lp_words; a.lp_gates = lp_gates;
+  if (!trunc) {
+    k_sample_pick<false><<<rows, SP_THREADS, 0, st>>>(a);
+  } else {
+    if (!c->sample_attr_set) {     // up to 192 KB at the largest vocabulary (per device, hence per handle)
+      VSR_CHECK_CUDA(cudaFuncSetAttribute(k_sample_pick<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 48 * 1024 * 4));
+      c->sample_attr_set = true;
+    }
+    k_sample_pick<true><<<rows, SP_THREADS, sizeof(float) * (size_t)round_up(c->V, 4), st>>>(a);
+  }
   VSR_CHECK_CUDA(cudaGetLastError()); c->launches++;
   return VSR_OK;
 }

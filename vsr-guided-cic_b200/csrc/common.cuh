@@ -365,6 +365,7 @@ struct Ctx {
   float *m0, *m1, *m0n, *m1n;        // sticky EOS masks [caps][beam]
   int32_t *sel_beam, *sel_word, *sel_gate;  // [caps][beam] selections of the current step
   int32_t *sel_beam_n, *sel_word_n, *sel_gate_n;
+  int cap_sel = 0;                   // capacity of the six sel_* buffers in rows (ensure_sel)
   int32_t *hist_parent, *hist_word, *hist_gate;  // [T][caps][beam]
   float *hist_score, *hist_lpw, *hist_lpg;       // [T][caps][beam]
   int hist_T = 0, hist_b = 0, hist_k = 0;
@@ -401,6 +402,7 @@ struct Ctx {
   uint64_t epoch = 0, graph_clock = 0;
   cudaStream_t cap_stream = nullptr;
   bool attend_attr_set = false;
+  bool sample_attr_set = false;     // k_sample_pick may take up to 192 KB of dynamic shared memory
   bool state_h32 = true;             // the last step wrote fp32 h1'/h2' (always on the FFMA twin)
   bool use_graphs = true;            // VSRDEC_GRAPH=0 disables
   bool zero_state_opt = true;        // VSRDEC_ZERO_STATE=0: run the h-dependent GEMM parts at t = 0 although h = 0
@@ -425,6 +427,7 @@ int run_prologue(Ctx* c, const void* det, int64_t det_stride, cudaStream_t st);
 int run_prologue_indexed(Ctx* c, const void* det, int64_t det_stride, cudaStream_t st);
 int ensure_rows(Ctx* c, int rows);
 int ensure_beam_ws(Ctx* c, int caps, int T);
+int ensure_sel(Ctx* c, int rows);
 
 struct StepIO {
   int rows;          // rows processed this step
@@ -455,8 +458,9 @@ int launch_commit_identity(Ctx* c, int rows, const int64_t* next_words, int64_t 
                            int next_slot, cudaStream_t st);
 int launch_greedy_pick(Ctx* c, int rows, int t, int T, int64_t* out_words, int64_t* out_gates,
                        cudaStream_t st);
-int launch_sample_pick(Ctx* c, int rows, int t, int T, uint64_t seed, int64_t* out_words, int64_t* out_gates,
-                       float* lp_words, float* lp_gates, cudaStream_t st);
+// draws of the sampling decode: rows = captions * p.n, row = caption * p.n + draw
+int launch_sample_pick(Ctx* c, int rows, int t, int T, const VsrSampleParams& p, int64_t* out_words,
+                       int64_t* out_gates, float* lp_words, float* lp_gates, cudaStream_t st);
 int launch_gate_head(Ctx* c, int rows, float* gate_out, int64_t gate_stride, cudaStream_t st);
 int launch_rows_to_all(Ctx* c, const F16Pair& src, const F16Pair& dst, int rows, int T, int t, cudaStream_t st);
 int run_vocab_rows(Ctx* c, const F16Pair& a_b, float* logits, int M, float* out_logp, cudaStream_t st, bool softmax_only);

@@ -12,7 +12,7 @@ slot read at that step) and `slot` (int64, the token outputs' shape: that slot).
 attended feature (0 at padding regions), untouched by verb forcing and not masked after a caption's EOS.  For beam search
 they follow each returned beam's back-pointer path, unlike the log-probs, which are in slot order as in the reference.
 
-Every driver (`beam_search`, `beam_search_v`, `beam_search_v_indexed`, `forward`, `test`, `sample_rl`, and `step` /
+Every driver (`beam_search`, `beam_search_v`, `beam_search_v_indexed`, `forward`, `test`, `sample_rl`, `sample_v`, and `step` /
 `step_v` of the sub-class) takes region features in float32, float16 or bfloat16, one dtype for the detections and the
 slot tiles.  The kernels widen half-precision values to fp32 as they load them, so every output is bit-identical to that
 of the same call on the features' float32 upcast; only the bytes read and copied halve.
@@ -66,16 +66,35 @@ class CaptioningModel(nn.Module):
         res, att = self._run(eng, eng.greedy, return_attention)
         return res if att is None else (*res, att)
 
-    def sample_rl(self, statics, *args, seed=None, return_attention=False):
+    def sample_rl(self, statics, *args, seed=None, return_attention=False, n=1, temperature=1.0, top_k=0, top_p=1.0):
         """Multinomial sampling with log-probs (reference CaptioningModel.py:54-76): at every step both heads are
         sampled from the step's distributions and fed back; returns ((words, gates), (lp_words, lp_gates)), each (b,T).
         The whole loop runs on the device (vsr_sample: Gumbel-max over the vocabulary row with a Philox stream).  The
         stream's seed is drawn from torch's CPU generator unless given, so torch.manual_seed() makes it reproducible
-        (the draws differ from torch.distributions' — another generator — but follow the same distributions)."""
+        (the draws differ from torch.distributions' — another generator — but follow the same distributions).
+        Extensions (keywords only): n independent draws per caption, returned as (b, n, T) when n > 1 (draw j is the
+        same for every n > j); the word head sampled at `temperature`, from its top_k most likely words (0 = off) and
+        then from the smallest set of those that holds top_p of their mass (1 = off).  The log-probs stay the model's
+        own (untempered, untruncated).  Semantics: include/vsrdec.h, vsr_sample_ex."""
+        return self._sample(statics[:2], False, False, seed, return_attention, n, temperature, top_k, top_p)
+
+    def sample_v(self, statics, *, n=1, temperature=1.0, top_k=0, top_p=1.0, gt=False, seed=None, return_attention=False):
+        """sample_rl with verb forcing (step_v semantics, gt as in beam_search_v): statics = (detections, det_seqs,
+        verbs).  A step whose slot holds a verb takes the forced word and gate 1, both with log-prob 0; the other steps
+        are sampled as in sample_rl.  Same return structure as sample_rl."""
+        if len(statics) < 3 or statics[2] is None:
+            from vsrdec import VsrError
+            raise VsrError("sample_v needs statics = (detections, det_seqs, verbs)")
+        return self._sample(statics, True, gt, seed, return_attention, n, temperature, top_k, top_p)
+
+    def _sample(self, statics, use_verbs, gt, seed, return_attention, n, temperature, top_k, top_p):
+        from vsrdec.engine import check_sample_args
+        check_sample_args(n, temperature, top_k, top_p, statics[0].size(0))   # before the prologue: nothing runs
         eng = self._engine_for(statics)
         if seed is None:
             seed = int(torch.randint(0, 2 ** 62, (1,)).item())
-        res, att = self._run(eng, lambda: eng.sample(seed), return_attention)
+        res, att = self._run(eng, lambda: eng.sample(seed, n=n, temperature=temperature, top_k=top_k, top_p=top_p,
+                                                     use_verbs=use_verbs, gt=gt), return_attention)
         return res if att is None else (*res, att)
 
     def _select_beam(self, input, selected_beam, cur_beam_size, beam_size, b_s, reduced=True):

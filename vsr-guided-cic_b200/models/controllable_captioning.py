@@ -3,7 +3,8 @@
 Keeps the reference's class surface (models/controllable_captioning.py:10-303): constructor
 signature, the 28-tensor state_dict (same names, shapes, dtypes, registration order),
 `init_state`, `step`, `step_v`, `test`, `sample_rl`, and the inherited `forward` /
-`beam_search` / `beam_search_v`.  Every decode driver also returns the per-word attention on request
+`beam_search` / `beam_search_v`.  `sample_rl` and the inherited `sample_v` (sampling with verb forcing) also take
+n draws per caption, a temperature and top-k / top-p truncation (models/CaptioningModel.py).  Every decode driver also returns the per-word attention on request
 (`return_attention=True`, see models/CaptioningModel.py), which the reference only exposes as a local of `step_v`.
 Region features (detections, det_seqs / ctrl_det_seqs) may be float16 or bfloat16 as well as float32: a decode of
 half-precision features is bit-identical to the decode of their float32 upcast, and reads half the bytes.  The parameters live in ordinary torch modules so that
@@ -23,6 +24,9 @@ LIMITS the reference does not have (each raises VsrError with a message, never a
     on the activation scale, not the input format: it is the same for float32, float16 and bfloat16 features;
   * region features are float32, float16 or bfloat16, one dtype for the detections and the slot tiles (a mismatch or
     any other dtype raises); half precision is refused under VSRDEC_GEMM=simt (the fp32 FFMA verification twin).
+  * sampling (`sample_rl`, `sample_v`): captions x n draws <= 2^30 rows per call; temperature a finite float32 > 0 and
+    top_p in (0, 1] as float32 values (where logits / temperature overflows float32 it is clamped to +-FLT_MAX: the
+    overflowing words tie and the lowest index among them wins).
 Among candidates whose fp32 scores tie EXACTLY the order is (score desc, flat index asc); torch.sort leaves it unspecified.
 """
 import json
@@ -203,5 +207,7 @@ class ControllableCaptioningModel(_CaptioningModel):
     def test(self, detections, ctrl_det_seqs_test, return_attention=False):
         return super().test((detections, ctrl_det_seqs_test), return_attention=return_attention)
 
-    def sample_rl(self, detections, ctrl_det_seqs_test, seed=None, return_attention=False):
-        return super().sample_rl((detections, ctrl_det_seqs_test), seed=seed, return_attention=return_attention)
+    def sample_rl(self, detections, ctrl_det_seqs_test, seed=None, return_attention=False, n=1, temperature=1.0,
+                  top_k=0, top_p=1.0):
+        return super().sample_rl((detections, ctrl_det_seqs_test), seed=seed, return_attention=return_attention, n=n,
+                                 temperature=temperature, top_k=top_k, top_p=top_p)

@@ -28,6 +28,11 @@ class VsrTrace(ctypes.Structure):
                 ("forced_word", c_vp), ("forced_gate", c_vp)]
 
 
+class VsrSampleParams(ctypes.Structure):
+    _fields_ = [("seed", ctypes.c_uint64), ("n", c_i32), ("temperature", c_f), ("top_k", c_i32), ("top_p", c_f),
+                ("use_verbs", c_i32), ("gt", c_i32)]
+
+
 # every symbol include/vsrdec.h declares: name -> (restype, argtypes)
 EXPORTED_SYMBOLS = {
     "vsr_last_error": (ctypes.c_char_p, []),
@@ -49,6 +54,7 @@ EXPORTED_SYMBOLS = {
     "vsr_forward_teacher": (ctypes.c_int, [c_vp, c_vp, c_i32, c_vp, c_vp, c_vp]),
     "vsr_greedy": (ctypes.c_int, [c_vp, c_vp, c_vp, c_vp]),
     "vsr_sample": (ctypes.c_int, [c_vp, ctypes.c_uint64, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "vsr_sample_ex": (ctypes.c_int, [c_vp, ctypes.POINTER(VsrSampleParams), c_vp, c_vp, c_vp, c_vp, c_vp]),
     "vsr_set_attention_capture": (ctypes.c_int, [c_vp, c_i32]),
     "vsr_get_attention": (ctypes.c_int, [c_vp, c_vp, c_vp, c_vp]),
     "vsr_launch_count": (c_i64, [c_vp]),

@@ -3,12 +3,14 @@
 PyTorch is plumbing here (device memory, streams); every hot operation runs in libvsrdec's
 sm_100a kernels.  CPU tensors are rejected — there is no fallback path."""
 import ctypes
+import math
+import numbers
 from typing import Dict, List, Optional, Sequence
 
 import torch
 
 from . import _lib
-from ._lib import VsrError, VsrDims, VsrTrace, c_vp, c_i32, c_i64, c_f
+from ._lib import VsrError, VsrDims, VsrSampleParams, VsrTrace, c_vp, c_i32, c_i64, c_f
 
 # state_dict registration order of the reference model (controllable_captioning.py:23-68);
 # the order of the `weights` array of vsr_create().
@@ -39,6 +41,30 @@ def _feat_dtype(*feats):
         if t.dtype != dt:
             raise VsrError(f"detections and det_seqs must share one dtype, got {dt} and {t.dtype}")
     return _FEAT_DT[dt]
+
+
+MAX_SAMPLE_ROWS = 2 ** 30       # captions x draws of one sampling call (vsr_sample_ex)
+
+
+def check_sample_args(n, temperature, top_k, top_p, b=None):
+    """Raise VsrError unless (n, temperature, top_k, top_p) are valid sampling parameters (vsr_sample_ex) for b
+    captions.  temperature and top_p are checked as the float32 values the library receives: a finite temperature that
+    rounds to 0 in float32 (e.g. 1e-50) is refused here, not after the prologue has run."""
+    if isinstance(n, bool) or not isinstance(n, numbers.Integral) or not 1 <= n < 2 ** 31:
+        raise VsrError(f"n (draws per caption) must be an int >= 1, got {n!r}")
+    if b is not None and b * n > MAX_SAMPLE_ROWS:
+        raise VsrError(f"{b} captions x n={n} draws exceed {MAX_SAMPLE_ROWS} rows per sampling call")
+    if isinstance(top_k, bool) or not isinstance(top_k, numbers.Integral) or top_k < 0:
+        raise VsrError(f"top_k must be an int >= 0 (0 = off), got {top_k!r}")
+    try:
+        tau, p = float(temperature), float(top_p)
+    except (TypeError, ValueError):
+        raise VsrError(f"temperature and top_p must be numbers, got {temperature!r} / {top_p!r}") from None
+    tau32, p32 = c_f(tau).value, c_f(p).value
+    if not math.isfinite(tau32) or tau32 <= 0.0:
+        raise VsrError(f"temperature must be a finite float32 > 0, got {temperature!r}")
+    if not (0.0 < p <= 1.0) or p32 <= 0.0:
+        raise VsrError(f"top_p must be in (0, 1] (1 = off) and nonzero in float32, got {top_p!r}")
 
 
 def _req_cuda(t: torch.Tensor, name: str, dtype=None):
@@ -276,18 +302,29 @@ class DecoderEngine:
         self._attn_shape = (b, None, T, self.R)
         return words, gates
 
-    def sample(self, seed: int):
-        """Multinomial sampling decode (vsr_sample): (words, gates) int64 (b,T), (lp_words, lp_gates) fp32 (b,T)."""
+    def sample(self, seed: int, n=1, temperature=1.0, top_k=0, top_p=1.0, use_verbs=False, gt=False):
+        """Sampling decode (vsr_sample_ex): n independent draws per caption, the word head at `temperature`, truncated
+        to the top_k most likely words (0 = off) and then to the smallest set of them holding top_p of their mass
+        (1 = off); use_verbs / gt force verb slots as step_v does.  Returns (words, gates) int64 and (lp_words, lp_gates)
+        fp32, shaped (b, T) when n == 1 and (b, n, T) otherwise; the log-probs are the model's own, untempered and
+        untruncated.  Draw j of a caption is the same for every n > j.  The semantics are spelled out in
+        include/vsrdec.h (vsr_sample_ex)."""
+        check_sample_args(n, temperature, top_k, top_p, self.b)
+        if use_verbs and (self._keep is None or self._keep[2] is None):
+            raise VsrError("use_verbs needs a prologue with a verbs tensor")
         b, T = self.b, self.dims["seq_len"]
-        words = torch.empty((b, T), device=self.device, dtype=torch.long)
-        gates = torch.empty((b, T), device=self.device, dtype=torch.long)
-        lpw = torch.empty((b, T), device=self.device, dtype=torch.float32)
-        lpg = torch.empty((b, T), device=self.device, dtype=torch.float32)
+        shape = (b, T) if n == 1 else (b, int(n), T)
+        words = torch.empty(shape, device=self.device, dtype=torch.long)
+        gates = torch.empty(shape, device=self.device, dtype=torch.long)
+        lpw = torch.empty(shape, device=self.device, dtype=torch.float32)
+        lpg = torch.empty(shape, device=self.device, dtype=torch.float32)
+        prm = VsrSampleParams(int(seed) & 0xFFFFFFFFFFFFFFFF, int(n), float(temperature), int(min(top_k, 2 ** 31 - 1)), float(top_p),
+                              int(bool(use_verbs)), int(bool(gt)))
         with torch.cuda.device(self.device):
-            _lib.check(self.lib, self.lib.vsr_sample(self.handle, int(seed) & 0xFFFFFFFFFFFFFFFF, words.data_ptr(),
-                                                     gates.data_ptr(), lpw.data_ptr(), lpg.data_ptr(),
-                                                     _stream_ptr(self.device)))
-        self._attn_shape = (b, None, T, self.R)
+            _lib.check(self.lib, self.lib.vsr_sample_ex(self.handle, ctypes.byref(prm), words.data_ptr(),
+                                                        gates.data_ptr(), lpw.data_ptr(), lpg.data_ptr(),
+                                                        _stream_ptr(self.device)))
+        self._attn_shape = (b, None if n == 1 else int(n), T, self.R)
         return (words, gates), (lpw, lpg)
 
     # ------------------------------------------------------------------ attention capture
@@ -298,7 +335,7 @@ class DecoderEngine:
     def attention(self):
         """Attention of the last decode (vsr_get_attention): {"alpha": float32, "slot": int64}, shaped
         (b, out_size, T, R+1) / (b, out_size, T) after a beam search (following each returned beam's back-pointer
-        path), (b, T, R+1) / (b, T) after the other drivers.  alpha[..., 0] is the sentinel, alpha[..., r+1] region r
+        path), (b, n, T, R+1) / (b, n, T) after sample(n > 1), (b, T, R+1) / (b, T) after the other drivers.  alpha[..., 0] is the sentinel, alpha[..., r+1] region r
         of the slot read at that step.  Raises VsrError when that decode ran without capture."""
         if self._attn_shape is None:
             raise VsrError("attention(): no decode has run on this engine")

@@ -79,43 +79,37 @@ static int pad_rows(int n_valid, int bn, int alt_bn) {
 }
 
 // kind of twin set: fp16 hi + fp16 residual (f16x3 GEMMs) or fp16 hi + e4m3 hi8 / lo8 (f16+f8x2 GEMMs)
-enum PairKind { PAIR_F16X3 = 0, PAIR_F8 = 1, PAIR_BOTH = 2 };     // BOTH: operands of a GEMM that runs in either mode
+enum PairKind { PAIR_F16X3 = 0, PAIR_F8 = 1 };
 static PairKind step_kind(const Ctx* c) { return c->gemm_f8 ? PAIR_F8 : PAIR_F16X3; }
 
 int alloc_pair(Ctx* c, F16Pair* b, int rows, int ld, int box_rows, PairKind kind, bool weight = false, int n_valid = 0,
-               int alt_bn = 0, int alt_kb = 64) {
+               int alt_bn = 0) {
   dev_free(c, b->hi); dev_free(c, b->lo); dev_free(c, b->hi8); dev_free(c, b->lo8);
   b->hi = b->lo = b->hi8 = b->lo8 = nullptr;
   if (!c->use_tc) return VSR_OK;
   VSR_TRY(dev_alloc(c, &b->hi, (size_t)rows * ld * 2));
   b->rows = rows; b->ld = ld; b->box_rows = box_rows;
   VSR_TRY(make_tmap_f16(b->map_hi, b->hi, rows, ld, ld, box_rows));
-  VSR_TRY(make_tmap_f16(b->map32_hi, b->hi, rows, ld, ld, box_rows, 32));
-  if (kind == PAIR_F16X3 || kind == PAIR_BOTH) {
+  if (kind == PAIR_F16X3) {
     VSR_TRY(dev_alloc(c, &b->lo, (size_t)rows * ld * 2));
     VSR_TRY(make_tmap_f16(b->map_lo, b->lo, rows, ld, ld, box_rows));
-    VSR_TRY(make_tmap_f16(b->map32_lo, b->lo, rows, ld, ld, box_rows, 32));
-  }
-  if (kind == PAIR_F8 || kind == PAIR_BOTH) {
+  } else {
     VSR_TRY(dev_alloc(c, &b->hi8, (size_t)rows * ld));
     VSR_TRY(dev_alloc(c, &b->lo8, (size_t)rows * ld));
     VSR_TRY(make_tmap_u8(b->map8_hi, b->hi8, rows, ld, ld, box_rows));
     VSR_TRY(make_tmap_u8(b->map8_lo, b->lo8, rows, ld, ld, box_rows));
-    VSR_TRY(make_tmap_u8(b->map8_32_hi, b->hi8, rows, ld, ld, box_rows, 32));
-    VSR_TRY(make_tmap_u8(b->map8_32_lo, b->lo8, rows, ld, ld, box_rows, 32));
   }
-  b->act_scale = (!weight && kind != PAIR_F16X3) ? ACT_SCALE_F8 : 1.f;
-  b->kb = c->gemm_kb;
+  b->act_scale = (!weight && kind == PAIR_F8) ? ACT_SCALE_F8 : 1.f;
   b->n_valid = n_valid > 0 ? n_valid : rows;
-  b->alt_bn = 0;
-  if (alt_bn > 0 && c->use_alt_tiles) {
-    VSR_TRY(make_tmap_f16(b->alt_hi, b->hi, rows, ld, ld, alt_bn, alt_kb));
-    if (kind != PAIR_F8) VSR_TRY(make_tmap_f16(b->alt_lo, b->lo, rows, ld, ld, alt_bn, alt_kb));
-    if (kind != PAIR_F16X3) {
-      VSR_TRY(make_tmap_u8(b->alt8_hi, b->hi8, rows, ld, ld, alt_bn, alt_kb));
-      VSR_TRY(make_tmap_u8(b->alt8_lo, b->lo8, rows, ld, ld, alt_bn, alt_kb));
+  b->alt_bn = alt_bn;
+  if (alt_bn > 0) {
+    VSR_TRY(make_tmap_f16(b->alt_hi, b->hi, rows, ld, ld, alt_bn));
+    if (kind == PAIR_F16X3) {
+      VSR_TRY(make_tmap_f16(b->alt_lo, b->lo, rows, ld, ld, alt_bn));
+    } else {
+      VSR_TRY(make_tmap_u8(b->alt8_hi, b->hi8, rows, ld, ld, alt_bn));
+      VSR_TRY(make_tmap_u8(b->alt8_lo, b->lo8, rows, ld, ld, alt_bn));
     }
-    b->alt_bn = alt_bn; b->alt_kb = alt_kb;
   }
   if (weight && b->scale == nullptr) VSR_TRY(dev_alloc(c, (void**)&b->scale, 2 * sizeof(float)));
   return VSR_OK;
@@ -146,13 +140,11 @@ int ensure_rows(Ctx* c, int rows) {
   VSR_TRY(dev_alloc(c, (void**)&c->forced, sizeof(int32_t) * n));
   VSR_TRY(dev_alloc(c, (void**)&c->cand, sizeof(int32_t) * n * VSR_MAX_BEAM));
   VSR_TRY(dev_alloc(c, (void**)&c->word_in, sizeof(int64_t) * n));
-  // the recurrent states feed GEMM-A, which runs f16x3 when the CTA-pair kernel is disabled (step_kernels.cu: run_step),
-  // and GEMM-D, which runs f16+f8x2: h1 / h2 (and the h1' / h2' they are copied from) carry both residual forms
-  const PairKind sk = step_kind(c), hk = sk == PAIR_F8 ? PAIR_BOTH : sk;
-  VSR_TRY(alloc_pair(c, &c->h1_b, cap, c->Hp, MPAD, hk)); VSR_TRY(alloc_pair(c, &c->h2_b, cap, c->Hp, MPAD, hk));
+  const PairKind sk = step_kind(c);
+  VSR_TRY(alloc_pair(c, &c->h1_b, cap, c->Hp, MPAD, sk)); VSR_TRY(alloc_pair(c, &c->h2_b, cap, c->Hp, MPAD, sk));
   VSR_TRY(alloc_pair(c, &c->s_t_b, cap, c->Hp, MPAD, sk));
-  VSR_TRY(alloc_pair(c, &c->h1n_b, cap, c->Hp, MPAD, hk)); VSR_TRY(alloc_pair(c, &c->g_t_b, cap, c->Hp, MPAD, sk));
-  VSR_TRY(alloc_pair(c, &c->att_b, cap, c->Fp, MPAD, sk)); VSR_TRY(alloc_pair(c, &c->h2n_b, cap, c->Hp, MPAD, hk));
+  VSR_TRY(alloc_pair(c, &c->h1n_b, cap, c->Hp, MPAD, sk)); VSR_TRY(alloc_pair(c, &c->g_t_b, cap, c->Hp, MPAD, sk));
+  VSR_TRY(alloc_pair(c, &c->att_b, cap, c->Fp, MPAD, sk)); VSR_TRY(alloc_pair(c, &c->h2n_b, cap, c->Hp, MPAD, sk));
   c->cap_rows = cap;
   return VSR_OK;
 }
@@ -283,33 +275,21 @@ static int create_impl(const VsrDims* d, const float* const* w, Ctx** out) {
     c->use_tc = !(mode != nullptr && strcmp(mode, "simt") == 0);
     c->gemm_f8 = !(mode != nullptr && strcmp(mode, "f16x3") == 0);
   }
-  // UMMA N tile per GEMM (128 or 256): 128 measured faster on B200 for every per-step shape (more CTAs
-  // in flight, 3-stage ring); VSRDEC_BN=256 switches all of them for experiments
-  int bn = 128;
-  if (const char* e = getenv("VSRDEC_BN")) bn = atoi(e) == 256 ? 256 : 128;
-  // GEMM-A / GEMM-D tiles are fixed by their fused LSTM epilogues: 6 gates x 32 units = 192, 4 x 32 = 128.
   if (const char* e = getenv("VSRDEC_GRAPH")) c->use_graphs = atoi(e) != 0;
   if (const char* e = getenv("VSRDEC_PDL")) c->use_pdl = atoi(e) != 0;
-  if (const char* e = getenv("VSRDEC_ZERO_STATE")) c->zero_state_opt = atoi(e) != 0;
-  if (const char* e = getenv("VSRDEC_PDL_MODE")) c->pdl_mode = atoi(e);
-  if (const char* e = getenv("VSRDEC_KB")) c->gemm_kb = atoi(e) == 32 ? 32 : 64;
-  if (const char* e = getenv("VSRDEC_ALT_TILES")) c->use_alt_tiles = atoi(e) != 0;
-  // weight pairs are power-of-two scaled per tensor (F16Pair::scale)
+  // UMMA N tile of the single-CTA kernel: 128 (wider tiles measured slower on B200 for every per-step shape: fewer CTAs
+  // in flight, shallower ring).  GEMM-A / GEMM-D tiles are fixed by their fused LSTM epilogues: 6 gates x 32 units = 192,
+  // 4 x 32 = 128.  Weight pairs are power-of-two scaled per tensor (F16Pair::scale).
   const PairKind sk = step_kind(c);
-  VSR_TRY(alloc_pair(c, &c->WA_b, c->NA, c->KA, 192, sk == PAIR_F8 ? PAIR_BOTH : sk, true)); VSR_TRY(alloc_pair(c, &c->WB1_b, c->NB1, c->Hp, bn, sk, true, c->NB1v));
-  VSR_TRY(alloc_pair(c, &c->WB2_b, c->NB2, c->Hp, bn, sk, true, c->NB2v)); VSR_TRY(alloc_pair(c, &c->WC_b, c->NC, c->Hp, 128, sk, true));
-  VSR_TRY(alloc_pair(c, &c->WD_b, c->ND, c->KD, 128, sk, true)); VSR_TRY(alloc_pair(c, &c->WE_b, c->NE, c->Hp, bn, sk, true, c->V, 144, 64));
-  if (const char* e = getenv("VSRDEC_PAIR")) c->use_pair = atoi(e) != 0;
-  if (const char* e = getenv("VSRDEC_PAIR_MIN_ROWS")) c->pair_min_rows = atoi(e);
-  if (c->use_pair && c->use_tc) {     // CTA-pair kernel for the large-batch launches: 256 x 192 tiles for A, 256 x 256 for B, D + C
+  VSR_TRY(alloc_pair(c, &c->WA_b, c->NA, c->KA, 192, sk, true)); VSR_TRY(alloc_pair(c, &c->WB1_b, c->NB1, c->Hp, 128, sk, true, c->NB1v));
+  VSR_TRY(alloc_pair(c, &c->WB2_b, c->NB2, c->Hp, 128, sk, true, c->NB2v)); VSR_TRY(alloc_pair(c, &c->WC_b, c->NC, c->Hp, 128, sk, true));
+  VSR_TRY(alloc_pair(c, &c->WD_b, c->ND, c->KD, 128, sk, true)); VSR_TRY(alloc_pair(c, &c->WE_b, c->NE, c->Hp, 128, sk, true, c->V, 144));
+  if (c->use_tc) {     // CTA-pair kernel for the large-batch launches: 256 x 192 tiles for A and E, 256 x 256 for B, D + C
     VSR_TRY(make_pair_maps(&c->WA_b, 96)); VSR_TRY(make_pair_maps(&c->WB1_b, 128)); VSR_TRY(make_pair_maps(&c->WB2_b, 128));
     VSR_TRY(make_pair_maps(&c->WC_b, 128)); VSR_TRY(make_pair_maps(&c->WD_b, 128)); VSR_TRY(make_pair_maps(&c->WE_b, 96));
   }
-  // GEMM-A's 192-wide tile only fits 2 ring stages with 64-element k-blocks; 32-element blocks give 5
-  c->WA_b.kb = 32;
-  if (const char* e = getenv("VSRDEC_KB_A")) c->WA_b.kb = atoi(e) == 32 ? 32 : 64;
   // the once-per-batch prologue GEMMs (U, U2, att_va projection) keep all three passes in fp16
-  VSR_TRY(alloc_pair(c, &c->WU_b, c->NA, c->Fp, 128, PAIR_F16X3, true)); VSR_TRY(alloc_pair(c, &c->Wva_b, c->NVA, c->Fp, bn, PAIR_F16X3, true));
+  VSR_TRY(alloc_pair(c, &c->WU_b, c->NA, c->Fp, 128, PAIR_F16X3, true)); VSR_TRY(alloc_pair(c, &c->Wva_b, c->NVA, c->Fp, 128, PAIR_F16X3, true));
   if (d->img_second_lstm) VSR_TRY(alloc_pair(c, &c->WU2_b, c->ND, c->Fp, 128, PAIR_F16X3, true));
   VSR_TRY(pack_weights(c, w, 0));
   VSR_CHECK_CUDA(cudaStreamSynchronize(0));
@@ -532,7 +512,7 @@ static int enqueue_beam_steps(Ctx* c, int k, const int64_t* eos, int use_verbs, 
     const int rows = b * cur;
     StepIO io{};
     io.rows = rows; io.cur_beam = cur; io.use_verbs = use_verbs != 0; io.gt = gt != 0; io.topk = k;
-    io.zero_state = t == 0 && c->zero_state_opt;
+    io.zero_state = t == 0;
     if (tr && tr->step_out) { io.out_logp = tr->step_out + (size_t)t * b * k * c->V; io.out_stride = c->V; }
     if (tr && tr->step_gate) { io.gate_out = tr->step_gate + (size_t)t * b * k * 2; io.gate_stride = 2; }
     attn_step_io(c, io, t, (int64_t)b * k);
@@ -612,7 +592,7 @@ static int enqueue_forward_steps(Ctx* c, const int64_t* captions, int T, bool ba
     }
     StepIO io{};
     io.rows = b; io.cur_beam = 1; io.use_verbs = false; io.gt = false; io.topk = 0;
-    io.zero_state = t == 0 && c->zero_state_opt;
+    io.zero_state = t == 0;
     attn_step_io(c, io, t, b);
     if (batched) {
       io.skip_vocab = true;
@@ -669,7 +649,7 @@ static int greedy_impl(Ctx* c, int64_t* out_words, int64_t* out_gates, cudaStrea
   for (int t = 0; t < T; ++t) {
     StepIO io{};
     io.rows = b; io.cur_beam = 1; io.use_verbs = false; io.gt = false; io.topk = 1;
-    io.zero_state = t == 0 && c->zero_state_opt;
+    io.zero_state = t == 0;
     attn_step_io(c, io, t, b);
     VSR_TRY(run_step(c, io, st));
     VSR_TRY(launch_greedy_pick(c, b, t, T, out_words, out_gates, st));
@@ -704,7 +684,7 @@ static int sample_impl(Ctx* c, const VsrSampleParams& p, int64_t* out_words, int
     StepIO io{};
     io.rows = rows; io.cur_beam = p.n; io.use_verbs = p.use_verbs != 0; io.gt = p.gt != 0;
     io.topk = 0;     // statistics + gate head (+ forced word) only
-    io.zero_state = t == 0 && c->zero_state_opt;
+    io.zero_state = t == 0;
     attn_step_io(c, io, t, rows);
     VSR_TRY(run_step(c, io, st));
     VSR_TRY(launch_sample_pick(c, rows, t, T, p, out_words, out_gates, lp_words, lp_gates, st));

@@ -632,7 +632,7 @@ int launch_beam_step(Ctx* c, int t, int b, int cur, int k, int64_t eos0, int64_t
   AdvanceArgs ad{};
   ad.rows_new = b * k; ad.cur = cur; ad.k = k; ad.fixed_slot = -1;
   fill_advance(c, ad);
-  VSR_CHECK_CUDA(launch_k(k_beam_step, dim3(b, advance ? k : 1), dim3(256), 0, st, c->use_pdl && (c->pdl_mode & 2), a, ad, advance ? 1 : 0));
+  k_beam_step<<<dim3(b, advance ? k : 1), 256, 0, st>>>(a, ad, advance ? 1 : 0);
   VSR_CHECK_CUDA(cudaGetLastError()); c->launches++;
   std::swap(c->sel_beam, c->sel_beam_n);
   std::swap(c->sel_word, c->sel_word_n);

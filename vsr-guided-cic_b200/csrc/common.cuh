@@ -97,15 +97,10 @@ struct F16Pair {
   // so lo parts of small weights stay out of the fp16 subnormals; the GEMM epilogue multiplies the accumulator by 1/s
   // (exact).  Null = unscaled (activations: |x| ~ 1).
   float* scale = nullptr;
-  int kb = 64;          // (weights only) k-block of the GEMMs that use this weight: 64 (128B swizzle) or 32 (64B)
   alignas(64) unsigned char map_hi[128];
   alignas(64) unsigned char map_lo[128];
-  alignas(64) unsigned char map32_hi[128];   // 32-element k-blocks, 64-byte swizzle
-  alignas(64) unsigned char map32_lo[128];
   alignas(64) unsigned char map8_hi[128];    // e4m3 twins, 64-element k-blocks (64-byte rows, 64-byte swizzle)
   alignas(64) unsigned char map8_lo[128];
-  alignas(64) unsigned char map8_32_hi[128]; // e4m3 twins, 32-element k-blocks (32-byte rows, 32-byte swizzle)
-  alignas(64) unsigned char map8_32_lo[128];
   alignas(64) unsigned char alt8_hi[128];    // e4m3 twins, alternative N tile
   alignas(64) unsigned char alt8_lo[128];
   // (weights only) CTA-pair kernel: each CTA of the pair loads pair_rows = BN / 2 rows of a BN-wide W tile (64-element k-blocks)
@@ -116,7 +111,7 @@ struct F16Pair {
   alignas(64) unsigned char pair_h8[128];    // e4m3 copy of hi (f16+f8x2)
   // (weights only) alternative N tile, chosen per launch when it needs fewer waves over the 148 SMs
   int n_valid = 0;      // real number of output rows (<= rows)
-  int alt_bn = 0, alt_kb = 64;
+  int alt_bn = 0;
   alignas(64) unsigned char alt_hi[128];
   alignas(64) unsigned char alt_lo[128];
 };
@@ -181,7 +176,10 @@ __host__ __device__ inline int cell_col(int g, int u, int ng) {
 // kernel N+1 may become resident while kernel N drains: it runs its own set-up (barrier init, TMEM allocation,
 // descriptor prefetch, WEIGHT tile prefetch) and then blocks in pdl_wait() until kernel N has completed and its
 // writes are visible.  Rule for every such kernel: before pdl_wait() touch nothing but launch arguments and data
-// that is constant over the whole decode (weights, prologue products); write nothing.
+// that is constant over the whole decode (weights, prologue products); write nothing.  Only the step GEMMs launch with
+// the attribute (VSRDEC_PDL=0: none).  The small step kernels (attention, softmax / vocab merge, beam step) launch
+// without it, so their pdl_wait() is a no-op, but they still call pdl_trigger() at entry: the GEMM after them may
+// start its set-up only once every CTA of its predecessor has triggered or exited.
 #ifdef __CUDACC__
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
@@ -234,13 +232,13 @@ struct GemmArgs {
   const uint8_t* row_skip;  // optional [M]: a row tile whose flags are all 0 is skipped
   const F16Pair* wb = nullptr;  // fp16 hi/lo twin of w (tensor-core path), or null
   bool allow_pair = false;      // may run on the CTA-pair kernel when the launch is large enough (step GEMMs A, B, D+C, E)
-  int pair_min_rows = 1024;     //   ... i.e. has at least this many rows
+  int pair_min_rows = 1024;     //   ... i.e. has at least this many rows (run_step: PAIR_MIN_ROWS)
   bool no_alt = false;          // keep the weight's default N tile (whose epilogue is the coalesced shared-memory tile one)
   bool f8 = false;              // f16+f8x2 mode: residual products on the fp8 tensor path (operand pairs need hi8 / lo8)
-  bool pdl = false;             // launch with programmatic dependent launch (decoder-step GEMMs only)
+  bool pdl = false;             // launch with programmatic dependent launch, weight tiles fetched before the dependency
+                                //   wait (decoder-step GEMMs only)
   bool relu = false;            // FFMA twin only: max(0, .) on the output (feed-forward layers of the S-level SSP sorter)
   bool zero_acc = false;        // every A operand is known to be zero (h = 0 at t = 0): skip the main loop, acc := 0
-  int pdl_flags = 0;            // bit 0: weight tiles before the dependency wait; bit 1: trigger after the main loop
   FusedCell cell;               // epilogue fusion (tensor-core path only)
 };
 struct Ctx;
@@ -249,8 +247,8 @@ int launch_gemm(Ctx* c, const GemmArgs& g, cudaStream_t st, const GemmArgs* g2 =
 int launch_gemm_simt(const GemmArgs& g, cudaStream_t st);
 int launch_gemm_tc(const GemmArgs& g, const GemmArgs* g2, cudaStream_t st);
 bool gemm_uses_tc(const Ctx* c, const GemmArgs& g);
-int make_tmap_f16(void* out_map, const void* base, int rows, int cols, int ld, int box_rows, int kb = 64);
-int make_tmap_u8(void* out_map, const void* base, int rows, int cols, int ld, int box_rows, int kb = 64);
+int make_tmap_f16(void* out_map, const void* base, int rows, int cols, int ld, int box_rows);
+int make_tmap_u8(void* out_map, const void* base, int rows, int cols, int ld, int box_rows);
 int make_pair_maps(F16Pair* b, int pair_rows);   // tensor maps of a weight for the CTA-pair kernel (after hi/lo/hi8/lo8 are set)
 // x -> pair (fp16 hi + fp16 lo and/or e4m3 hi8/lo8, whichever arrays the pair has); scale = device {s, 1/s} computed
 // here from max|x| (weights), or null: x is multiplied by p.act_scale (activations)
@@ -301,12 +299,7 @@ struct Ctx {
   int NVA;                     // padded rows of Wva
   // fp16 hi/lo twins for the tcgen05 GEMMs
   bool use_tc = true;
-  int pair_min_rows = 640;       // B, D + C, E take the CTA-pair kernel from this many rows (VSRDEC_PAIR_MIN_ROWS; measured:
-                                 //   slower at 500 rows, 6 % faster at 1000)
-  bool use_pair = true;          // CTA-pair (cta_group::2) kernel for the large-batch step GEMMs (VSRDEC_PAIR=0 disables)
   bool gemm_f8 = true;           // step GEMMs in f16+f8x2 mode (VSRDEC_GEMM=f16x3 keeps all three passes in fp16)
-  bool use_alt_tiles = true;     // per-launch choice between the default and the alternative N tile (VSRDEC_ALT_TILES=0)
-  int gemm_kb = 64;              // k-block of the tensor-core GEMMs (VSRDEC_KB=32: 64-byte swizzle, deeper ring)
   F16Pair WA_b, WB1_b, WB2_b, WC_b, WD_b, WE_b;
   F16Pair WU_b, WU2_b, Wva_b;   // prologue weights
   F16Pair ds_b, img_b;          // prologue activations: slot rows [b*L*R][Fp], image descriptors [n_img][Fp]
@@ -405,12 +398,7 @@ struct Ctx {
   bool sample_attr_set = false;     // k_sample_pick may take up to 192 KB of dynamic shared memory
   bool state_h32 = true;             // the last step wrote fp32 h1'/h2' (always on the FFMA twin)
   bool use_graphs = true;            // VSRDEC_GRAPH=0 disables
-  bool zero_state_opt = true;        // VSRDEC_ZERO_STATE=0: run the h-dependent GEMM parts at t = 0 although h = 0
-  bool use_pdl = true;               // VSRDEC_PDL=0: plain stream serialization between the step kernels
-  // VSRDEC_PDL_MODE bits: 1 = GEMM launches, 2 = small kernels, 4 = weight prefetch before the wait, 8 = GEMMs
-  // trigger after their main loop.  Measured inside the decode graph (ms per decode): off 4.07, 1: 4.02, 1|4: 4.00,
-  // 1|2|4: 4.18 (early-resident CTAs of the many-CTA kernels pile up on the SMs that drain first), 1|2|8: 4.08.
-  int pdl_mode = 5;
+  bool use_pdl = true;               // VSRDEC_PDL=0: plain stream serialization between the step GEMMs
 };
 
 int dev_alloc(Ctx* c, void** p, size_t bytes, bool zero = true);

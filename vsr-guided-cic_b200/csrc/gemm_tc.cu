@@ -18,11 +18,10 @@
 //   warps 2-9: epilogue (two warps per TMEM lane quarter): bias -> smem behind the main loop; then one lane quarter at
 //              a time TMEM -> swizzled smem tile -> all eight warps with lanes along a row (coalesced operands and
 //              outputs): plain / g_t / fused LSTM cells; the vocabulary head keeps the row-per-thread form
-// smem ring: kStages x {A_hi, A_lo (128 x KB fp16), W_hi, W_lo (BN x KB fp16)}, full/empty mbarriers; the accumulator
+// smem ring: kStages x {A_hi, A_lo (128 x 64 fp16), W_hi, W_lo (BN x 64 fp16)}, full/empty mbarriers; the accumulator
 // hand-off to the epilogue is a tcgen05.commit on a third mbarrier.  k_gemm_tcp is the persistent variant
-// (double-buffered TMEM accumulator), k_gemm_tc2 the CTA-pair experiment.
+// (double-buffered TMEM accumulator), k_gemm_pair the CTA-pair kernel.
 #include <cuda.h>
-#include <stdlib.h>
 #include <string.h>
 #include <cuda_fp16.h>
 
@@ -43,15 +42,14 @@ constexpr int TC_EPI_WARPS = 8;
 constexpr int TC_EPI_THREADS = 32 * TC_EPI_WARPS;
 constexpr int TC_THREADS = 64 + TC_EPI_THREADS;
 
-// KB = fp16 elements per k-block: 64 (one 128-byte swizzle row) or 32 (64-byte swizzle).  The smaller
-// block halves the stage size, i.e. doubles the ring depth that fits in 227 KB of shared memory — these
-// GEMMs are bound by operand-delivery latency (measured: 2 -> 3 stages = +17..26 % on the K = 3072 shapes).
-template <int BN, int KB> struct TcCfg {
-  static constexpr int kStageB = 2 * BM * KB * 2 + 2 * BN * KB * 2;
+// Ring stages of BK-element k-blocks that fit in 220 KB of shared memory (at most 8): 3 at BN = 128 and 144, 2 at 192.
+// These GEMMs are bound by operand-delivery latency (measured: 2 -> 3 stages = +17..26 % on the K = 3072 shapes).
+template <int BN> struct TcCfg {
+  static constexpr int kStageB = 2 * BM * BK * 2 + 2 * BN * BK * 2;
   static constexpr int kStages = (220 * 1024) / kStageB > 8 ? 8 : (220 * 1024) / kStageB;
   static constexpr int kTmemCols = (BN <= 128) ? 128 : 256;   // power of two >= BN
-  static constexpr int kABytes = BM * KB * 2;            // 16 / 8 KB
-  static constexpr int kWBytes = BN * KB * 2;
+  static constexpr int kABytes = BM * BK * 2;            // 16 KB
+  static constexpr int kWBytes = BN * BK * 2;
   static constexpr int kStageBytes = 2 * kABytes + 2 * kWBytes;
   static constexpr int kRingBytes = kStages * kStageBytes;
   // epilogue tile: one TMEM lane quarter (32 rows x BN fp32) staged through shared memory (tile_epilogue)
@@ -89,7 +87,7 @@ __device__ __forceinline__ void prefetch_tmap(const CUtensorMap* map) {
   asm volatile("prefetch.tensormap [%0];" ::"l"(map) : "memory");
 }
 
-// K-major operand tile with 64-byte swizzle (rows of 64 B, 8-row groups 512 B apart)
+// K-major operand tile with 64-byte swizzle (rows of 64 B, 8-row groups 512 B apart): the e4m3 tiles of a k-block
 __device__ __forceinline__ uint64_t make_sw64_desc(uint32_t smem_addr) {
   uint64_t d = 0;
   d |= (uint64_t)((smem_addr >> 4) & 0x3FFF);
@@ -99,8 +97,6 @@ __device__ __forceinline__ uint64_t make_sw64_desc(uint32_t smem_addr) {
   d |= (uint64_t)4 << 61;                               // layout type: SWIZZLE_64B
   return d;
 }
-template <int KB> __device__ __forceinline__ uint64_t make_kmajor_desc(uint32_t smem_addr);
-
 // K-major, 128-byte-swizzled operand tile (rows of 128 B, 8-row groups 1024 B apart): UMMA smem descriptor
 __device__ __forceinline__ uint64_t make_sw128_desc(uint32_t smem_addr) {
   uint64_t d = 0;
@@ -111,24 +107,6 @@ __device__ __forceinline__ uint64_t make_sw128_desc(uint32_t smem_addr) {
   d |= (uint64_t)2 << 61;                               // layout type: SWIZZLE_128B
   return d;
 }
-
-template <> __device__ __forceinline__ uint64_t make_kmajor_desc<64>(uint32_t a) { return make_sw128_desc(a); }
-template <> __device__ __forceinline__ uint64_t make_kmajor_desc<32>(uint32_t a) { return make_sw64_desc(a); }
-
-// K-major operand tile with 32-byte swizzle (rows of 32 B, 8-row groups 256 B apart)
-__device__ __forceinline__ uint64_t make_sw32_desc(uint32_t smem_addr) {
-  uint64_t d = 0;
-  d |= (uint64_t)((smem_addr >> 4) & 0x3FFF);
-  d |= (uint64_t)1 << 16;
-  d |= (uint64_t)(256 >> 4) << 32;                      // stride byte offset: 8 rows x 32 B
-  d |= (uint64_t)1 << 46;
-  d |= (uint64_t)6 << 61;                               // layout type: SWIZZLE_32B
-  return d;
-}
-// 8-bit (e4m3) operand tiles of a KB-element k-block: rows of KB bytes
-template <int KB> __device__ __forceinline__ uint64_t make_kmajor_desc8(uint32_t smem_addr);
-template <> __device__ __forceinline__ uint64_t make_kmajor_desc8<64>(uint32_t a) { return make_sw64_desc(a); }
-template <> __device__ __forceinline__ uint64_t make_kmajor_desc8<32>(uint32_t a) { return make_sw32_desc(a); }
 
 // instruction descriptor, kind::f16: D=f32 (bit 4), A=B=f16 (format 0), both K-major, M=128, N=BN
 template <int BN> __device__ __forceinline__ constexpr uint32_t make_idesc() {
@@ -200,7 +178,7 @@ struct TcProblem {
 struct TcParams {
   TcProblem pr[2];
   int nprob;
-  int pdl_flags;
+  int pdl;          // launched with programmatic dependent launch: weight tiles of the first ring pass before pdl_wait
 };
 
 // ---------------------------------------------------------------- epilogues
@@ -551,10 +529,10 @@ __device__ __forceinline__ void rowwise_plain(const TcProblem& p, uint32_t tmem_
 }
 
 // epilogue of the single-CTA kernels (eight epilogue warps)
-template <int BN, int KB>
+template <int BN>
 __device__ __forceinline__ void tc_epilogue(const TcProblem& p, uint32_t tmem_base, int m0, int n0, int n_tile,
                                             int warp, int lane, const float* s_bias, float* tile) {
-  using Cfg = TcCfg<BN, KB>;
+  using Cfg = TcCfg<BN>;
   const int q = warp & 3, hsel = (warp - 2) >> 2;
   if (p.mode == EPI_VOCAB) {
     const int row = m0 + q * 32 + lane;
@@ -569,55 +547,55 @@ __device__ __forceinline__ void tc_epilogue(const TcProblem& p, uint32_t tmem_ba
 // ---------------------------------------------------------------- one ring stage: operand loads and MMA issue
 // Stage layout (same bytes in both modes): A hi16 | A second half | W hi16 | W second half, where the second half is
 // the fp16 residual tile (f16x3) or the two e4m3 tiles hi8 | lo8 (f16+f8x2).
-template <int BN, int KB>
+template <int BN>
 __device__ __forceinline__ void load_w_stage(const TcProblem& p, uint64_t* bar, uint8_t* base, int kb, int n0) {
-  using Cfg = TcCfg<BN, KB>;
+  using Cfg = TcCfg<BN>;
   uint8_t* w = base + 2 * Cfg::kABytes;
-  tma_load_2d(&p.w_hi, bar, w, kb * KB, n0);
+  tma_load_2d(&p.w_hi, bar, w, kb * BK, n0);
   if (p.f8) {
-    tma_load_2d(&p.w_h8, bar, w + Cfg::kWBytes, kb * KB, n0);
-    tma_load_2d(&p.w_lo, bar, w + Cfg::kWBytes + Cfg::kWBytes / 2, kb * KB, n0);
+    tma_load_2d(&p.w_h8, bar, w + Cfg::kWBytes, kb * BK, n0);
+    tma_load_2d(&p.w_lo, bar, w + Cfg::kWBytes + Cfg::kWBytes / 2, kb * BK, n0);
   } else {
-    tma_load_2d(&p.w_lo, bar, w + Cfg::kWBytes, kb * KB, n0);
+    tma_load_2d(&p.w_lo, bar, w + Cfg::kWBytes, kb * BK, n0);
   }
 }
-template <int BN, int KB>
+template <int BN>
 __device__ __forceinline__ void load_a_stage(const TcProblem& p, uint64_t* bar, uint8_t* base, int seg, int kk, int m0) {
-  using Cfg = TcCfg<BN, KB>;
-  tma_load_2d(&p.a_hi[seg], bar, base, kk * KB, m0);
+  using Cfg = TcCfg<BN>;
+  tma_load_2d(&p.a_hi[seg], bar, base, kk * BK, m0);
   if (p.f8) {
-    tma_load_2d(&p.a_h8[seg], bar, base + Cfg::kABytes, kk * KB, m0);
-    tma_load_2d(&p.a_lo[seg], bar, base + Cfg::kABytes + Cfg::kABytes / 2, kk * KB, m0);
+    tma_load_2d(&p.a_h8[seg], bar, base + Cfg::kABytes, kk * BK, m0);
+    tma_load_2d(&p.a_lo[seg], bar, base + Cfg::kABytes + Cfg::kABytes / 2, kk * BK, m0);
   } else {
-    tma_load_2d(&p.a_lo[seg], bar, base + Cfg::kABytes, kk * KB, m0);
+    tma_load_2d(&p.a_lo[seg], bar, base + Cfg::kABytes, kk * BK, m0);
   }
 }
 // the MMAs of one k-block into the accumulator at tmem_acc (first = the k-block overwrites instead of accumulating)
-template <int BN, int KB>
+template <int BN>
 __device__ __forceinline__ void issue_stage(const TcProblem& p, uint32_t tmem_acc, uint32_t base, bool first) {
-  using Cfg = TcCfg<BN, KB>;
+  using Cfg = TcCfg<BN>;
   constexpr uint32_t idesc = make_idesc<BN>();
-  const uint64_t ah = make_kmajor_desc<KB>(base), wh = make_kmajor_desc<KB>(base + 2 * Cfg::kABytes);
+  const uint64_t ah = make_sw128_desc(base), wh = make_sw128_desc(base + 2 * Cfg::kABytes);
   if (p.f8) {
     // x_hi*w_hi on the fp16 path; x_hi8*w_lo8 + x_lo8*w_hi8 on the fp8 path (K = 32 per instruction, twice the rate)
-    const uint64_t a8 = make_kmajor_desc8<KB>(base + Cfg::kABytes), al = make_kmajor_desc8<KB>(base + Cfg::kABytes + Cfg::kABytes / 2);
-    const uint64_t w8 = make_kmajor_desc8<KB>(base + 2 * Cfg::kABytes + Cfg::kWBytes);
-    const uint64_t wl = make_kmajor_desc8<KB>(base + 2 * Cfg::kABytes + Cfg::kWBytes + Cfg::kWBytes / 2);
+    const uint64_t a8 = make_sw64_desc(base + Cfg::kABytes), al = make_sw64_desc(base + Cfg::kABytes + Cfg::kABytes / 2);
+    const uint64_t w8 = make_sw64_desc(base + 2 * Cfg::kABytes + Cfg::kWBytes);
+    const uint64_t wl = make_sw64_desc(base + 2 * Cfg::kABytes + Cfg::kWBytes + Cfg::kWBytes / 2);
 #pragma unroll
-    for (int k = 0; k < KB / UMMA_K; ++k) {
+    for (int k = 0; k < BK / UMMA_K; ++k) {
       const uint64_t off = (uint64_t)((k * UMMA_K * 2) >> 4);     // 32 bytes inside the swizzle row
       umma_f16(tmem_acc, ah + off, wh + off, idesc, (first && k == 0) ? 0u : 1u);
     }
 #pragma unroll
-    for (int k = 0; k < KB / 32; ++k) {
+    for (int k = 0; k < BK / 32; ++k) {
       const uint64_t off = (uint64_t)((k * 32) >> 4);             // 32 e4m3 = 32 bytes
       umma_f8(tmem_acc, a8 + off, wl + off, idesc, 1u);
       umma_f8(tmem_acc, al + off, w8 + off, idesc, 1u);
     }
   } else {
-    const uint64_t al = make_kmajor_desc<KB>(base + Cfg::kABytes), wl = make_kmajor_desc<KB>(base + 2 * Cfg::kABytes + Cfg::kWBytes);
+    const uint64_t al = make_sw128_desc(base + Cfg::kABytes), wl = make_sw128_desc(base + 2 * Cfg::kABytes + Cfg::kWBytes);
 #pragma unroll
-    for (int k = 0; k < KB / UMMA_K; ++k) {
+    for (int k = 0; k < BK / UMMA_K; ++k) {
       const uint64_t off = (uint64_t)((k * UMMA_K * 2) >> 4);     // advance inside the swizzle row
       umma_f16(tmem_acc, ah + off, wh + off, idesc, (first && k == 0) ? 0u : 1u);
       umma_f16(tmem_acc, ah + off, wl + off, idesc, 1u);
@@ -626,9 +604,9 @@ __device__ __forceinline__ void issue_stage(const TcProblem& p, uint32_t tmem_ac
   }
 }
 
-template <int BN, int KB>
+template <int BN>
 __global__ void __launch_bounds__(TC_THREADS, 1) k_gemm_tc(const __grid_constant__ TcParams params) {
-  using Cfg = TcCfg<BN, KB>;
+  using Cfg = TcCfg<BN>;
   extern __shared__ uint8_t smem_raw[];
   __shared__ __align__(8) uint64_t full_bar[Cfg::kStages];
   __shared__ __align__(8) uint64_t empty_bar[Cfg::kStages];
@@ -646,7 +624,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_gemm_tc(const __grid_constant
   const int m_tile = t % p.m_tiles, n_tile = t / p.m_tiles;
   const int m0 = m_tile * BM, n0 = n_tile * BN;
 
-  if (!(params.pdl_flags & 2)) pdl_trigger();
+  pdl_trigger();
   if (p.row_skip != nullptr) {   // all-padding row tiles produce nothing (block-uniform)
     pdl_wait();                  // the flags come from the previous kernel
     int any = 0;
@@ -683,10 +661,10 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_gemm_tc(const __grid_constant
   if (warp == 0) {
     if (lane == 0) {
       // the WEIGHT halves of the first ring pass do not depend on the previous kernel: fetch them, then wait
-      const int pre = !(params.pdl_flags & 1) ? 0 : (total_kb < Cfg::kStages ? total_kb : Cfg::kStages);
+      const int pre = !params.pdl ? 0 : (total_kb < Cfg::kStages ? total_kb : Cfg::kStages);
       for (int kb = 0; kb < pre; ++kb) {
         mbar_expect_tx(&full_bar[kb], Cfg::kStageBytes);
-        load_w_stage<BN, KB>(p, &full_bar[kb], smem + kb * Cfg::kStageBytes, kb, n0);
+        load_w_stage<BN>(p, &full_bar[kb], smem + kb * Cfg::kStageBytes, kb, n0);
       }
       pdl_wait();
       int seg = 0, kk = 0;
@@ -697,9 +675,9 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_gemm_tc(const __grid_constant
         if (kb >= pre) {
           mbar_wait(&empty_bar[st], ph ^ 1);
           mbar_expect_tx(&full_bar[st], Cfg::kStageBytes);
-          load_w_stage<BN, KB>(p, &full_bar[st], base, kb, n0);
+          load_w_stage<BN>(p, &full_bar[st], base, kb, n0);
         }
-        load_a_stage<BN, KB>(p, &full_bar[st], base, seg, kk, m0);
+        load_a_stage<BN>(p, &full_bar[st], base, seg, kk, m0);
         if (++kk == p.kblocks[seg]) { kk = 0; ++seg; }
       }
     }
@@ -711,11 +689,10 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_gemm_tc(const __grid_constant
         const uint32_t ph = (kb / Cfg::kStages) & 1;
         mbar_wait(&full_bar[st], ph);
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        issue_stage<BN, KB>(p, tmem_base, smem_u32(smem + st * Cfg::kStageBytes), kb == 0);
+        issue_stage<BN>(p, tmem_base, smem_u32(smem + st * Cfg::kStageBytes), kb == 0);
         umma_commit(&empty_bar[st]);          // frees the smem slot once these MMAs have read it
       }
       umma_commit(&tmem_full_bar);            // accumulator complete -> epilogue
-      if (params.pdl_flags & 2) pdl_trigger();
     }
     __syncwarp();
   } else {
@@ -729,10 +706,10 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_gemm_tc(const __grid_constant
 #ifdef VSR_DBG_CLK
     const long long tk1 = clock64();
 #endif
-    tc_epilogue<BN, KB>(p, tmem_base, m0, n0, n_tile, warp, lane, s_bias, reinterpret_cast<float*>(smem + Cfg::kRingBytes));
+    tc_epilogue<BN>(p, tmem_base, m0, n0, n_tile, warp, lane, s_bias, reinterpret_cast<float*>(smem + Cfg::kRingBytes));
 #ifdef VSR_DBG_CLK
     if (lane == 0 && warp == 2 && (blockIdx.x == 5 || blockIdx.x == 100) && p.M > 200)
-      printf("gemm BN=%d KB=%d grid=%d cta=%d mode=%d kblocks=%d: main loop %lld cyc, epilogue %lld cyc\n", BN, KB, (int)gridDim.x,
+      printf("gemm BN=%d grid=%d cta=%d mode=%d kblocks=%d: main loop %lld cyc, epilogue %lld cyc\n", BN, (int)gridDim.x,
              (int)blockIdx.x, p.mode, total_kb, tk1 - tk0, clock64() - tk1);
 #endif
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
@@ -759,9 +736,9 @@ __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 
-template <int BN, int KB>
+template <int BN>
 __global__ void __launch_bounds__(TC_THREADS, 1) k_gemm_tcp(const __grid_constant__ TcParams params) {
-  using Cfg = TcCfg<BN, KB>;
+  using Cfg = TcCfg<BN>;
   constexpr int kAccCols = (BN <= 128) ? 128 : 256;     // TMEM column stride between the two accumulators
   constexpr int kTmemCols = 2 * kAccCols;
   extern __shared__ uint8_t smem_raw[];
@@ -777,7 +754,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_gemm_tcp(const __grid_constan
   const int total_tiles = tiles0 + (params.nprob > 1 ? params.pr[1].n_tiles * params.pr[1].m_tiles : 0);
   uint8_t* smem = reinterpret_cast<uint8_t*>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
 
-  if (!(params.pdl_flags & 2)) pdl_trigger();
+  pdl_trigger();
   bool pdl_waited = false;
   for (int q = 0; q < params.nprob; ++q)
     if (params.pr[q].row_skip != nullptr) pdl_waited = true;     // tile skipping reads the previous kernel's flags
@@ -825,10 +802,10 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_gemm_tcp(const __grid_constan
         // first tile of this CTA: weight halves of the first ring pass before the dependency wait (see k_gemm_tc)
         int pre = 0;
         if (!pdl_waited) {
-          pre = !(params.pdl_flags & 1) ? 0 : (total_kb < Cfg::kStages ? total_kb : Cfg::kStages);
+          pre = !params.pdl ? 0 : (total_kb < Cfg::kStages ? total_kb : Cfg::kStages);
           for (int kb = 0; kb < pre; ++kb) {
             mbar_expect_tx(&full_bar[kb], Cfg::kStageBytes);
-            load_w_stage<BN, KB>(p, &full_bar[kb], smem + kb * Cfg::kStageBytes, kb, n0);
+            load_w_stage<BN>(p, &full_bar[kb], smem + kb * Cfg::kStageBytes, kb, n0);
           }
           pdl_wait();
           pdl_waited = true;
@@ -841,9 +818,9 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_gemm_tcp(const __grid_constan
           if (kb >= pre) {
             mbar_wait(&empty_bar[st], ph ^ 1);
             mbar_expect_tx(&full_bar[st], Cfg::kStageBytes);
-            load_w_stage<BN, KB>(p, &full_bar[st], base, kb, n0);
+            load_w_stage<BN>(p, &full_bar[st], base, kb, n0);
           }
-          load_a_stage<BN, KB>(p, &full_bar[st], base, seg, kk, m0);
+          load_a_stage<BN>(p, &full_bar[st], base, seg, kk, m0);
           if (++kk == p.kblocks[seg]) { kk = 0; ++seg; }
         }
       }
@@ -857,18 +834,17 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_gemm_tcp(const __grid_constan
           const uint32_t ph = ((it + kb) / Cfg::kStages) & 1;
           mbar_wait(&full_bar[st], ph);
           asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-          issue_stage<BN, KB>(p, tmem_acc, smem_u32(smem + st * Cfg::kStageBytes), kb == 0);
+          issue_stage<BN>(p, tmem_acc, smem_u32(smem + st * Cfg::kStageBytes), kb == 0);
           umma_commit(&empty_bar[st]);
         }
         umma_commit(&tmem_full_bar[acc]);
-        if ((params.pdl_flags & 2) && tile + (int)gridDim.x >= total_tiles) pdl_trigger();   // last tile of this CTA
       }
       __syncwarp();
     } else {
       epi_bias<BN>(p, m0, n0, n_tile, warp, lane, s_bias, ti != 0);
       mbar_wait(&tmem_full_bar[acc], aph);
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-      tc_epilogue<BN, KB>(p, tmem_acc, m0, n0, n_tile, warp, lane, s_bias, reinterpret_cast<float*>(smem + Cfg::kRingBytes));
+      tc_epilogue<BN>(p, tmem_acc, m0, n0, n_tile, warp, lane, s_bias, reinterpret_cast<float*>(smem + Cfg::kRingBytes));
       asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
       __syncwarp();
       if (lane == 0) mbar_arrive(&tmem_empty_bar[acc]);   // every epilogue warp -> accumulator free again
@@ -886,7 +862,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_gemm_tcp(const __grid_constan
 // x -> (fp16 hi, fp16 lo) with lo = fp16(x - hi)
 // ---------------------------------------------------------------- CTA-pair kernel (cta_group::2), persistent
 // What bounds the single-CTA kernels once the batch is large (ncu on the stacked 400-caption decode: tensor pipe 40-45 %
-// active, L2 -> SM 10-12 TB/s) is operand delivery: a 128 x 128 tile pulls (128 + 128) x KB x 4 bytes through L2 and
+// active, L2 -> SM 10-12 TB/s) is operand delivery: a 128 x 128 tile pulls (128 + 128) x 64 x 4 bytes through L2 and
 // shared memory per k-block, whichever passes are issued.  Here the two CTAs of a cluster (one TPC) compute a 256 x BN
 // tile: each stages its own 128 rows of A and HALF of the W tile (BN / 2 rows); the leader issues tcgen05.mma
 // .cta_group::2 (M = 256), which reads both CTAs' shared memory, and each CTA ends up with its 128 x BN accumulator in
@@ -895,11 +871,10 @@ __global__ void __launch_bounds__(TC_THREADS, 1) k_gemm_tcp(const __grid_constan
 // same shared-memory-tile epilogues as the single-CTA kernels (plain / g_t / LSTM cell 1 at BN = 192 / LSTM cell 2 at 256).
 // VOCAB: the row-per-thread vocabulary epilogue needs no shared-memory tile, which buys one more stage (measured: -2 %).
 // (32-element k-blocks — the same ring bytes in twice as many, finer stages — were measured SLOWER for the fp16-only
-// GEMM-A: 201 vs 179 us on the M=1900, N=6144, K=3072 self-test shape; KB_ stays 64.)
-template <int BN, int KB_ = 64, bool VOCAB = false> struct PairCfg {
-  static constexpr int KB = KB_;
-  static constexpr int kABytes = BM * KB * 2;                 // fp16 tile of this CTA's 128 A rows (the second half of the
-  static constexpr int kWBytes = (BN / 2) * KB * 2;           //   stage holds lo16, or hi8 | lo8); this CTA's half of the W tile
+// GEMM-A: 201 vs 179 us on the M=1900, N=6144, K=3072 self-test shape.)
+template <int BN, bool VOCAB = false> struct PairCfg {
+  static constexpr int kABytes = BM * BK * 2;                 // fp16 tile of this CTA's 128 A rows (the second half of the
+  static constexpr int kWBytes = (BN / 2) * BK * 2;           //   stage holds lo16, or hi8 | lo8); this CTA's half of the W tile
   static constexpr int kStageBytes = 2 * kABytes + 2 * kWBytes;
   static constexpr int kEpiBytes = VOCAB ? 0 : 32 * BN * 4;
   static constexpr int kStages = (227 * 1024 - 2048 - 1024 - kEpiBytes) / kStageBytes;      // (2 KB: static shared memory)
@@ -956,10 +931,9 @@ template <int BN> __device__ __forceinline__ constexpr uint32_t make_idesc_pair(
   return (1u << 4) | ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);
 }
 
-template <int BN, int KB_, bool VOCAB>
+template <int BN, bool VOCAB>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1) k_gemm_pair(const __grid_constant__ TcParams params) {
-  using Cfg = PairCfg<BN, KB_, VOCAB>;
-  constexpr int KB = Cfg::KB;
+  using Cfg = PairCfg<BN, VOCAB>;
   extern __shared__ uint8_t smem_raw[];
   __shared__ __align__(8) uint64_t full_bar[Cfg::kStages];       // waited on in the leader CTA only
   __shared__ __align__(8) uint64_t empty_bar[Cfg::kStages];      // per CTA, signalled by the leader's multicast commits
@@ -1032,16 +1006,16 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1) k_gem
           uint8_t* base = smem + st * Cfg::kStageBytes;
           uint8_t* wb = base + 2 * Cfg::kABytes;
           if (rank == 0) mbar_expect_tx(&full_bar[st], 2 * Cfg::kStageBytes);   // both CTAs' bytes land on the leader's barrier
-          tma_load_2d_pair(&p.a_hi[seg], &full_bar[st], base, kk * KB, m0);
-          tma_load_2d_pair(&p.w_hi, &full_bar[st], wb, kb * KB, wrow);
+          tma_load_2d_pair(&p.a_hi[seg], &full_bar[st], base, kk * BK, m0);
+          tma_load_2d_pair(&p.w_hi, &full_bar[st], wb, kb * BK, wrow);
           if (p.f8) {
-            tma_load_2d_pair(&p.a_h8[seg], &full_bar[st], base + Cfg::kABytes, kk * KB, m0);
-            tma_load_2d_pair(&p.a_lo[seg], &full_bar[st], base + Cfg::kABytes + Cfg::kABytes / 2, kk * KB, m0);
-            tma_load_2d_pair(&p.w_h8, &full_bar[st], wb + Cfg::kWBytes, kb * KB, wrow);
-            tma_load_2d_pair(&p.w_lo, &full_bar[st], wb + Cfg::kWBytes + Cfg::kWBytes / 2, kb * KB, wrow);
+            tma_load_2d_pair(&p.a_h8[seg], &full_bar[st], base + Cfg::kABytes, kk * BK, m0);
+            tma_load_2d_pair(&p.a_lo[seg], &full_bar[st], base + Cfg::kABytes + Cfg::kABytes / 2, kk * BK, m0);
+            tma_load_2d_pair(&p.w_h8, &full_bar[st], wb + Cfg::kWBytes, kb * BK, wrow);
+            tma_load_2d_pair(&p.w_lo, &full_bar[st], wb + Cfg::kWBytes + Cfg::kWBytes / 2, kb * BK, wrow);
           } else {
-            tma_load_2d_pair(&p.a_lo[seg], &full_bar[st], base + Cfg::kABytes, kk * KB, m0);
-            tma_load_2d_pair(&p.w_lo, &full_bar[st], wb + Cfg::kWBytes, kb * KB, wrow);
+            tma_load_2d_pair(&p.a_lo[seg], &full_bar[st], base + Cfg::kABytes, kk * BK, m0);
+            tma_load_2d_pair(&p.w_lo, &full_bar[st], wb + Cfg::kWBytes, kb * BK, wrow);
           }
           if (++kk == p.kblocks[seg]) { kk = 0; ++seg; }
         }
@@ -1073,25 +1047,25 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1) k_gem
           asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
           const uint32_t base = smem_u32(smem + st * Cfg::kStageBytes);
           const uint32_t wbase = base + 2 * Cfg::kABytes;
-          const uint64_t ah = make_kmajor_desc<KB>(base), wh = make_kmajor_desc<KB>(wbase);
+          const uint64_t ah = make_sw128_desc(base), wh = make_sw128_desc(wbase);
           if (p.f8) {
-            const uint64_t a8 = make_kmajor_desc8<KB>(base + Cfg::kABytes), al = make_kmajor_desc8<KB>(base + Cfg::kABytes + Cfg::kABytes / 2);
-            const uint64_t w8 = make_kmajor_desc8<KB>(wbase + Cfg::kWBytes), wl = make_kmajor_desc8<KB>(wbase + Cfg::kWBytes + Cfg::kWBytes / 2);
+            const uint64_t a8 = make_sw64_desc(base + Cfg::kABytes), al = make_sw64_desc(base + Cfg::kABytes + Cfg::kABytes / 2);
+            const uint64_t w8 = make_sw64_desc(wbase + Cfg::kWBytes), wl = make_sw64_desc(wbase + Cfg::kWBytes + Cfg::kWBytes / 2);
 #pragma unroll
-            for (int k = 0; k < KB / UMMA_K; ++k) {
+            for (int k = 0; k < BK / UMMA_K; ++k) {
               const uint64_t off = (uint64_t)((k * UMMA_K * 2) >> 4);
               umma_f16_pair(tmem_acc, ah + off, wh + off, idesc, (kb | k) != 0 ? 1u : 0u);
             }
 #pragma unroll
-            for (int k = 0; k < KB / 32; ++k) {
+            for (int k = 0; k < BK / 32; ++k) {
               const uint64_t off = (uint64_t)((k * 32) >> 4);
               umma_f8_pair(tmem_acc, a8 + off, wl + off, idesc, 1u);
               umma_f8_pair(tmem_acc, al + off, w8 + off, idesc, 1u);
             }
           } else {
-            const uint64_t al = make_kmajor_desc<KB>(base + Cfg::kABytes), wl = make_kmajor_desc<KB>(wbase + Cfg::kWBytes);
+            const uint64_t al = make_sw128_desc(base + Cfg::kABytes), wl = make_sw128_desc(wbase + Cfg::kWBytes);
 #pragma unroll
-            for (int k = 0; k < KB / UMMA_K; ++k) {
+            for (int k = 0; k < BK / UMMA_K; ++k) {
               const uint64_t off = (uint64_t)((k * UMMA_K * 2) >> 4);
               umma_f16_pair(tmem_acc, ah + off, wh + off, idesc, (kb | k) != 0 ? 1u : 0u);
               umma_f16_pair(tmem_acc, ah + off, wl + off, idesc, 1u);
@@ -1171,15 +1145,15 @@ EncodeTiledFn get_encode() {
 }  // namespace
 
 // 2-D fp16 tensor map over a row-major [rows][ld] buffer: box = 64 (K) x box_rows, 128-byte swizzle
-int make_tmap_f16(void* out_map, const void* base, int rows, int cols, int ld, int box_rows, int kb) {
+int make_tmap_f16(void* out_map, const void* base, int rows, int cols, int ld, int box_rows) {
   EncodeTiledFn enc = get_encode();
   VSR_REQUIRE(enc != nullptr, VSR_ECUDA, "cuTensorMapEncodeTiled entry point not available");
   const cuuint64_t gdim[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
   const cuuint64_t gstr[1] = {(cuuint64_t)ld * 2};
-  const cuuint32_t box[2] = {(cuuint32_t)kb, (cuuint32_t)box_rows};
+  const cuuint32_t box[2] = {(cuuint32_t)BK, (cuuint32_t)box_rows};
   const cuuint32_t estr[2] = {1, 1};
   CUresult r = enc((CUtensorMap*)out_map, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void*>(base), gdim, gstr,
-                   box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, kb == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B,
+                   box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
                    CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   VSR_REQUIRE(r == CUDA_SUCCESS, VSR_ECUDA, "cuTensorMapEncodeTiled failed (%d) rows=%d cols=%d ld=%d", (int)r, rows, cols, ld);
   return VSR_OK;
@@ -1206,16 +1180,16 @@ __global__ void k_pick_scale(float* scale) {
   scale[1] = ldexpf(1.f, -e);
 }
 
-// 2-D e4m3 (uint8) tensor map over a row-major [rows][ld] buffer: box = kb (K) x box_rows, rows of kb bytes
-int make_tmap_u8(void* out_map, const void* base, int rows, int cols, int ld, int box_rows, int kb) {
+// 2-D e4m3 (uint8) tensor map over a row-major [rows][ld] buffer: box = 64 (K) x box_rows, 64-byte swizzle
+int make_tmap_u8(void* out_map, const void* base, int rows, int cols, int ld, int box_rows) {
   EncodeTiledFn enc = get_encode();
   VSR_REQUIRE(enc != nullptr, VSR_ECUDA, "cuTensorMapEncodeTiled entry point not available");
   const cuuint64_t gdim[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
   const cuuint64_t gstr[1] = {(cuuint64_t)ld};
-  const cuuint32_t box[2] = {(cuuint32_t)kb, (cuuint32_t)box_rows};
+  const cuuint32_t box[2] = {(cuuint32_t)BK, (cuuint32_t)box_rows};
   const cuuint32_t estr[2] = {1, 1};
   CUresult r = enc((CUtensorMap*)out_map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<void*>(base), gdim, gstr,
-                   box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, kb == 32 ? CU_TENSOR_MAP_SWIZZLE_32B : CU_TENSOR_MAP_SWIZZLE_64B,
+                   box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B,
                    CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   VSR_REQUIRE(r == CUDA_SUCCESS, VSR_ECUDA, "cuTensorMapEncodeTiled (u8) failed (%d) rows=%d cols=%d ld=%d", (int)r, rows, cols, ld);
   return VSR_OK;
@@ -1265,16 +1239,13 @@ int tc_gemm_init() {
   VSR_CHECK_CUDA(cudaGetDevice(&dev));
   const bool done = dev < 64 && ((done_mask >> dev) & 1ull);
   if (done) return VSR_OK;
-#define TC_SET_SMEM(BN_, KB_) VSR_CHECK_CUDA(cudaFuncSetAttribute(k_gemm_tc<BN_, KB_>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcCfg<BN_, KB_>::kSmemBytes))
-  TC_SET_SMEM(256, 64); TC_SET_SMEM(192, 64); TC_SET_SMEM(128, 64);
-  TC_SET_SMEM(256, 32); TC_SET_SMEM(192, 32); TC_SET_SMEM(128, 32);
-  TC_SET_SMEM(144, 64); TC_SET_SMEM(240, 32);
-#define TCP_SET_SMEM(BN_, KB_) VSR_CHECK_CUDA(cudaFuncSetAttribute(k_gemm_tcp<BN_, KB_>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcCfg<BN_, KB_>::kSmemBytes))
-  TCP_SET_SMEM(128, 64); TCP_SET_SMEM(144, 64); TCP_SET_SMEM(192, 32); TCP_SET_SMEM(192, 64); TCP_SET_SMEM(128, 32);
-#undef TCP_SET_SMEM
+#define TC_SET_SMEM(BN_)                                                                                                     \
+  VSR_CHECK_CUDA(cudaFuncSetAttribute(k_gemm_tc<BN_>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcCfg<BN_>::kSmemBytes)); \
+  VSR_CHECK_CUDA(cudaFuncSetAttribute(k_gemm_tcp<BN_>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcCfg<BN_>::kSmemBytes))
+  TC_SET_SMEM(128); TC_SET_SMEM(144); TC_SET_SMEM(192);
 #undef TC_SET_SMEM
-#define PAIR_SET_SMEM(BN_, KB_, V_) VSR_CHECK_CUDA(cudaFuncSetAttribute(k_gemm_pair<BN_, KB_, V_>, cudaFuncAttributeMaxDynamicSharedMemorySize, PairCfg<BN_, KB_, V_>::kSmemBytes))
-  PAIR_SET_SMEM(192, 64, false); PAIR_SET_SMEM(192, 64, true); PAIR_SET_SMEM(256, 64, false);
+#define PAIR_SET_SMEM(BN_, V_) VSR_CHECK_CUDA(cudaFuncSetAttribute(k_gemm_pair<BN_, V_>, cudaFuncAttributeMaxDynamicSharedMemorySize, PairCfg<BN_, V_>::kSmemBytes))
+  PAIR_SET_SMEM(192, false); PAIR_SET_SMEM(192, true); PAIR_SET_SMEM(256, false);
 #undef PAIR_SET_SMEM
   if (dev < 64) done_mask |= 1ull << dev;
   return VSR_OK;
@@ -1351,7 +1322,7 @@ void tc_dbg_clk_report(const char* label) {
 }
 #endif
 
-static int fill_problem(TcProblem* p, const GemmArgs& g, int BN, int kb = 64, bool pair = false) {
+static int fill_problem(TcProblem* p, const GemmArgs& g, int BN, bool pair = false) {
   VSR_REQUIRE(g.M > 0 && g.N >= round_up(g.wb->n_valid, BN), VSR_EINVAL, "launch_gemm_tc: N=%d too small for N tile %d", g.N, BN);
   p->nseg = g.nseg;
   p->f8 = g.f8 ? 1 : 0;
@@ -1363,29 +1334,29 @@ static int fill_problem(TcProblem* p, const GemmArgs& g, int BN, int kb = 64, bo
     VSR_REQUIRE(g.f8 ? (b->hi8 != nullptr && b->lo8 != nullptr) : b->lo != nullptr, VSR_EINVAL,
                 "launch_gemm_tc: segment %d has no %s twin", s, g.f8 ? "e4m3" : "fp16 residual");
     VSR_REQUIRE(b->act_scale == g.seg[0].b->act_scale, VSR_EINVAL, "launch_gemm_tc: segments with different activation scales");
-    memcpy(&p->a_hi[s], kb == 32 ? b->map32_hi : b->map_hi, sizeof(CUtensorMap));
+    memcpy(&p->a_hi[s], b->map_hi, sizeof(CUtensorMap));
     if (g.f8) {
-      memcpy(&p->a_h8[s], kb == 32 ? b->map8_32_hi : b->map8_hi, sizeof(CUtensorMap));
-      memcpy(&p->a_lo[s], kb == 32 ? b->map8_32_lo : b->map8_lo, sizeof(CUtensorMap));
+      memcpy(&p->a_h8[s], b->map8_hi, sizeof(CUtensorMap));
+      memcpy(&p->a_lo[s], b->map8_lo, sizeof(CUtensorMap));
     } else {
-      memcpy(&p->a_lo[s], kb == 32 ? b->map32_lo : b->map_lo, sizeof(CUtensorMap));
+      memcpy(&p->a_lo[s], b->map_lo, sizeof(CUtensorMap));
     }
-    p->kblocks[s] = g.seg[s].k / kb;
+    p->kblocks[s] = g.seg[s].k / BK;
   }
   const bool alt = !pair && BN == g.wb->alt_bn && BN != g.wb->box_rows;
-  if (pair) {       // CTA-pair kernel: half-tile maps (BN / 2 rows), 64-element k-blocks
-    VSR_REQUIRE(g.wb->pair_rows * 2 == BN && kb == 64, VSR_EINVAL, "launch_gemm_tc: weight has no pair maps for N tile %d", BN);
+  if (pair) {       // CTA-pair kernel: half-tile maps (BN / 2 rows)
+    VSR_REQUIRE(g.wb->pair_rows * 2 == BN, VSR_EINVAL, "launch_gemm_tc: weight has no pair maps for N tile %d", BN);
     memcpy(&p->w_hi, g.wb->pair_hi, sizeof(CUtensorMap));
     memcpy(&p->w_lo, g.f8 ? g.wb->pair_lo : g.wb->pair_lo16, sizeof(CUtensorMap));
     if (g.f8) memcpy(&p->w_h8, g.wb->pair_h8, sizeof(CUtensorMap));
   } else {
-  memcpy(&p->w_hi, alt ? g.wb->alt_hi : (kb == 32 ? g.wb->map32_hi : g.wb->map_hi), sizeof(CUtensorMap));
-  if (g.f8) {
-    memcpy(&p->w_h8, alt ? g.wb->alt8_hi : (kb == 32 ? g.wb->map8_32_hi : g.wb->map8_hi), sizeof(CUtensorMap));
-    memcpy(&p->w_lo, alt ? g.wb->alt8_lo : (kb == 32 ? g.wb->map8_32_lo : g.wb->map8_lo), sizeof(CUtensorMap));
-  } else {
-    memcpy(&p->w_lo, alt ? g.wb->alt_lo : (kb == 32 ? g.wb->map32_lo : g.wb->map_lo), sizeof(CUtensorMap));
-  }
+    memcpy(&p->w_hi, alt ? g.wb->alt_hi : g.wb->map_hi, sizeof(CUtensorMap));
+    if (g.f8) {
+      memcpy(&p->w_h8, alt ? g.wb->alt8_hi : g.wb->map8_hi, sizeof(CUtensorMap));
+      memcpy(&p->w_lo, alt ? g.wb->alt8_lo : g.wb->map8_lo, sizeof(CUtensorMap));
+    } else {
+      memcpy(&p->w_lo, alt ? g.wb->alt_lo : g.wb->map_lo, sizeof(CUtensorMap));
+    }
   }
   p->acc_scale = g.wb->scale != nullptr ? g.wb->scale + 1 : nullptr;
   p->act_inv = 1.f / g.seg[0].b->act_scale;
@@ -1431,24 +1402,23 @@ static bool pair_ok(const GemmArgs& g) {
 static int launch_gemm_pair(const GemmArgs& g, const GemmArgs* g2, cudaStream_t st) {
   const int BN = 2 * g.wb->pair_rows;
   const bool vocab = g.cell.mode == EPI_VOCAB;
-  const int kb = 64;
   TcParams p;
   memset(&p, 0, sizeof(p));
-  VSR_TRY(fill_problem(&p.pr[0], g, BN, kb, true));
+  VSR_TRY(fill_problem(&p.pr[0], g, BN, true));
   p.nprob = 1;
   int tiles = p.pr[0].n_tiles * ((p.pr[0].m_tiles + 1) / 2);
   if (g2 != nullptr) {
-    VSR_TRY(fill_problem(&p.pr[1], *g2, BN, kb, true));
+    VSR_TRY(fill_problem(&p.pr[1], *g2, BN, true));
     p.nprob = 2;
     tiles += p.pr[1].n_tiles * ((p.pr[1].m_tiles + 1) / 2);
   }
   static int sms = 0;
   if (sms == 0) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, 0);
   const int clusters = tiles < sms / 2 ? tiles : sms / 2;
-#define PAIR_LAUNCH(BN_, KB_, V_) VSR_CHECK_CUDA(launch_k(k_gemm_pair<BN_, KB_, V_>, dim3(2 * clusters), dim3(TC_THREADS), PairCfg<BN_, KB_, V_>::kSmemBytes, st, g.pdl, p))
-  if (BN == 192 && vocab) PAIR_LAUNCH(192, 64, true);
-  else if (BN == 192) PAIR_LAUNCH(192, 64, false);
-  else PAIR_LAUNCH(256, 64, false);
+#define PAIR_LAUNCH(BN_, V_) VSR_CHECK_CUDA(launch_k(k_gemm_pair<BN_, V_>, dim3(2 * clusters), dim3(TC_THREADS), PairCfg<BN_, V_>::kSmemBytes, st, g.pdl, p))
+  if (BN == 192 && vocab) PAIR_LAUNCH(192, true);
+  else if (BN == 192) PAIR_LAUNCH(192, false);
+  else PAIR_LAUNCH(256, false);
 #undef PAIR_LAUNCH
   VSR_CHECK_CUDA(cudaGetLastError());
   return VSR_OK;
@@ -1459,12 +1429,10 @@ int launch_gemm_tc(const GemmArgs& g, const GemmArgs* g2, cudaStream_t st) {
   VSR_TRY(tc_gemm_init());
   if (pair_ok(g) && (g2 == nullptr || (pair_ok(*g2) && g2->wb->pair_rows == g.wb->pair_rows))) return launch_gemm_pair(g, g2, st);
   int BN = g.wb->box_rows;
-  VSR_REQUIRE(BN == 128 || BN == 192 || BN == 256, VSR_EINVAL, "launch_gemm_tc: unsupported N tile %d", BN);
+  VSR_REQUIRE(BN == 128 || BN == 144 || BN == 192, VSR_EINVAL, "launch_gemm_tc: unsupported N tile %d", BN);
   VSR_REQUIRE(g2 == nullptr || g2->wb->box_rows == BN, VSR_EINVAL, "launch_gemm_tc: grouped problems need one tile shape");
   TcParams p;            // ~2.7 KB; passed by value at launch
   memset(&p, 0, sizeof(p));
-  int kb = g.wb->kb;          // k-block (64 or 32 fp16) chosen per weight at pack time
-  VSR_REQUIRE(g2 == nullptr || g2->wb->kb == kb, VSR_EINVAL, "launch_gemm_tc: grouped problems need one k-block size");
   // Tile choice: operand delivery bounds these GEMMs, so a tile costs ~ (BM + BN) and a launch costs
   // waves(tiles / 148 SMs) * (BM + BN).  Take the alternative N tile when that is cheaper.
   if (g.wb->alt_bn > 0 && !g.no_alt && (g.cell.mode == 0 || g.cell.mode == EPI_VOCAB) && (g2 == nullptr || (g2->wb->alt_bn == g.wb->alt_bn && g2->cell.mode == 0))) {
@@ -1476,44 +1444,31 @@ int launch_gemm_tc(const GemmArgs& g, const GemmArgs* g2, cudaStream_t st) {
       if (g2 != nullptr) tiles += ((g2->M + BM - 1) / BM) * ((g2->wb->n_valid + bn - 1) / bn);
       return ((tiles + sms - 1) / sms) * (BM + bn);
     };
-    if (cost(g.wb->alt_bn) < cost(BN)) { BN = g.wb->alt_bn; kb = g.wb->alt_kb; }
+    if (cost(g.wb->alt_bn) < cost(BN)) BN = g.wb->alt_bn;
   }
-  VSR_TRY(fill_problem(&p.pr[0], g, BN, kb));
+  VSR_TRY(fill_problem(&p.pr[0], g, BN));
   p.nprob = 1;
-  p.pdl_flags = g.pdl_flags;
+  p.pdl = g.pdl ? 1 : 0;
   int tiles = p.pr[0].n_tiles * p.pr[0].m_tiles;
   if (g2 != nullptr) {
-    VSR_TRY(fill_problem(&p.pr[1], *g2, BN, kb));
+    VSR_TRY(fill_problem(&p.pr[1], *g2, BN));
     p.nprob = 2;
     tiles += p.pr[1].n_tiles * p.pr[1].m_tiles;
   }
-  static int persist = -1, sms = 148;
-  if (persist < 0) {
-    const char* e = getenv("VSRDEC_PERSIST");
-    persist = (e == nullptr) ? 1 : atoi(e);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, 0);
-  }
+  static int sms = 0;
+  if (sms == 0) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, 0);
   // persistent tiles pay off only when a CTA gets more than one tile (epilogue / main-loop overlap);
   // for single-wave launches the plain kernel measured 5-10 % faster
   // (and measured neutral-to-worse for the grouped two-problem launch, whose tiles are uneven)
-  if (persist && tiles > sms && g2 == nullptr && (BN == 128 || BN == 144 || BN == 192)) {
-    const int grid = tiles < sms ? tiles : sms;
-#define TCP_LAUNCH(BN_, KB_) VSR_CHECK_CUDA(launch_k(k_gemm_tcp<BN_, KB_>, dim3(grid), dim3(TC_THREADS), TcCfg<BN_, KB_>::kSmemBytes, st, g.pdl, p))
-    if (BN == 144) TCP_LAUNCH(144, 64);
-    else if (BN == 192) { if (kb == 32) TCP_LAUNCH(192, 32); else TCP_LAUNCH(192, 64); }
-    else { if (kb == 32) TCP_LAUNCH(128, 32); else TCP_LAUNCH(128, 64); }
+  if (tiles > sms && g2 == nullptr) {
+#define TCP_LAUNCH(BN_) VSR_CHECK_CUDA(launch_k(k_gemm_tcp<BN_>, dim3(sms), dim3(TC_THREADS), TcCfg<BN_>::kSmemBytes, st, g.pdl, p))
+    if (BN == 144) TCP_LAUNCH(144); else if (BN == 192) TCP_LAUNCH(192); else TCP_LAUNCH(128);
 #undef TCP_LAUNCH
     VSR_CHECK_CUDA(cudaGetLastError());
     return VSR_OK;
   }
-#define TC_LAUNCH(BN_, KB_) VSR_CHECK_CUDA(launch_k(k_gemm_tc<BN_, KB_>, dim3(tiles), dim3(TC_THREADS), TcCfg<BN_, KB_>::kSmemBytes, st, g.pdl, p))
-  if (BN == 144) TC_LAUNCH(144, 64);
-  else if (BN == 240) TC_LAUNCH(240, 32);
-  else if (kb == 32) {
-    if (BN == 256) TC_LAUNCH(256, 32); else if (BN == 192) TC_LAUNCH(192, 32); else TC_LAUNCH(128, 32);
-  } else {
-    if (BN == 256) TC_LAUNCH(256, 64); else if (BN == 192) TC_LAUNCH(192, 64); else TC_LAUNCH(128, 64);
-  }
+#define TC_LAUNCH(BN_) VSR_CHECK_CUDA(launch_k(k_gemm_tc<BN_>, dim3(tiles), dim3(TC_THREADS), TcCfg<BN_>::kSmemBytes, st, g.pdl, p))
+  if (BN == 144) TC_LAUNCH(144); else if (BN == 192) TC_LAUNCH(192); else TC_LAUNCH(128);
 #undef TC_LAUNCH
   VSR_CHECK_CUDA(cudaGetLastError());
   return VSR_OK;

@@ -5,6 +5,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <numeric>
 #include <vector>
 
 #include "common.cuh"
@@ -26,22 +27,17 @@ static void make_pair(F16Pair* b, const float* f, int rows, int ld, int box, boo
   CK(cudaMalloc(&b->hi, (size_t)rows * ld * 2));
   b->rows = rows; b->ld = ld; b->box_rows = box; b->n_valid = rows;
   VK(make_tmap_f16(b->map_hi, b->hi, rows, ld, ld, box));
-  VK(make_tmap_f16(b->map32_hi, b->hi, rows, ld, ld, box, 32));
   if (!f8) {
     CK(cudaMalloc(&b->lo, (size_t)rows * ld * 2));
     VK(make_tmap_f16(b->map_lo, b->lo, rows, ld, ld, box));
-    VK(make_tmap_f16(b->map32_lo, b->lo, rows, ld, ld, box, 32));
   } else {
     CK(cudaMalloc(&b->hi8, (size_t)rows * ld)); CK(cudaMalloc(&b->lo8, (size_t)rows * ld));
     VK(make_tmap_u8(b->map8_hi, b->hi8, rows, ld, ld, box));
     VK(make_tmap_u8(b->map8_lo, b->lo8, rows, ld, ld, box));
-    VK(make_tmap_u8(b->map8_32_hi, b->hi8, rows, ld, ld, box, 32));
-    VK(make_tmap_u8(b->map8_32_lo, b->lo8, rows, ld, ld, box, 32));
   }
   b->act_scale = (!weight && f8) ? ACT_SCALE_F8 : 1.f;
   if (weight) CK(cudaMalloc(&b->scale, 2 * sizeof(float)));     // weights: power-of-two scaled split
   VK(launch_split_pair(f, *b, (size_t)rows * ld, 0, weight));
-  b->kb = getenv("VSRDEC_KB") && atoi(getenv("VSRDEC_KB")) == 32 ? 32 : 64;
 }
 
 static bool g_time = true;
@@ -49,6 +45,7 @@ static bool g_f8 = false;
 static bool g_pair = false;      // CTA-pair kernel (needs M >= 1024; BN = pair tile width)
 static bool g_vocab = false;     // vocabulary-head epilogue (logits + chunk records; the logits are checked)
 static int run_case(int M, int N, int nseg, const int* ks, bool extras, int BN, float wscale = 0.05f) {
+  N = round_up(N, std::lcm(BN, 64));     // whole N tiles of both GEMMs (the FFMA GEMM's tiles are 64 wide)
   const int Mp = (M + 127) / 128 * 128;
   int K = 0; for (int s = 0; s < nseg; ++s) K += ks[s];
   float* W = dev_rand((size_t)N * K, wscale, 1);
@@ -127,7 +124,7 @@ int main(int argc, char** argv) {
     run_case(500, 5632, 1, kb, true, 128);    // B2
     run_case(500, 4096, 2, kd, true, 128);    // D
     run_case(500, 10240, 1, kb, true, 128);   // E
-    run_case(500, 6144, 3, ka, true, 256);    // A, BN=256
+    run_case(500, 6144, 3, ka, true, 192);    // A, BN=192
     return 0;
   }
   const int k1[] = {64}, k2[] = {1024}, k3[] = {1024, 1024, 1024}, k4[] = {2048, 1024}, k5[] = {64, 64, 64};
@@ -146,7 +143,8 @@ int main(int argc, char** argv) {
       g_f8 = pass == 1;
       g_pair = false;
       bad += run_case(300, 512, 1, k2, true, 128);
-      bad += run_case(300, 768, 3, k5, true, 256);
+      bad += run_case(300, 768, 3, k5, true, 192);
+      bad += run_case(300, 768, 1, k2, true, 144);
       g_pair = true;
       bad += run_case(1100, 512, 1, k2, true, 256);
       bad += run_case(1100, 768, 3, k5, true, 192);
@@ -154,10 +152,10 @@ int main(int argc, char** argv) {
     printf("%s\n", bad ? "SELFTEST FAILED" : "SELFTEST PASSED");
     return bad ? 1 : 0;
   }
-  const int bns[2] = {256, 128};
-  for (int pass = 0; pass < 4; ++pass) {
-    const int BN = bns[pass & 1];
-    g_f8 = pass >= 2;
+  const int bns[3] = {128, 192, 144};     // the single-CTA kernel's tiles: B / C / D / E, A, the vocabulary GEMM's alternative
+  for (int pass = 0; pass < 6; ++pass) {
+    const int BN = bns[pass % 3];
+    g_f8 = pass >= 3;
     bad += run_case(128, 256, 1, k1, false, BN);
     bad += run_case(100, 256, 3, k5, true, BN);
     bad += run_case(500, 512, 1, k2, false, BN);

@@ -7,7 +7,6 @@
 
 #include <cuda_fp16.h>
 
-#include <cstdlib>
 #include <cstring>
 #include <type_traits>
 #include "common.cuh"
@@ -738,6 +737,9 @@ int run_vocab_rows(Ctx* c, const F16Pair& a_b, float* logits, int M, float* out_
 // ---------------------------------------------------------------- one decoder step (host side)
 static PairOut pair_out(const Ctx* c, const F16Pair& b) { return twin_out(&b, c->use_tc); }
 
+// B, D + C and E take the CTA-pair kernel from this many rows (measured: slower at 500 rows, 6 % faster at 1000)
+constexpr int PAIR_MIN_ROWS = 640;
+
 int run_step(Ctx* c, const StepIO& io, cudaStream_t st) {
   const int rows = io.rows, H = c->H;
   VSR_REQUIRE(rows > 0 && rows <= c->cap_rows, VSR_ESTATE, "run_step: rows=%d cap=%d", rows, c->cap_rows);
@@ -758,14 +760,13 @@ int run_step(Ctx* c, const StepIO& io, cudaStream_t st) {
     g.rowadd = c->U; g.ld_rowadd = c->NA; g.row_div = io.cur_beam; g.rowadd_mul = (c->n_img == 1 ? 0 : 1);
     g.c = c->pre1; g.ldc = c->NA; g.M = rows; g.N = c->NA;
     g.zero_acc = io.zero_state;           // [h2 | h1] = 0 at t = 0: pre1 = U[caption] + X[bos], no main loop
-    g.pdl = c->use_pdl && (c->pdl_mode & 1); g.pdl_flags = ((c->pdl_mode & 4) ? 1 : 0) | ((c->pdl_mode & 8) ? 2 : 0);
+    g.pdl = c->use_pdl;
     g.allow_pair = true;
     // GEMM-A runs on the CTA-pair kernel at EVERY row count (its 32 N tiles fill the machine from 2 row tiles on, and
     // below that the pair splits the weight stream over two SMs: faster than the single-CTA kernel at 100, 500 and 5000
-    // rows alike), with the residual passes in fp8.  One kernel and one operand mode at every batch size keeps a
-    // caption's result independent of what else is in the batch.  (On the single-CTA kernel its 192-wide tile only fits
-    // 32-element k-blocks, whose 32-byte e4m3 rows load poorly: that path keeps three fp16 passes, VSRDEC_PAIR=0.)
-    g.f8 = c->gemm_f8 && c->use_pair; g.pair_min_rows = 1;
+    // rows alike).  One kernel and one operand mode at every batch size keeps a caption's result independent of what
+    // else is in the batch.  Only the t = 0 launch (zero_acc: no main loop) takes the single-CTA kernel.
+    g.f8 = c->gemm_f8; g.pair_min_rows = 1;
     fused = gemm_uses_tc(c, g);
     c->state_h32 = !fused || io.need_h32;
     if (fused) {   // LSTM cell 1 + sentinel gate in the epilogue: pre1 is never written
@@ -792,14 +793,14 @@ int run_step(Ctx* c, const StepIO& io, cudaStream_t st) {
     g.c = c->sent; g.ldc = c->NB1; g.M = rows; g.N = c->NB1;
     GemmArgs g2{};
     g2.nseg = 1; g2.seg[0] = {c->h1n, c->Hp, c->Hp, c->Hp, &c->h1n_b};
-    g2.w = c->WB2; g2.ldw = c->Hp; g2.wb = &c->WB2_b; g2.f8 = c->gemm_f8; g2.allow_pair = true; g2.pair_min_rows = c->pair_min_rows;
+    g2.w = c->WB2; g2.ldw = c->Hp; g2.wb = &c->WB2_b; g2.f8 = c->gemm_f8; g2.allow_pair = true; g2.pair_min_rows = PAIR_MIN_ROWS;
     g2.c = c->hb; g2.ldc = c->NB2; g2.M = rows; g2.N = c->NB2;
     if (fused) {   // g_t = sig(gq + W1_hg.h1') * tanh(c1') on the hg column block of the h1' projection
       g2.cell.gt_cols = c->oB2_ha; g2.cell.gt_gq = c->gq; g2.cell.gt_c1n = c->c1n; g2.cell.g_t = nullptr;
       g2.cell.g_b = &c->g_t_b; g2.cell.ld_state = c->Hp;
     }
-    g.pdl = c->use_pdl && (c->pdl_mode & 1); g.pdl_flags = ((c->pdl_mode & 4) ? 1 : 0) | ((c->pdl_mode & 8) ? 2 : 0);
-    g.f8 = c->gemm_f8; g.allow_pair = true; g.pair_min_rows = c->pair_min_rows;
+    g.pdl = c->use_pdl;
+    g.f8 = c->gemm_f8; g.allow_pair = true; g.pair_min_rows = PAIR_MIN_ROWS;
     VSR_TRY(launch_gemm(c, g, st, &g2)); c->launches += fused ? 1 : 2;   // one grouped launch on tensor cores
   }
   if (!fused) {
@@ -829,7 +830,7 @@ int run_step(Ctx* c, const StepIO& io, cudaStream_t st) {
     }
     VSR_REQUIRE(smem <= 200 * 1024, VSR_EINVAL, "attention tile (R=%d x A=%d) does not fit shared memory", c->R, c->A);
     const int ki = c->feat_dtype == VSR_DT_F16 ? 1 : c->feat_dtype == VSR_DT_BF16 ? 2 : 0;
-    VSR_CHECK_CUDA(launch_k(kern[ki], dim3(rows), dim3(ATT_THREADS), smem, st, c->use_pdl && (c->pdl_mode & 2), a));
+    kern[ki]<<<rows, ATT_THREADS, smem, st>>>(a);
     VSR_CHECK_CUDA(cudaGetLastError()); c->launches++;
   }
   {  // D: pre2 = WD . [att | h2_old | h1'] + b (+ U2[img]);  C: ga = att_ga . g_t rides in the same launch
@@ -837,7 +838,7 @@ int run_step(Ctx* c, const StepIO& io, cudaStream_t st) {
     PhaseScope ps(c, PH_GEMM_D, st);
     GemmArgs gc{};
     gc.nseg = 1; gc.seg[0] = {c->g_t, c->Hp, c->Hp, c->Hp, &c->g_t_b};
-    gc.w = c->WC; gc.ldw = c->Hp; gc.wb = &c->WC_b; gc.f8 = c->gemm_f8; gc.allow_pair = true; gc.pair_min_rows = c->pair_min_rows;
+    gc.w = c->WC; gc.ldw = c->Hp; gc.wb = &c->WC_b; gc.f8 = c->gemm_f8; gc.allow_pair = true; gc.pair_min_rows = PAIR_MIN_ROWS;
     gc.c = c->ga; gc.ldc = c->NC; gc.M = rows; gc.N = c->NC;
     GemmArgs g{};
     g.nseg = io.zero_state ? 2 : 3;       // h2 = 0 at t = 0: its K segment (last in WD) is not read
@@ -853,8 +854,8 @@ int run_step(Ctx* c, const StepIO& io, cudaStream_t st) {
       g.cell.mode = 2; g.cell.c_old = c->c2; g.cell.c_new = c->c2n; g.cell.h_new = io.need_h32 ? c->h2n : nullptr;
       g.cell.h_b = &c->h2n_b; g.cell.ld_state = c->Hp;
     }
-    g.pdl = c->use_pdl && (c->pdl_mode & 1); g.pdl_flags = ((c->pdl_mode & 4) ? 1 : 0) | ((c->pdl_mode & 8) ? 2 : 0);
-    g.f8 = c->gemm_f8; g.allow_pair = true; g.pair_min_rows = c->pair_min_rows;
+    g.pdl = c->use_pdl;
+    g.f8 = c->gemm_f8; g.allow_pair = true; g.pair_min_rows = PAIR_MIN_ROWS;
     VSR_TRY(launch_gemm(c, g, st, &gc)); c->launches += fused ? 1 : 2;
   }
   if (!fused) {
@@ -865,16 +866,15 @@ int run_step(Ctx* c, const StepIO& io, cudaStream_t st) {
   if (io.skip_vocab) return VSR_OK;     // batched forward: the vocabulary projection of all steps runs after the loop
   // Fused vocabulary head (tensor-core path, nobody needs full log-prob rows): the GEMM epilogue also reduces
   // every tile to a softmax record and k_vocab_merge finishes the row without scanning the logits.
-  static const bool fuse_enabled = [] { const char* e = getenv("VSRDEC_FUSE_VOCAB"); return e == nullptr || atoi(e) != 0; }();
-  const bool fuse_vocab = fuse_enabled && fused && io.out_logp == nullptr && io.topk > 0;
+  const bool fuse_vocab = fused && io.out_logp == nullptr && io.topk > 0;
   {  // E: logits = out_fc . h2' + b
     PhaseScope ps(c, PH_GEMM_E, st);
     GemmArgs g{};
     g.nseg = 1; g.seg[0] = {c->h2n, c->Hp, c->Hp, c->Hp, &c->h2n_b};
     g.w = c->WE; g.ldw = c->Hp; g.bias = c->bE; g.wb = &c->WE_b;
     g.c = c->logits; g.ldc = c->NE; g.M = rows; g.N = c->NE;
-    g.pdl = c->use_pdl && (c->pdl_mode & 1); g.pdl_flags = ((c->pdl_mode & 4) ? 1 : 0) | ((c->pdl_mode & 8) ? 2 : 0);
-    g.f8 = c->gemm_f8; g.allow_pair = true; g.pair_min_rows = c->pair_min_rows;
+    g.pdl = c->use_pdl;
+    g.f8 = c->gemm_f8; g.allow_pair = true; g.pair_min_rows = PAIR_MIN_ROWS;
     if (fuse_vocab) {
       g.cell.mode = 3; g.cell.vocab_part = c->vpart;
     }
@@ -886,10 +886,9 @@ int run_step(Ctx* c, const StepIO& io, cudaStream_t st) {
     a.out_logp = io.out_logp; a.out_stride = io.out_stride;
     a.gate_out = io.gate_out; a.gate_stride = io.gate_stride;
     if (fuse_vocab) {
-      VSR_CHECK_CUDA(launch_k(k_vocab_merge, dim3((rows + VM_WARPS - 1) / VM_WARPS), dim3(VM_WARPS * 32), 0, st, c->use_pdl && (c->pdl_mode & 2),
-                              a, (const float*)c->vpart, c->NE / 16));
+      k_vocab_merge<<<(rows + VM_WARPS - 1) / VM_WARPS, VM_WARPS * 32, 0, st>>>(a, c->vpart, c->NE / 16);
     } else {
-      VSR_CHECK_CUDA(launch_k(k_softmax_topk, dim3(rows), dim3(SM_THREADS), 0, st, c->use_pdl && (c->pdl_mode & 2), a));
+      k_softmax_topk<<<rows, SM_THREADS, 0, st>>>(a);
     }
     VSR_CHECK_CUDA(cudaGetLastError()); c->launches++;
   }

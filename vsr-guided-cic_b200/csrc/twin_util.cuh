@@ -37,7 +37,7 @@ int make_pair(F16Pair* b, int rows, int ld, bool weight) {
   VSR_CHECK_CUDA(cudaMemset(b->hi, 0, (size_t)rows * ld * 2));
   VSR_CHECK_CUDA(cudaMemset(b->lo, 0, (size_t)rows * ld * 2));
   if (weight) VSR_CHECK_CUDA(cudaMalloc((void**)&b->scale, 2 * sizeof(float)));
-  b->rows = rows; b->ld = ld; b->box_rows = 128; b->kb = 64; b->n_valid = rows; b->act_scale = 1.f; b->alt_bn = 0; b->pair_rows = 0;
+  b->rows = rows; b->ld = ld; b->box_rows = 128; b->n_valid = rows; b->act_scale = 1.f; b->alt_bn = 0; b->pair_rows = 0;
   VSR_TRY(make_tmap_f16(b->map_hi, b->hi, rows, ld, ld, 128));
   VSR_TRY(make_tmap_f16(b->map_lo, b->lo, rows, ld, ld, 128));
   return VSR_OK;

@@ -259,6 +259,29 @@ int vsr_sample_ex(vsr_handle h, const VsrSampleParams* p, int64_t* out_words, in
 int vsr_set_attention_capture(vsr_handle h, int32_t enabled);
 int vsr_get_attention(vsr_handle h, float* alpha, int32_t* slot, void* stream);
 
+/* No-repeat n-gram blocking: a handle setting (like vsr_set_attention_capture) that applies to the decode drivers that
+ * choose words, vsr_beam_search, vsr_greedy, vsr_sample and vsr_sample_ex (not vsr_step or vsr_forward_teacher).
+ * n = 0 is off (the default): outputs, launches and graph replay are exactly those of a handle that never set it.
+ * With block size n >= 1, a row's emitted words y_0 .. y_{t-1} are the words it picked at steps 0 .. t-1 (for beam
+ * search the word path of the row's own beam, following the back-pointers; gates and BOS are not part of it).  At step
+ * t, word w is BANNED for the row when some i with 0 <= i <= t - n has y_i .. y_{i+n-2} = y_{t-n+1} .. y_{t-1} and
+ * y_{i+n-1} = w.  For n = 1 every word already emitted is banned.
+ *   - A banned word cannot be selected.  Beam search: it is not among the row's word candidates (the top-k stays exact
+ *     over the words that are not banned, ties in (value desc, index asc) order as always).  Greedy: the pick is the
+ *     best word that is not banned.  Sampling (vsr_sample_ex): banned entries leave the row before steps 1-5, as if
+ *     x_w = -inf, so K and P are taken over the words that are not banned.
+ *   - Log-probs do not change: lp_words, the beam scores and the traced rows (VsrTrace.step_out) stay the model's own
+ *     log-softmax over the full vocabulary, as the sampling log-probs ignore truncation.
+ *   - A verb-forced row (use_verbs) takes the forced word even if it completes a banned n-gram; beams frozen by the
+ *     double-EOS path (CaptioningModel.py:146-150) keep their synthetic candidates; blocking continues after a word EOS,
+ *     since those beams keep expanding.
+ *   - Each caption decodes to the same bits alone or with others, and sampling draw j is the same for every n > j.
+ * Limits (VSR_EINVAL, nothing enqueued): 0 <= n <= seq_len here; with n >= 1, vsr_beam_search needs
+ * vocab_size >= beam_size + seq_len - 1 and vsr_greedy / vsr_sample(_ex) need vocab_size >= seq_len, so that every row
+ * keeps enough words that are not banned.  While on, the handle keeps a [rows][seq_len] int32 history of the decode's
+ * words (two of them for beam search), allocated at the first decode that needs it. */
+int vsr_set_no_repeat_ngram(vsr_handle h, int32_t n);
+
 /* Number of kernels this handle has launched so far (bench.py's gpu_launches). */
 int64_t vsr_launch_count(vsr_handle h);
 

@@ -179,6 +179,18 @@ int ensure_beam_ws(Ctx* c, int caps, int T) {
   return VSR_OK;
 }
 
+// n-gram blocking histories of `rows` rows (grow-only; both buffers of the pair)
+int ensure_whist(Ctx* c, int rows) {
+  if (rows <= c->cap_whist) return VSR_OK;
+  dev_free(c, c->whist); dev_free(c, c->whist_n);
+  c->whist = c->whist_n = nullptr; c->cap_whist = 0;
+  const size_t n = (size_t)rows * c->d.seq_len;
+  VSR_TRY(dev_alloc(c, (void**)&c->whist, sizeof(int32_t) * n));
+  VSR_TRY(dev_alloc(c, (void**)&c->whist_n, sizeof(int32_t) * n));
+  c->cap_whist = rows;
+  return VSR_OK;
+}
+
 // grow-only capture buffers for a decode of T steps with up to step_rows rows per step (and a back-tracked path of
 // path entries); clears what the previous decode left.  Nothing is allocated while capture is off.
 static int attn_begin(Ctx* c, int64_t step_rows, int T, size_t path) {
@@ -513,6 +525,7 @@ static int enqueue_beam_steps(Ctx* c, int k, const int64_t* eos, int use_verbs, 
     StepIO io{};
     io.rows = rows; io.cur_beam = cur; io.use_verbs = use_verbs != 0; io.gt = gt != 0; io.topk = k;
     io.zero_state = t == 0;
+    io.ngram_block = c->ngram > 0; io.t = t;
     if (tr && tr->step_out) { io.out_logp = tr->step_out + (size_t)t * b * k * c->V; io.out_stride = c->V; }
     if (tr && tr->step_gate) { io.gate_out = tr->step_gate + (size_t)t * b * k * 2; io.gate_stride = 2; }
     attn_step_io(c, io, t, (int64_t)b * k);
@@ -534,6 +547,7 @@ static int beam_steps_graphed(Ctx* c, int k, const int64_t* eos, int use_verbs, 
   Ctx::GraphKey key = graph_key(c, 0);
   key.eos0 = eos[0]; key.eos1 = eos[1];
   key.k = k; key.use_verbs = use_verbs; key.gt = gt; key.T = c->d.seq_len; key.attn = c->attn_capture;
+  key.ngram = c->ngram;
   return run_graphed(c, key, st, [&](cudaStream_t s) { return enqueue_beam_steps(c, k, eos, use_verbs, gt, nullptr, s); });
 }
 
@@ -550,7 +564,10 @@ static int beam_search_impl(Ctx* c, int k, int out_size, const int64_t* eos, int
   VSR_REQUIRE(eos && out_words && out_gates && lp_words && lp_gates, VSR_EINVAL, "vsr_beam_search: null argument");
   VSR_REQUIRE(!use_verbs || c->verbs != nullptr, VSR_EINVAL, "vsr_beam_search: use_verbs without a verbs tensor");
   const int b = c->b, T = c->d.seq_len;
+  VSR_REQUIRE(c->ngram == 0 || c->V >= k + T - 1, VSR_EINVAL, "vsr_beam_search: n-gram blocking needs vocab_size (%d) >= "
+              "beam + seq_len - 1 (%d), so that every row keeps beam words that are not banned", c->V, k + T - 1);
   VSR_TRY(ensure_rows(c, b * k));
+  if (c->ngram > 0) VSR_TRY(ensure_whist(c, b * k));
   VSR_TRY(ensure_beam_ws(c, b, T));
   VSR_TRY(attn_begin(c, (int64_t)b * k, T, (size_t)b * out_size * T));
   c->hist_T = T; c->hist_b = b; c->hist_k = k;
@@ -604,7 +621,7 @@ static int enqueue_forward_steps(Ctx* c, const int64_t* captions, int T, bool ba
       io.gate_out = gate + (size_t)t * 2; io.gate_stride = (int64_t)T * 2;
       VSR_TRY(run_step(c, io, st));
     }
-    if (t + 1 < T) VSR_TRY(launch_commit_identity(c, b, captions + (t + 1), T, t + 1, st));
+    if (t + 1 < T) VSR_TRY(launch_commit_identity(c, b, captions + (t + 1), T, t + 1, -1, st));
   }
   if (batched) VSR_TRY(run_vocab_rows(c, c->h2all_b, c->logits_all, b * T, nullptr, st, false));   // M = b*T rows
   return VSR_OK;
@@ -642,7 +659,10 @@ static int greedy_impl(Ctx* c, int64_t* out_words, int64_t* out_gates, cudaStrea
   VSR_REQUIRE(c->have_prologue, VSR_ESTATE, "vsr_greedy: call vsr_prologue first");
   VSR_REQUIRE(out_words && out_gates, VSR_EINVAL, "vsr_greedy: null argument");
   const int b = c->b, T = c->d.seq_len;
+  VSR_REQUIRE(c->ngram == 0 || c->V >= T, VSR_EINVAL, "vsr_greedy: n-gram blocking needs vocab_size (%d) >= seq_len (%d)",
+              c->V, T);
   VSR_TRY(ensure_rows(c, b));
+  if (c->ngram > 0) VSR_TRY(ensure_whist(c, b));
   VSR_TRY(ensure_beam_ws(c, b, T));
   VSR_TRY(attn_begin(c, b, T, 0));
   VSR_TRY(launch_state_init(c, b, st));
@@ -650,10 +670,11 @@ static int greedy_impl(Ctx* c, int64_t* out_words, int64_t* out_gates, cudaStrea
     StepIO io{};
     io.rows = b; io.cur_beam = 1; io.use_verbs = false; io.gt = false; io.topk = 1;
     io.zero_state = t == 0;
+    io.ngram_block = c->ngram > 0; io.t = t;
     attn_step_io(c, io, t, b);
     VSR_TRY(run_step(c, io, st));
     VSR_TRY(launch_greedy_pick(c, b, t, T, out_words, out_gates, st));
-    if (t + 1 < T) VSR_TRY(launch_commit_identity(c, b, nullptr, 0, -1, st));
+    if (t + 1 < T) VSR_TRY(launch_commit_identity(c, b, nullptr, 0, -1, c->ngram > 0 ? t : -1, st));
   }
   attn_done(c, false, T, b, b);
   return VSR_OK;
@@ -675,9 +696,12 @@ static int sample_impl(Ctx* c, const VsrSampleParams& p, int64_t* out_words, int
   const int b = c->b, T = c->d.seq_len;
   VSR_REQUIRE((int64_t)b * p.n <= (int64_t)1 << 30, VSR_EINVAL, "vsr_sample_ex: b*n = %lld rows > 2^30 unsupported",
               (long long)b * p.n);
+  VSR_REQUIRE(c->ngram == 0 || c->V >= T, VSR_EINVAL, "vsr_sample_ex: n-gram blocking needs vocab_size (%d) >= seq_len (%d)",
+              c->V, T);
   const int rows = b * p.n;
   VSR_TRY(ensure_rows(c, rows));
   VSR_TRY(ensure_sel(c, rows));
+  if (c->ngram > 0) VSR_TRY(ensure_whist(c, rows));
   VSR_TRY(attn_begin(c, rows, T, 0));
   VSR_TRY(launch_state_init(c, rows, st));
   for (int t = 0; t < T; ++t) {
@@ -688,7 +712,7 @@ static int sample_impl(Ctx* c, const VsrSampleParams& p, int64_t* out_words, int
     attn_step_io(c, io, t, rows);
     VSR_TRY(run_step(c, io, st));
     VSR_TRY(launch_sample_pick(c, rows, t, T, p, out_words, out_gates, lp_words, lp_gates, st));
-    if (t + 1 < T) VSR_TRY(launch_commit_identity(c, rows, nullptr, 0, -1, st));
+    if (t + 1 < T) VSR_TRY(launch_commit_identity(c, rows, nullptr, 0, -1, c->ngram > 0 ? t : -1, st));
   }
   attn_done(c, false, T, rows, rows);
   return VSR_OK;
@@ -837,6 +861,15 @@ int vsr_get_history(vsr_handle h, int32_t* parent, int32_t* word, int32_t* gate,
 int vsr_set_attention_capture(vsr_handle h, int32_t enabled) {
   if (!h) { vsr::set_error("vsr_set_attention_capture: null handle"); return VSR_EINVAL; }
   ((Ctx*)h)->attn_capture = enabled != 0;
+  return VSR_OK;
+}
+
+int vsr_set_no_repeat_ngram(vsr_handle h, int32_t n) {
+  if (!h) { vsr::set_error("vsr_set_no_repeat_ngram: null handle"); return VSR_EINVAL; }
+  Ctx* c = (Ctx*)h;
+  VSR_REQUIRE(n >= 0 && n <= c->d.seq_len, VSR_EINVAL, "vsr_set_no_repeat_ngram: n=%d not in [0, seq_len=%d] (0 = off)", n,
+              c->d.seq_len);
+  c->ngram = n;
   return VSR_OK;
 }
 

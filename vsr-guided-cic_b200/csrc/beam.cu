@@ -155,6 +155,8 @@ struct AdvanceArgs {
   float *h1, *c1, *h2, *c2;
   const int32_t* ptr; int32_t* ptrn;
   int32_t* word_idx;
+  // n-gram blocking histories [rows][whist_ld] (null = off): row n gets its parent's first hist_t words, then w
+  const int32_t* whist; int32_t* whist_n; int whist_ld, hist_t;
   // tensor-core twins of h1 / h2 (none on the fp32 path), moved as raw 16-byte vectors: per state up to three arrays
   // (fp16 hi + fp16 lo, or fp16 hi + e4m3 hi8 + e4m3 lo8) of `tw_vec[i]` vectors per row
   int n_tw;
@@ -188,6 +190,12 @@ __device__ __forceinline__ void advance_row(const AdvanceArgs& a, int n, int p, 
       s = s < 0 ? 0 : (s > a.L - 1 ? a.L - 1 : s);             // (controllable_captioning.py:139-140)
     }
     a.ptrn[n] = s;
+  }
+  if (a.whist_n != nullptr) {
+    int32_t* dst = a.whist_n + (size_t)n * a.whist_ld;
+    if (a.whist != a.whist_n)
+      for (int i = threadIdx.x; i < a.hist_t; i += blockDim.x) dst[i] = a.whist[(size_t)p * a.whist_ld + i];
+    if (threadIdx.x == 0) dst[a.hist_t] = (int32_t)w;
   }
 }
 
@@ -271,6 +279,7 @@ struct SampleArgs {
   float tau; int top_k; float top_p;
   int32_t *sel_word, *sel_gate;
   int64_t *out_words, *out_gates; float *lp_words, *lp_gates;
+  const int32_t* whist; int whist_ld, ngram;   // n-gram blocking: the rows' words of steps 0 .. t-1 (null = off)
 };
 
 constexpr int SP_THREADS = 256;
@@ -364,6 +373,22 @@ __device__ void sp_bounds(const SampleArgs& a, int n, const float* x, float* s_x
   for (int v = tid * 4; v < V; v += SP_THREADS * 4)
     *reinterpret_cast<float4*>(s_x + v) = *reinterpret_cast<const float4*>(x + v);   // rows are padded to 4 columns
   __syncthreads();
+  // n-gram blocking: banned entries leave the row as x = -inf (last in the order, zero mass; the draw skips them), and
+  // the masses are taken relative to the largest entry that is left
+  float xmax = a.row_max[n];
+  if (a.whist != nullptr && a.t >= a.ngram) {
+    for_each_banned(a.whist + (size_t)n * a.whist_ld, a.t, a.ngram, tid, SP_THREADS, [&](int w) { s_x[w] = -INFINITY; });
+    __syncthreads();
+    float m = -INFINITY;
+    for (int v = tid; v < V; v += SP_THREADS) m = fmaxf(m, s_x[v]);
+    m = warp_max(m);
+    if (lane == 0) s_cnt[0][warp] = __float_as_uint(m);
+    __syncthreads();
+    xmax = __uint_as_float(s_cnt[0][0]);
+#pragma unroll
+    for (int w = 1; w < SP_THREADS / 32; ++w) xmax = fmaxf(xmax, __uint_as_float(s_cnt[0][w]));
+    __syncthreads();
+  }
   // ---- K: the first min(top_k, V) entries
   if (a.top_k > 0 && a.top_k < V) {
     unsigned need = (unsigned)a.top_k, prefix = 0u;
@@ -390,7 +415,7 @@ __device__ void sp_bounds(const SampleArgs& a, int n, const float* x, float* s_x
   // ---- P: the shortest prefix of K whose mass exp(z - max z) reaches top_p of K's
   if (a.top_p < 1.f) {
     const unsigned kkey = pkey; const int kidx = pidx;
-    const float zmax = sp_z(a.row_max[n], tau);
+    const float zmax = sp_z(xmax, tau);
     auto mass = [&](float xv) { return (unsigned long long)__float2ull_rz(expf(sp_z(xv, tau) - zmax) * SP_FIX); };
     unsigned long long need = 0ull;
     unsigned pre = 0u;
@@ -441,6 +466,7 @@ template <bool TRUNC>
 __global__ void __launch_bounds__(SP_THREADS, TRUNC ? 4 : 6) k_sample_pick(const SampleArgs a) {
   __shared__ float s_v[SP_THREADS / 32];
   __shared__ int s_i[SP_THREADS / 32];
+  __shared__ unsigned s_ban[TRUNC ? 1 : BAN_WORDS];   // untruncated draw under n-gram blocking: banned words (bitmap)
   const int n = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int c = n / a.n, j = n - c * a.n, V = a.V;
   const float* x = a.logits + (size_t)n * a.ld;
@@ -457,10 +483,14 @@ __global__ void __launch_bounds__(SP_THREADS, TRUNC ? 4 : 6) k_sample_pick(const
   const float tau = a.tau;
   const float* src = x;
   unsigned pk = 0u; int pi = 0x7fffffff;           // bound of P
+  bool ban = false;
   if constexpr (TRUNC) {
     extern __shared__ __align__(16) float s_x[];
     sp_bounds(a, n, x, s_x, pk, pi);
     src = s_x;
+  } else {
+    ban = a.whist != nullptr && a.t >= a.ngram;     // block-uniform
+    if (ban) build_ban_bitmap(s_ban, a.whist + (size_t)n * a.whist_ld, a.t, a.ngram, V);
   }
   // ---- draw: Gumbel-max over P, lanes of one Philox block = 4 consecutive vocabulary entries
   float bv = -INFINITY; int bi = 0x7fffffff;
@@ -469,10 +499,12 @@ __global__ void __launch_bounds__(SP_THREADS, TRUNC ? 4 : 6) k_sample_pick(const
     const float xs[4] = {q.x, q.y, q.z, q.w};
     bool in[4];
     bool any = false;
+    const unsigned bb = ban ? s_ban[v0 >> 5] >> (v0 & 31) : 0u;   // (v0 % 4 == 0: one bitmap word)
 #pragma unroll
     for (int e = 0; e < 4; ++e) {
       const unsigned k = orderable(xs[e]);
-      in[e] = v0 + e < V && (!TRUNC || k > pk || (k == pk && v0 + e <= pi));
+      // (TRUNC: -inf is a banned entry, logits are finite)
+      in[e] = v0 + e < V && !((bb >> e) & 1u) && (!TRUNC || ((k > pk || (k == pk && v0 + e <= pi)) && xs[e] > -INFINITY));
       any |= in[e];
     }
     if (!any) continue;
@@ -632,6 +664,7 @@ int launch_beam_step(Ctx* c, int t, int b, int cur, int k, int64_t eos0, int64_t
   AdvanceArgs ad{};
   ad.rows_new = b * k; ad.cur = cur; ad.k = k; ad.fixed_slot = -1;
   fill_advance(c, ad);
+  if (c->ngram > 0) { ad.whist = c->whist; ad.whist_n = c->whist_n; ad.whist_ld = c->d.seq_len; ad.hist_t = t; }
   k_beam_step<<<dim3(b, advance ? k : 1), 256, 0, st>>>(a, ad, advance ? 1 : 0);
   VSR_CHECK_CUDA(cudaGetLastError()); c->launches++;
   std::swap(c->sel_beam, c->sel_beam_n);
@@ -641,6 +674,7 @@ int launch_beam_step(Ctx* c, int t, int b, int cur, int k, int64_t eos0, int64_t
   std::swap(c->m0, c->m0n);
   std::swap(c->m1, c->m1n);
   if (advance) std::swap(c->ptr, c->ptrn);
+  if (advance && c->ngram > 0) std::swap(c->whist, c->whist_n);
   return VSR_OK;
 }
 
@@ -653,7 +687,7 @@ static int launch_advance(Ctx* c, AdvanceArgs& a, cudaStream_t st) {
 }
 
 int launch_commit_identity(Ctx* c, int rows, const int64_t* next_words, int64_t word_stride,
-                           int next_slot, cudaStream_t st) {
+                           int next_slot, int hist_t, cudaStream_t st) {
   PhaseScope ps(c, PH_REORDER, st);
   AdvanceArgs a{};
   a.rows_new = rows; a.cur = 1; a.k = 1;
@@ -661,6 +695,7 @@ int launch_commit_identity(Ctx* c, int rows, const int64_t* next_words, int64_t 
   if (next_words != nullptr) { a.word64 = next_words; a.word64_stride = word_stride; a.gate32 = nullptr; }
   else { a.word32 = c->sel_word; a.gate32 = c->sel_gate; }
   a.fixed_slot = next_slot;
+  if (hist_t >= 0) { a.whist = c->whist; a.whist_n = c->whist; a.whist_ld = c->d.seq_len; a.hist_t = hist_t; }   // in place
   return launch_advance(c, a, st);
 }
 
@@ -685,6 +720,7 @@ int launch_sample_pick(Ctx* c, int rows, int t, int T, const VsrSampleParams& p,
   const bool trunc = (p.top_k > 0 && p.top_k < c->V) || p.top_p < 1.f;
   a.sel_word = c->sel_word; a.sel_gate = c->sel_gate;
   a.out_words = out_words; a.out_gates = out_gates; a.lp_words = lp_words; a.lp_gates = lp_gates;
+  if (c->ngram > 0) { a.whist = c->whist; a.whist_ld = c->d.seq_len; a.ngram = c->ngram; }
   if (!trunc) {
     k_sample_pick<false><<<rows, SP_THREADS, 0, st>>>(a);
   } else {

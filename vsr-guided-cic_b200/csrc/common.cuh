@@ -363,6 +363,11 @@ struct Ctx {
   float *hist_score, *hist_lpw, *hist_lpg;       // [T][caps][beam]
   int hist_T = 0, hist_b = 0, hist_k = 0;
   int64_t* word_in = nullptr;        // [rows] scratch (teacher forcing / step)
+  // n-gram blocking (vsr_set_no_repeat_ngram): block size (0 = off) and, while on, every row's emitted words
+  // [rows][seq_len], double-buffered like ptr / ptrn (beam rows copy their parent's prefix); grow-only, cap in rows
+  int ngram = 0;
+  int32_t *whist = nullptr, *whist_n = nullptr;
+  int cap_whist = 0;
   // attention capture (vsr_set_attention_capture): per step t, rows t * attn_step_rows .. of [R+1] weights and the
   // slot each row read; attn_path = the back-tracked rows of the returned beams [b][out_size][T]
   bool attn_capture = false;
@@ -387,7 +392,7 @@ struct Ctx {
     const void* captions;
     const void *det, *det_seqs, *slot_index, *verbs;
     int64_t det_stride, eos0, eos1;
-    int32_t b, D, L, R, n_img, verbs_dtype, k, use_verbs, gt, T, attn, feat_dtype;
+    int32_t b, D, L, R, n_img, verbs_dtype, k, use_verbs, gt, T, attn, feat_dtype, ngram;
   };
   struct GraphEntry { GraphKey key; cudaGraphExec_t exec; int64_t launches; uint64_t last_use; };
   std::vector<GraphEntry> graphs;
@@ -431,6 +436,8 @@ struct StepIO {
   bool need_h32;     // the caller reads the fp32 h1'/h2' (vsr_step); the tensor-core path itself only needs the fp16 twins
   float* attn_alpha;    // optional [rows][R+1] attention weights of the step (capture), with ...
   int32_t* attn_slot;   // ... [rows] the slot each row read; both null when capture is off
+  bool ngram_block;     // the head kernels skip the words n-gram blocking bans (Ctx::ngram, histories in Ctx::whist) ...
+  int t;                // ... at step t of the decode
 };
 int run_step(Ctx* c, const StepIO& io, cudaStream_t st);
 
@@ -442,8 +449,10 @@ int launch_beam_step(Ctx* c, int t, int b, int cur, int k, int64_t eos0, int64_t
 int launch_backtrack(Ctx* c, int b, int k, int T, int out_size, int64_t* out_words,
                      int64_t* out_gates, float* lp_words, float* lp_gates, int32_t* path_row, cudaStream_t st);
 int launch_attn_gather(Ctx* c, const int32_t* path_row, int n_out, int T, float* alpha, int32_t* slot, cudaStream_t st);
+// hist_t >= 0: also append the new input words at position hist_t of the rows' n-gram blocking histories
 int launch_commit_identity(Ctx* c, int rows, const int64_t* next_words, int64_t word_stride,
-                           int next_slot, cudaStream_t st);
+                           int next_slot, int hist_t, cudaStream_t st);
+int ensure_whist(Ctx* c, int rows);
 int launch_greedy_pick(Ctx* c, int rows, int t, int T, int64_t* out_words, int64_t* out_gates,
                        cudaStream_t st);
 // draws of the sampling decode: rows = captions * p.n, row = caption * p.n + draw

@@ -416,6 +416,7 @@ __global__ void __launch_bounds__(SM_THREADS) k_softmax_topk(const SoftmaxArgs a
   __shared__ int red_i[2][NW];
   __shared__ int s_forced, s_slow;
   __shared__ int s_pick[VSR_MAX_BEAM];
+  __shared__ unsigned s_ban[BAN_WORDS];         // n-gram blocking: banned words of the row (bitmap)
   const int n = blockIdx.x;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   pdl_trigger();
@@ -424,6 +425,9 @@ __global__ void __launch_bounds__(SM_THREADS) k_softmax_topk(const SoftmaxArgs a
   const int V = a.V;
   const int n4 = (V + 3) >> 2;
   const int topk = a.topk;
+  // banned words stay in the log-sum-exp and out of the candidate tracking (fast and slow path alike)
+  const bool ban = topk > 0 && a.whist != nullptr && a.hist_t >= a.ngram;      // block-uniform
+  if (ban) build_ban_bitmap(s_ban, a.whist + (size_t)n * a.whist_ld, a.hist_t, a.ngram, V);
 
   // thread 0 starts its dependent loads early (slot pointer -> verb id, shift logit)
   int64_t verb = -1; float shift_logit = 0.f;
@@ -462,11 +466,12 @@ __global__ void __launch_bounds__(SM_THREADS) k_softmax_topk(const SoftmaxArgs a
         if (v0 >= V) q[u].x = -INFINITY;
       }
       const float e4[4] = {q[u].x, q[u].y, q[u].z, q[u].w};
+      const unsigned bb = (ban && v0 < V) ? s_ban[v0 >> 5] >> (v0 & 31) : 0u;   // (v0 % 4 == 0: one bitmap word)
 #pragma unroll
       for (int e = 0; e < 4; ++e) {
         const float val = e4[e];
         bm = fmaxf(bm, val);
-        if (val > v2) {                         // strict: equal values keep the earlier (smaller) index
+        if (val > v2 && !((bb >> e) & 1u)) {    // strict: equal values keep the earlier (smaller) index
           if (val > v1) { v2 = v1; i2 = i1; v1 = val; i1 = v0 + e; } else { v2 = val; i2 = v0 + e; }
         }
       }
@@ -626,9 +631,12 @@ __global__ void __launch_bounds__(SM_THREADS) k_softmax_topk(const SoftmaxArgs a
         const float4 qq = *reinterpret_cast<const float4*>(x + jj * 4);
         const int v0 = jj * 4;
         const float e4[4] = {qq.x, qq.y, qq.z, qq.w};
+        const unsigned bb = ban ? s_ban[v0 >> 5] >> (v0 & 31) : 0u;
 #pragma unroll
         for (int u = 0; u < 4; ++u)
-          if (v0 + u < V && before(bv, bi, e4[u], v0 + u) && before(e4[u], v0 + u, cv, ci)) { cv = e4[u]; ci = v0 + u; }
+          if (v0 + u < V && !((bb >> u) & 1u) && before(bv, bi, e4[u], v0 + u) && before(e4[u], v0 + u, cv, ci)) {
+            cv = e4[u]; ci = v0 + u;
+          }
       }
     }
   }
@@ -636,7 +644,7 @@ __global__ void __launch_bounds__(SM_THREADS) k_softmax_topk(const SoftmaxArgs a
 
 constexpr int VM_WARPS = 4;
 // k_vocab_merge: vocab_head.cuh (merge_row) — one warp per row finishes the vocabulary head from the GEMM's records
-__global__ void __launch_bounds__(VM_WARPS * 32) k_vocab_merge(const SoftmaxArgs a, const float* __restrict__ vpart, int n_chunks) {
+__global__ void __launch_bounds__(VM_WARPS * 32) k_vocab_merge(const SoftmaxArgs a, float* vpart, int n_chunks) {
   const int lane = threadIdx.x & 31;
   const int n = blockIdx.x * VM_WARPS + (threadIdx.x >> 5);
   pdl_trigger();
@@ -884,6 +892,9 @@ int run_step(Ctx* c, const StepIO& io, cudaStream_t st) {
     PhaseScope ps(c, PH_SOFTMAX_TOPK, st);
     SoftmaxArgs a = make_softmax_args(c, rows, io.cur_beam, io.topk, io.use_verbs, io.gt);
     a.out_logp = io.out_logp; a.out_stride = io.out_stride;
+    if (io.ngram_block && c->ngram > 0) {
+      a.whist = c->whist; a.whist_ld = c->d.seq_len; a.hist_t = io.t; a.ngram = c->ngram;
+    }
     a.gate_out = io.gate_out; a.gate_stride = io.gate_stride;
     if (fuse_vocab) {
       k_vocab_merge<<<(rows + VM_WARPS - 1) / VM_WARPS, VM_WARPS * 32, 0, st>>>(a, c->vpart, c->NE / 16);

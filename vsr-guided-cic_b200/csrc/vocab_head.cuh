@@ -50,9 +50,32 @@ __device__ __forceinline__ void warp_argbest_redux(float v, int i, unsigned& kbe
   ibest = (int)__reduce_min_sync(0xffffffffu, key == kbest ? (unsigned)i : 0xffffffffu);
 }
 
+// n-gram blocking (vsr_set_no_repeat_ngram).  h = a row's emitted words y_0 .. y_{t-1}; with block size N the word
+// y_{i+N-1} is banned at step t for every start 0 <= i <= t - N with y_i .. y_{i+N-2} == y_{t-N+1} .. y_{t-1}.  f(w) is
+// called once per matching start (a word may come up more than once); the caller's threads split the starts as
+// first, first + stride, ...  Every consumer of the ban (merge_row, k_softmax_topk, k_sample_pick) goes through here.
+template <typename F>
+__device__ __forceinline__ void for_each_banned(const int32_t* h, int t, int N, int first, int stride, F&& f) {
+  for (int i = first; i <= t - N; i += stride) {
+    bool match = true;
+    for (int q = 0; q < N - 1 && match; ++q) match = h[i + q] == h[t - N + 1 + q];
+    if (match) f((int)h[i + N - 1]);
+  }
+}
+// shared-memory bitmap of the banned words of a row for one CTA (bit w of word w >> 5), vocabularies up to 49152
+constexpr int BAN_WORDS = 49152 / 32;
+__device__ __forceinline__ void build_ban_bitmap(unsigned* bits, const int32_t* h, int t, int N, int V) {
+  for (int i = threadIdx.x; i < (V + 31) >> 5; i += blockDim.x) bits[i] = 0u;
+  __syncthreads();
+  for_each_banned(h, t, N, threadIdx.x, blockDim.x, [&](int w) { atomicOr(&bits[w >> 5], 1u << (w & 31)); });
+  __syncthreads();
+}
+
 struct SoftmaxArgs {
   const float* logits; int ld;   // [rows][ld]
   int rows, V, cur_beam, L, topk;
+  // n-gram blocking: whist [rows][whist_ld] = the rows' words of steps 0 .. hist_t - 1, block size ngram; null = off
+  const int32_t* whist; int whist_ld, hist_t, ngram;
   const int32_t* ptr;
   const void* verbs; int verbs_dtype; int use_verbs, gt;
   const int64_t* vt_keys; const int32_t* vt_off; const int32_t* vt_idx; int vt_n;
@@ -128,12 +151,24 @@ struct RowHead {
 // of the topk chunks ahead of C would hold an element ordered before e (larger, or equal with a smaller index).
 // Composite keys orderable(value) : ~position make "ordered before" a plain unsigned 64-bit '>'.  The chunk maxima stay
 // in registers across the topk rounds when the row has at most 32 * VM_CPL chunks (V <= 12288), else they are re-read.
+// N-gram blocking (a.whist): the log-sum-exp still comes from the unchanged records.  Then every chunk that holds a
+// banned word gets the max of its words that are not banned, from its 16 re-read logits, written over the record's max
+// (-inf when all of them are banned: the chunk drops out), and both rounds run as above with banned words skipped.  The
+// argument above carries over unchanged with "element" read as "word that is not banned": each chunk's key is then
+// the max of exactly those words.
 constexpr int VM_CPL = 24;
 
-__device__ __forceinline__ void merge_row(const SoftmaxArgs& a, const float* __restrict__ vpart, int n_chunks,
-                                          int n, int lane, RowHead& out) {
+// bits e of the banned words C * 16 + e of chunk C
+__device__ __forceinline__ unsigned chunk_ban_mask(const int32_t* h, int t, int N, int C) {
+  unsigned m = 0u;
+  for_each_banned(h, t, N, 0, 1, [&](int w) { if ((w >> 4) == C) m |= 1u << (w & 15); });
+  return m;
+}
+
+__device__ __forceinline__ void merge_row(const SoftmaxArgs& a, float* vpart, int n_chunks, int n, int lane,
+                                          RowHead& out) {
   const int V = a.V, topk = a.topk;
-  const float2* rec = reinterpret_cast<const float2*>(vpart) + (size_t)n * n_chunks;
+  float2* rec = reinterpret_cast<float2*>(vpart) + (size_t)n * n_chunks;
   const float* x = a.logits + (size_t)n * a.ld;
   const int used = (V + 15) >> 4;               // chunks that hold vocabulary entries
 
@@ -182,6 +217,28 @@ __device__ __forceinline__ void merge_row(const SoftmaxArgs& a, const float* __r
   const float lsum = logf(se);
   stay = warp_sum(stay);
 
+  const bool ban = a.whist != nullptr && a.hist_t >= a.ngram;   // warp-uniform
+  const int32_t* hrow = ban ? a.whist + (size_t)n * a.whist_ld : nullptr;
+  if (ban) {
+    __syncwarp();                                 // every lane has read its records
+    for_each_banned(hrow, a.hist_t, a.ngram, lane, 32, [&](int w) {
+      const int C = w >> 4;
+      const unsigned m = chunk_ban_mask(hrow, a.hist_t, a.ngram, C);
+      float cm = -INFINITY;
+      for (int e = 0; e < 16; ++e)
+        if (!((m >> e) & 1u) && C * 16 + e < V) cm = fmaxf(cm, x[C * 16 + e]);
+      rec[C].x = cm;                              // (lanes that hit the same chunk write the same value)
+    });
+    __syncwarp();
+    if (in_regs) {
+#pragma unroll
+      for (int q = 0; q < VM_CPL; ++q) {
+        const int t = lane + 32 * q;
+        if (t < used) cmx[q] = rec[t].x;
+      }
+    }
+  }
+
   //   1. the topk CHUNKS by chunk max (round j: every lane's best key strictly below the previous winner, then a warp
   //      arg-best; lane j keeps winner j)
   unsigned long long prev = ~0ull;
@@ -211,12 +268,14 @@ __device__ __forceinline__ void merge_row(const SoftmaxArgs& a, const float* __r
   //   2. the topk ELEMENTS among those chunks' logits: lane owns elements e = lane + 32 * q of the topk * 16
   constexpr int EQ = VSR_MAX_BEAM * 16 / 32;
   float cv[EQ]; int ci[EQ];
+  const unsigned my_mask = (ban && my_chunk >= 0) ? chunk_ban_mask(hrow, a.hist_t, a.ngram, my_chunk) : 0u;
 #pragma unroll
   for (int q = 0; q < EQ; ++q) {
     const int e = lane + 32 * q;
     const int chunk = __shfl_sync(0xffffffffu, my_chunk, (e >> 4) & 31);
+    const unsigned cmask = ban ? __shfl_sync(0xffffffffu, my_mask, (e >> 4) & 31) : 0u;
     cv[q] = -INFINITY; ci[q] = 0x7fffffff;
-    if (e < topk * 16 && chunk >= 0) {
+    if (e < topk * 16 && chunk >= 0 && !((cmask >> (e & 15)) & 1u)) {
       const int col = chunk * 16 + (e & 15);
       if (col < V) { cv[q] = x[col]; ci[q] = col; }
     }

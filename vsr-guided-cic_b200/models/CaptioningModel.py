@@ -16,6 +16,14 @@ Every driver (`beam_search`, `beam_search_v`, `beam_search_v_indexed`, `forward`
 `step_v` of the sub-class) takes region features in float32, float16 or bfloat16, one dtype for the detections and the
 slot tiles.  The kernels widen half-precision values to fp32 as they load them, so every output is bit-identical to that
 of the same call on the features' float32 upcast; only the bytes read and copied halve.
+
+Every driver that chooses words (`beam_search`, `beam_search_v`, `beam_search_v_indexed`, `test`, `sample_rl`, `sample_v`)
+takes `no_repeat_ngram_size=0`.  With n >= 1 a word that would complete an n-gram the row (for beam search: the beam's
+own word path) has already emitted is banned at that step: beam search keeps the exact top-k of the words that are not
+banned, greedy takes the best of them, sampling drops banned words before temperature / top-k / top-p.  The returned
+log-probs stay the model's own; verb-forced words are never blocked.  0 = off, bit-identical to a call without the
+keyword.  The semantics and limits (n <= seq_len; vocab_size >= beam_size + seq_len - 1, or >= seq_len for greedy and
+sampling) are spelled out in include/vsrdec.h, vsr_set_no_repeat_ngram.
 """
 import torch
 from torch import nn
@@ -39,18 +47,31 @@ class CaptioningModel(nn.Module):
     def _engine_for(self, statics, seqs=None):
         raise NotImplementedError
 
+    def _check_ngram(self, no_repeat_ngram_size, beam_size=1):
+        """VsrError unless the block size is valid for this model and a decode with beam_size rows per caption."""
+        from vsrdec.engine import check_no_repeat_ngram
+        check_no_repeat_ngram(no_repeat_ngram_size, self.seq_len, self.vocab_size, beam_size)
+
     @staticmethod
-    def _run(eng, decode, return_attention):
-        """decode() alone, or with the engine's attention capture on around it: (result, attention dict or None)."""
-        if not return_attention:
-            return decode(), None
-        eng.set_attention_capture(True)
+    def _run(eng, decode, return_attention, no_repeat_ngram_size=0):
+        """decode() alone, or with the engine's attention capture on around it: (result, attention dict or None).  The
+        engine's n-gram blocking is no_repeat_ngram_size for the duration of the call and restored afterwards."""
+        prev = eng.no_repeat_ngram
+        if no_repeat_ngram_size != prev:
+            eng.set_no_repeat_ngram(no_repeat_ngram_size)
         try:
-            res = decode()
-            att = eng.attention()
+            if not return_attention:
+                return decode(), None
+            eng.set_attention_capture(True)
+            try:
+                res = decode()
+                att = eng.attention()
+            finally:
+                eng.set_attention_capture(False)
+            return res, att
         finally:
-            eng.set_attention_capture(False)
-        return res, att
+            if eng.no_repeat_ngram != prev:
+                eng.set_no_repeat_ngram(prev)
 
     # ---- drivers
     def forward(self, statics, seqs, *args, return_attention=False):
@@ -60,13 +81,16 @@ class CaptioningModel(nn.Module):
         res, att = self._run(eng, lambda: eng.forward_teacher(seqs[0]), return_attention)
         return res if att is None else (*res, att)
 
-    def test(self, statics, *args, return_attention=False):
-        """Greedy decode (reference CaptioningModel.py:38-52): (words (b,T), gates (b,T)) (+ attention)."""
+    def test(self, statics, *args, return_attention=False, no_repeat_ngram_size=0):
+        """Greedy decode (reference CaptioningModel.py:38-52): (words (b,T), gates (b,T)) (+ attention).  With
+        no_repeat_ngram_size = n >= 1 each pick is the best word that does not repeat an n-gram of the caption."""
+        self._check_ngram(no_repeat_ngram_size)
         eng = self._engine_for(statics)
-        res, att = self._run(eng, eng.greedy, return_attention)
+        res, att = self._run(eng, eng.greedy, return_attention, no_repeat_ngram_size)
         return res if att is None else (*res, att)
 
-    def sample_rl(self, statics, *args, seed=None, return_attention=False, n=1, temperature=1.0, top_k=0, top_p=1.0):
+    def sample_rl(self, statics, *args, seed=None, return_attention=False, n=1, temperature=1.0, top_k=0, top_p=1.0,
+                  no_repeat_ngram_size=0):
         """Multinomial sampling with log-probs (reference CaptioningModel.py:54-76): at every step both heads are
         sampled from the step's distributions and fed back; returns ((words, gates), (lp_words, lp_gates)), each (b,T).
         The whole loop runs on the device (vsr_sample: Gumbel-max over the vocabulary row with a Philox stream).  The
@@ -75,26 +99,30 @@ class CaptioningModel(nn.Module):
         Extensions (keywords only): n independent draws per caption, returned as (b, n, T) when n > 1 (draw j is the
         same for every n > j); the word head sampled at `temperature`, from its top_k most likely words (0 = off) and
         then from the smallest set of those that holds top_p of their mass (1 = off).  The log-probs stay the model's
-        own (untempered, untruncated).  Semantics: include/vsrdec.h, vsr_sample_ex."""
-        return self._sample(statics[:2], False, False, seed, return_attention, n, temperature, top_k, top_p)
+        own (untempered, untruncated).  With no_repeat_ngram_size = m >= 1, words that would repeat an m-gram of the draw
+        leave the row before temperature and truncation.  Semantics: include/vsrdec.h, vsr_sample_ex."""
+        return self._sample(statics[:2], False, False, seed, return_attention, n, temperature, top_k, top_p,
+                            no_repeat_ngram_size)
 
-    def sample_v(self, statics, *, n=1, temperature=1.0, top_k=0, top_p=1.0, gt=False, seed=None, return_attention=False):
+    def sample_v(self, statics, *, n=1, temperature=1.0, top_k=0, top_p=1.0, gt=False, seed=None, return_attention=False,
+                 no_repeat_ngram_size=0):
         """sample_rl with verb forcing (step_v semantics, gt as in beam_search_v): statics = (detections, det_seqs,
         verbs).  A step whose slot holds a verb takes the forced word and gate 1, both with log-prob 0; the other steps
         are sampled as in sample_rl.  Same return structure as sample_rl."""
         if len(statics) < 3 or statics[2] is None:
             from vsrdec import VsrError
             raise VsrError("sample_v needs statics = (detections, det_seqs, verbs)")
-        return self._sample(statics, True, gt, seed, return_attention, n, temperature, top_k, top_p)
+        return self._sample(statics, True, gt, seed, return_attention, n, temperature, top_k, top_p, no_repeat_ngram_size)
 
-    def _sample(self, statics, use_verbs, gt, seed, return_attention, n, temperature, top_k, top_p):
+    def _sample(self, statics, use_verbs, gt, seed, return_attention, n, temperature, top_k, top_p, no_repeat_ngram_size):
         from vsrdec.engine import check_sample_args
         check_sample_args(n, temperature, top_k, top_p, statics[0].size(0))   # before the prologue: nothing runs
+        self._check_ngram(no_repeat_ngram_size)
         eng = self._engine_for(statics)
         if seed is None:
             seed = int(torch.randint(0, 2 ** 62, (1,)).item())
         res, att = self._run(eng, lambda: eng.sample(seed, n=n, temperature=temperature, top_k=top_k, top_p=top_p,
-                                                     use_verbs=use_verbs, gt=gt), return_attention)
+                                                     use_verbs=use_verbs, gt=gt), return_attention, no_repeat_ngram_size)
         return res if att is None else (*res, att)
 
     def _select_beam(self, input, selected_beam, cur_beam_size, beam_size, b_s, reduced=True):
@@ -120,10 +148,11 @@ class CaptioningModel(nn.Module):
         out = src[rows, selected_beam.long().reshape(b_s, beam_size)]
         return out.reshape((b_s * beam_size,) + tail) if reduced else out
 
-    def _beam_run(self, eng, eos_idxs, beam_size, out_size, use_verbs, gt, return_attention, slot_index=None):
+    def _beam_run(self, eng, eos_idxs, beam_size, out_size, use_verbs, gt, return_attention, slot_index=None,
+                  no_repeat_ngram_size=0):
         def decode():
             return eng.beam_search(beam_size, out_size, eos_idxs, use_verbs=use_verbs, gt=gt)
-        ((words, gates), (lpw, lpg), _), att = self._run(eng, decode, return_attention)
+        ((words, gates), (lpw, lpg), _), att = self._run(eng, decode, return_attention, no_repeat_ngram_size)
         outputs, log_probs = [words, gates], [lpw, lpg]
         if att is not None and slot_index is not None:      # detection row of every region of the slot read
             b, R = slot_index.size(0), slot_index.size(2)
@@ -136,30 +165,37 @@ class CaptioningModel(nn.Module):
                 att = {k: v.squeeze(1) for k, v in att.items()}
         return (outputs, log_probs) if att is None else (outputs, log_probs, att)
 
-    def _beam(self, statics, eos_idxs, beam_size, out_size, use_verbs, gt, return_attention=False):
+    def _beam(self, statics, eos_idxs, beam_size, out_size, use_verbs, gt, return_attention=False, no_repeat_ngram_size=0):
+        self._check_ngram(no_repeat_ngram_size, beam_size)
         eng = self._engine_for(statics)
-        return self._beam_run(eng, eos_idxs, beam_size, out_size, use_verbs, gt, return_attention)
+        return self._beam_run(eng, eos_idxs, beam_size, out_size, use_verbs, gt, return_attention,
+                              no_repeat_ngram_size=no_repeat_ngram_size)
 
-    def beam_search_v_indexed(self, statics, eos_idxs, beam_size, out_size=1, *args, gt=False, return_attention=False):
+    def beam_search_v_indexed(self, statics, eos_idxs, beam_size, out_size=1, *args, gt=False, return_attention=False,
+                              no_repeat_ngram_size=0):
         """Extension (SURVEY §8 f3): beam_search_v with the slots given as INDICES into the detections instead
         of materialised feature tiles: statics = (detections (b,D,F), slot_index (b,L,R) int, verbs (b,L) or None);
         slot_index >= 0 picks a detection row, -2 the mean of the image's valid detections, -1 is padding.
         Same return structure as beam_search_v; 10x fewer input bytes.  With return_attention the attention dict also
         holds det_index (..., R) int64 = slot_index[caption, slot, :]: the detection row each alpha[..., 1:] column
-        weighs (-2 the image's mean row, -1 padding)."""
+        weighs (-2 the image's mean row, -1 padding).  no_repeat_ngram_size as in beam_search."""
+        self._check_ngram(no_repeat_ngram_size, beam_size)
         eng = self._engine()
         verbs = statics[2] if len(statics) > 2 else None
         eng.prologue_indexed(statics[0], statics[1], verbs)
         self._prologue_key = None
         return self._beam_run(eng, eos_idxs, beam_size, out_size, verbs is not None, gt, return_attention,
-                              slot_index=statics[1])
+                              slot_index=statics[1], no_repeat_ngram_size=no_repeat_ngram_size)
 
-    def beam_search(self, statics, eos_idxs, beam_size, out_size=1, *args, return_attention=False):
+    def beam_search(self, statics, eos_idxs, beam_size, out_size=1, *args, return_attention=False, no_repeat_ngram_size=0):
         """Joint (word, gate) beam search (reference CaptioningModel.py:116-195).  beam_size <= 8, out_size <= beam_size,
-        <= 64 regions per slot (see the limits in models/controllable_captioning.py)."""
-        return self._beam(statics[:2], eos_idxs, beam_size, out_size, False, False, return_attention)
+        <= 64 regions per slot (see the limits in models/controllable_captioning.py).  With no_repeat_ngram_size = n >= 1
+        no beam picks a word that would repeat an n-gram of its own word path (the scores stay the model's)."""
+        return self._beam(statics[:2], eos_idxs, beam_size, out_size, False, False, return_attention, no_repeat_ngram_size)
 
-    def beam_search_v(self, statics, eos_idxs, beam_size, out_size=1, *args, gt=False, return_attention=False):
+    def beam_search_v(self, statics, eos_idxs, beam_size, out_size=1, *args, gt=False, return_attention=False,
+                      no_repeat_ngram_size=0):
         """Beam search with verb forcing (reference CaptioningModel.py:197-294).  beam_size <= 8, out_size <= beam_size,
-        <= 64 regions per slot (see the limits in models/controllable_captioning.py)."""
-        return self._beam(statics, eos_idxs, beam_size, out_size, True, gt, return_attention)
+        <= 64 regions per slot (see the limits in models/controllable_captioning.py).  no_repeat_ngram_size as in
+        beam_search; a verb-forced word is never blocked."""
+        return self._beam(statics, eos_idxs, beam_size, out_size, True, gt, return_attention, no_repeat_ngram_size)

@@ -24,6 +24,8 @@ LIMITS the reference does not have (each raises VsrError with a message, never a
     on the activation scale, not the input format: it is the same for float32, float16 and bfloat16 features;
   * region features are float32, float16 or bfloat16, one dtype for the detections and the slot tiles (a mismatch or
     any other dtype raises); half precision is refused under VSRDEC_GEMM=simt (the fp32 FFMA verification twin).
+  * no-repeat n-gram blocking (`no_repeat_ngram_size` of every word-choosing driver): an int in [0, seq_len]; when on,
+    vocab_size >= beam_size + seq_len - 1 (beam search) or >= seq_len (greedy, sampling);
   * sampling (`sample_rl`, `sample_v`): captions x n draws <= 2^30 rows per call; temperature a finite float32 > 0 and
     top_p in (0, 1] as float32 values (where logits / temperature overflows float32 it is clamped to +-FLT_MAX: the
     overflowing words tie and the lowest index among them wins).
@@ -204,10 +206,11 @@ class ControllableCaptioningModel(_CaptioningModel):
             (reference controllable_captioning.py:192-297) '''
         return self._step_impl(t, state, prev_outputs, statics, seqs, mode, True, gt)
 
-    def test(self, detections, ctrl_det_seqs_test, return_attention=False):
-        return super().test((detections, ctrl_det_seqs_test), return_attention=return_attention)
+    def test(self, detections, ctrl_det_seqs_test, return_attention=False, no_repeat_ngram_size=0):
+        return super().test((detections, ctrl_det_seqs_test), return_attention=return_attention,
+                            no_repeat_ngram_size=no_repeat_ngram_size)
 
     def sample_rl(self, detections, ctrl_det_seqs_test, seed=None, return_attention=False, n=1, temperature=1.0,
-                  top_k=0, top_p=1.0):
+                  top_k=0, top_p=1.0, no_repeat_ngram_size=0):
         return super().sample_rl((detections, ctrl_det_seqs_test), seed=seed, return_attention=return_attention, n=n,
-                                 temperature=temperature, top_k=top_k, top_p=top_p)
+                                 temperature=temperature, top_k=top_k, top_p=top_p, no_repeat_ngram_size=no_repeat_ngram_size)

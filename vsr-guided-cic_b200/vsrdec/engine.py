@@ -67,6 +67,17 @@ def check_sample_args(n, temperature, top_k, top_p, b=None):
         raise VsrError(f"top_p must be in (0, 1] (1 = off) and nonzero in float32, got {top_p!r}")
 
 
+def check_no_repeat_ngram(n, seq_len, vocab_size=None, beam_size=1):
+    """Raise VsrError unless n is a valid no-repeat n-gram block size (vsr_set_no_repeat_ngram) for a model of seq_len
+    steps: an int in [0, seq_len].  With vocab_size, also for a decode with beam_size rows per caption (1: greedy and
+    sampling): when on, vocab_size >= beam_size + seq_len - 1, so that every row keeps enough words that are not banned."""
+    if isinstance(n, bool) or not isinstance(n, numbers.Integral) or not 0 <= n <= seq_len:
+        raise VsrError(f"no_repeat_ngram_size must be an int in [0, seq_len={seq_len}] (0 = off), got {n!r}")
+    if n > 0 and vocab_size is not None and vocab_size < beam_size + seq_len - 1:
+        raise VsrError(f"no_repeat_ngram_size={n} needs vocab_size >= beam + seq_len - 1 = {beam_size + seq_len - 1}, "
+                       f"got {vocab_size}")
+
+
 def _req_cuda(t: torch.Tensor, name: str, dtype=None):
     if not isinstance(t, torch.Tensor) or not t.is_cuda:
         raise VsrError(f"{name} must be a CUDA tensor (no CPU fallback on this path)")
@@ -83,6 +94,7 @@ class DecoderEngine:
         self._keep = None
         self._weights = None
         self._attn_shape = None
+        self.no_repeat_ngram = 0
         self.handle = c_vp()
         d = VsrDims(*(int(self.dims[k]) for k in ("seq_len", "vocab_size", "bos_idx", "det_feat_size",
                                                    "input_encoding_size", "rnn_size", "att_size",
@@ -347,6 +359,14 @@ class DecoderEngine:
             _lib.check(self.lib, self.lib.vsr_get_attention(self.handle, alpha.data_ptr(), slot.data_ptr(),
                                                             _stream_ptr(self.device)))
         return {"alpha": alpha, "slot": slot.long()}
+
+    # ------------------------------------------------------------------ n-gram blocking
+    def set_no_repeat_ngram(self, n: int):
+        """Ban every word that would repeat an n-gram of the row's own words in the following beam-search, greedy and
+        sampling decodes (vsr_set_no_repeat_ngram); 0 = off, the default.  n is an int in [0, seq_len]."""
+        check_no_repeat_ngram(n, self.dims["seq_len"])
+        _lib.check(self.lib, self.lib.vsr_set_no_repeat_ngram(self.handle, int(n)))
+        self.no_repeat_ngram = int(n)
 
     # ------------------------------------------------------------------ instrumentation
     def launch_count(self) -> int:

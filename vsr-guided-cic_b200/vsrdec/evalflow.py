@@ -20,8 +20,10 @@ from .preorder import RoleOrderer, permute_slot_index
 
 class EvalFlow:
     def __init__(self, model, orderer: RoleOrderer, eos_idxs, beam_size: int = 5, out_size: int = 1, gt: bool = True,
-                 overlap: bool = True):
+                 overlap: bool = True, no_repeat_ngram_size: int = 0):
+        """no_repeat_ngram_size: n-gram blocking of every decode (see CaptioningModel.beam_search; 0 = off)."""
         self.model, self.orderer = model, orderer
+        self.no_repeat_ngram_size = no_repeat_ngram_size
         self.eos_idxs, self.beam_size, self.out_size, self.gt = eos_idxs, beam_size, out_size, gt
         self.overlap = bool(overlap)
         self._side = None
@@ -35,7 +37,8 @@ class EvalFlow:
     def _decode(self, b, src, verbs):
         dev = b["slot_index"].device
         statics = (b["detections"], permute_slot_index(b["slot_index"], src), verbs.to(dev).double())
-        return self.model.beam_search_v_indexed(statics, self.eos_idxs, self.beam_size, self.out_size, gt=self.gt)
+        return self.model.beam_search_v_indexed(statics, self.eos_idxs, self.beam_size, self.out_size, gt=self.gt,
+                                                no_repeat_ngram_size=self.no_repeat_ngram_size)
 
     def run(self, batches: Iterable[dict]) -> Iterator:
         it = iter(batches)

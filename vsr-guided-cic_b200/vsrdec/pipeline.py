@@ -22,11 +22,12 @@ import torch
 class DecodePipeline:
     def __init__(self, models: Sequence, eos_idxs, beam_size: int, out_size: int = 1, gt: bool = False,
                  indexed: bool = False, buffers: Optional[int] = None, stack: int = 1, ramp: bool = True,
-                 post: Optional[Callable[[torch.Tensor], torch.Tensor]] = None):
+                 post: Optional[Callable[[torch.Tensor], torch.Tensor]] = None, no_repeat_ngram_size: int = 0):
         """models: one drop-in model per lane (same weights, same device).  `stack` host batches (of equal shapes) are
         decoded per call; with `ramp` the first group of a run holds a single batch, so that the first decode starts after
         one batch's host->device copy instead of `stack` of them (the un-overlapped pipeline fill of a short run).  `post` is
-        applied to each batch's words tensor on the lane's stream (e.g. the all-gather of a caption-sharded job)."""
+        applied to each batch's words tensor on the lane's stream (e.g. the all-gather of a caption-sharded job).
+        `no_repeat_ngram_size` is passed to every decode (n-gram blocking, see beam_search; 0 = off)."""
         if not models:
             raise ValueError("DecodePipeline needs at least one model")
         self.models = list(models)
@@ -35,6 +36,7 @@ class DecodePipeline:
             raise RuntimeError("DecodePipeline: the models must live on a CUDA device (no CPU fallback)")
         self.eos_idxs, self.beam_size, self.out_size, self.gt, self.indexed = eos_idxs, beam_size, out_size, gt, indexed
         self.post = post
+        self.no_repeat_ngram_size = no_repeat_ngram_size
         self.stack = max(1, int(stack))
         self.ramp = bool(ramp)
         self.n_lanes = len(self.models)
@@ -86,7 +88,8 @@ class DecodePipeline:
         with torch.cuda.stream(lane):
             fn = model.beam_search_v_indexed if self.indexed else model.beam_search_v
             statics = tuple(t[:n * b] for t in self._bufs[slot])
-            (words, gates), (lpw, lpg) = fn(statics, self.eos_idxs, self.beam_size, self.out_size, gt=self.gt)
+            (words, gates), (lpw, lpg) = fn(statics, self.eos_idxs, self.beam_size, self.out_size, gt=self.gt,
+                                            no_repeat_ngram_size=self.no_repeat_ngram_size)
             self._freed[slot].record(lane)
             if self.post is not None:
                 words = torch.cat([self.post(words[i * b:(i + 1) * b]) for i in range(n)], 0)

@@ -307,6 +307,8 @@ int vsr_get_step_times(vsr_handle h, float* ms, int32_t cap);
  * eval_flickr.py likewise).  `weights` [host array of 10 device pointers] follows the state_dict order:
  *   W1_txt.weight (128,300) .bias | W1_vis.weight (512,2048) .bias | W2_vis.weight (128,512) .bias |
  *   W_fc_pos.weight (256,260) .bias | W_fc.weight (N,256) .bias          (sinkhorn_network.py:11-15)
+ * vsr_ssp_create:  N in [1,16], and only if the whole network of one problem fits a block's opt-in shared memory on the
+ *   current device (218,368 B at N = 16; 227 KB on a B200): every N it accepts runs at every batch size.
  * vsr_ssp_forward:  seq (B,N,2352) fp32 rows, split by column as sinkhorn_network.py:39-41 slices them: [0,300) -> W1_txt,
  *   [300,2348) -> W1_vis, [2348,2352) appended before W_fc_pos (the eval feeds the concatenation of eval_coco.py:146 unchanged);
  *   matrix (B,N,N) fp32 = SinkhornNet(seq);  assign (B,N) int32 or NULL = for every row r of matrix^T (the profit matrix

@@ -163,6 +163,9 @@ __global__ void __launch_bounds__(SSP_THREADS) k_sinkhorn(const SspWeights W, co
   }
 }
 
+// dynamic shared memory of the one-CTA kernel that runs the whole network: input rows, hidden layers and the two N x N tiles
+size_t ssp_smem_full(int N) { return sizeof(float) * ((size_t)N * (D_IN + H_VIS1 + H_Z + H_FC) + 2 * (size_t)N * N); }
+
 constexpr int K_TXT = 320, K_Z = 320;      // K of the text layer (300) and of W_fc_pos (260) padded to whole 64-element k-blocks
 
 // input rows -> operand twins of the two first-layer GEMMs: txt = columns [0, 300) (the pad columns stay zero), vis = [300, 2348)
@@ -193,6 +196,7 @@ struct SspCtx {
   float* w[10];
   size_t n[10];
   bool attr_set = false;
+  size_t smem_cap = 0;      // dynamic shared memory k_sinkhorn may use on this device (opt-in maximum less its static part)
   // batched GEMM path: padded fp32 copies of the two weights whose K is not a whole number of k-blocks, operand twins of the
   // four MLP weights, and a workspace for cap_rows input rows
   bool use_tc = true;
@@ -270,10 +274,19 @@ int vsr_ssp_create(const float* const* weights, int32_t N, int32_t n_iters, floa
   VSR_REQUIRE(n_iters >= 0 && tau > 0.f, VSR_EINVAL, "vsr_ssp_create: bad n_iters / tau");
   int ndev = 0;
   VSR_REQUIRE(cudaGetDeviceCount(&ndev) == cudaSuccess && ndev > 0, VSR_ECUDA, "vsr_ssp_create: no CUDA device (no CPU fallback)");
+  // the one-CTA kernel serves a few problems and VSRDEC_GEMM=simt: every N accepted here must fit its shared memory
+  int dev = 0, optin = 0;
+  cudaFuncAttributes fa{};
+  VSR_CHECK_CUDA(cudaGetDevice(&dev));
+  VSR_CHECK_CUDA(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+  VSR_CHECK_CUDA(cudaFuncGetAttributes(&fa, vsr::k_sinkhorn));
+  const size_t smem_cap = (size_t)optin - fa.sharedSizeBytes;
+  VSR_REQUIRE(vsr::ssp_smem_full(N) <= smem_cap, VSR_EINVAL, "vsr_ssp_create: N=%d needs %zu B of shared memory, the device allows %zu",
+              N, vsr::ssp_smem_full(N), smem_cap);
   SspCtx* c = new SspCtx();
   c->N = N; c->n_iters = n_iters; c->tau = tau;
+  c->device = dev; c->smem_cap = smem_cap;
   if (const char* e = getenv("VSRDEC_GEMM")) c->use_tc = strcmp(e, "simt") != 0;
-  VSR_CHECK_CUDA(cudaGetDevice(&c->device));
   for (int i = 0; i < 10; ++i) {
     c->n[i] = i == 8 ? (size_t)N * vsr::H_FC : i == 9 ? (size_t)N : kSspShape[i];
     c->w[i] = nullptr;
@@ -315,12 +328,10 @@ int vsr_ssp_forward(vsr_ssp_handle h, const float* seq, int32_t B, float* matrix
   cudaGetDevice(&prev);
   if (prev != c->device) cudaSetDevice(c->device);
   const int N = c->N;
-  const size_t smem = sizeof(float) * ((size_t)N * (vsr::D_IN + vsr::H_VIS1 + vsr::H_Z + vsr::H_FC) + 2 * (size_t)N * N);
   if (!c->attr_set) {
-    VSR_CHECK_CUDA(cudaFuncSetAttribute(vsr::k_sinkhorn, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    VSR_CHECK_CUDA(cudaFuncSetAttribute(vsr::k_sinkhorn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c->smem_cap));
     c->attr_set = true;
   }
-  VSR_REQUIRE(smem <= 200 * 1024, VSR_EINVAL, "vsr_ssp_forward: N=%d rows do not fit shared memory", N);
   vsr::SspWeights W{c->w[0], c->w[1], c->w[2], c->w[3], c->w[4], c->w[5], c->w[6], c->w[7], c->w[8], c->w[9]};
   cudaStream_t st = (cudaStream_t)stream;
   if (c->use_tc && B >= 8) {
@@ -346,6 +357,8 @@ int vsr_ssp_forward(vsr_ssp_handle h, const float* seq, int32_t B, float* matrix
     const size_t smem_tail = sizeof(float) * ((size_t)N * H_FC + 2 * (size_t)N * N);
     k_sinkhorn<<<B, SSP_THREADS, smem_tail, st>>>(W, seq, c->f, N, c->n_iters, c->tau, matrix, assign);
   } else {
+    const size_t smem = vsr::ssp_smem_full(N);
+    VSR_REQUIRE(smem <= c->smem_cap, VSR_EINVAL, "vsr_ssp_forward: N=%d rows do not fit shared memory", N);
     vsr::k_sinkhorn<<<B, vsr::SSP_THREADS, smem, st>>>(W, seq, nullptr, N, c->n_iters, c->tau, matrix, assign);
   }
   const cudaError_t e = cudaGetLastError();

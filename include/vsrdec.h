@@ -282,6 +282,37 @@ int vsr_get_attention(vsr_handle h, float* alpha, int32_t* slot, void* stream);
  * words (two of them for beam search), allocated at the first decode that needs it. */
 int vsr_set_no_repeat_ngram(vsr_handle h, int32_t n);
 
+/* Diverse beam search (Vijayakumar et al., AAAI 2018): a handle setting (like vsr_set_no_repeat_ngram) that applies to
+ * vsr_beam_search only (greedy, sampling, teacher forcing and vsr_step have no beams to group).  groups = 1 is off (the
+ * default): outputs, launches and graph keys are exactly those of a handle that never set it, whatever the penalty.
+ * With G = groups > 1, beam k, B = k / G beams per group and lambda = penalty, at step t for each caption:
+ *   1. Group g owns beam slots [g*B, (g+1)*B) at every step.  At t = 0 every group expands the single BOS row (all 2k
+ *      candidates); at t > 0 its candidates are the (parent j, word, gate) triples of its own slots j.  Candidate scores
+ *      sc are the ones of the plain search: fl(seq + fl(word + gate)) for a live beam; for a beam frozen by the
+ *      double-EOS path its old score at word 0 and -999 elsewhere.
+ *   2. Groups choose in order g = 0, 1, ..., G-1.
+ *   3. cnt_g(w) = the number of picks that groups 0 .. g-1 made AT THIS STEP whose word is w and whose parent is live
+ *      (not frozen).  Picks of verb-forced rows count: they emit a real word.
+ *   4. key = __fsub_rn(sc, __fmul_rn(lambda, (float)cnt_g(w))) for a candidate of a live row that is not verb-forced;
+ *      key = sc otherwise (forced words and frozen beams' synthetic candidates are never penalised).
+ *   5. Group g takes the B candidates with the largest key, ties by flat index ascending as always, in that order into
+ *      its slots.  Two groups may take the same candidate at t = 0.
+ *   6. The beam's accumulated score is sc, the model's own score, not key: the penalty steers the selection and is
+ *      never accumulated.
+ *   7. lp_words / lp_gates, the vsr_get_history scores and the traced rows (VsrTrace.step_out) stay the model's.
+ *   8. The final ranking is the plain one: all k final beams sorted by score, the top out_size returned (out_size =
+ *      beam_size returns every group's beams).
+ * lambda = 0 with G > 1 is allowed: the groups are then independent searches of beam B (bit-identical to a plain
+ * search of beam B except where two words of one row round to the same score: a group, which holds the row's top-k
+ * words, then takes the lower word index by the tie rule).  A trace with forced selections
+ * (VsrTrace.forced_*) replays them as always.  N-gram blocking composes (the candidates already exclude banned words);
+ * attention capture is unchanged; each caption decodes to the same bits alone, stacked or sharded.
+ * A penalty larger than the gap between a live score and -999 can rank a frozen beam's -999 synthetic candidates above
+ * penalised live ones: the rule is still followed, those beams simply sort last.
+ * Limits (VSR_EINVAL, nothing enqueued): 1 <= groups <= VSR_MAX_BEAM, penalty finite and >= 0; vsr_beam_search refuses
+ * a beam_size that is not a multiple of groups. */
+int vsr_set_beam_diversity(vsr_handle h, int32_t groups, float penalty);
+
 /* Number of kernels this handle has launched so far (bench.py's gpu_launches). */
 int64_t vsr_launch_count(vsr_handle h);
 

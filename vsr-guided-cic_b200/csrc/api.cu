@@ -548,6 +548,7 @@ static int beam_steps_graphed(Ctx* c, int k, const int64_t* eos, int use_verbs, 
   key.eos0 = eos[0]; key.eos1 = eos[1];
   key.k = k; key.use_verbs = use_verbs; key.gt = gt; key.T = c->d.seq_len; key.attn = c->attn_capture;
   key.ngram = c->ngram;
+  if (c->beam_groups > 1) { key.beam_groups = c->beam_groups; memcpy(&key.beam_penalty, &c->beam_penalty, 4); }
   return run_graphed(c, key, st, [&](cudaStream_t s) { return enqueue_beam_steps(c, k, eos, use_verbs, gt, nullptr, s); });
 }
 
@@ -566,6 +567,8 @@ static int beam_search_impl(Ctx* c, int k, int out_size, const int64_t* eos, int
   const int b = c->b, T = c->d.seq_len;
   VSR_REQUIRE(c->ngram == 0 || c->V >= k + T - 1, VSR_EINVAL, "vsr_beam_search: n-gram blocking needs vocab_size (%d) >= "
               "beam + seq_len - 1 (%d), so that every row keeps beam words that are not banned", c->V, k + T - 1);
+  VSR_REQUIRE(k % c->beam_groups == 0, VSR_EINVAL, "vsr_beam_search: beam_size=%d is not a multiple of the %d beam groups "
+              "(vsr_set_beam_diversity)", k, c->beam_groups);
   VSR_TRY(ensure_rows(c, b * k));
   if (c->ngram > 0) VSR_TRY(ensure_whist(c, b * k));
   VSR_TRY(ensure_beam_ws(c, b, T));
@@ -870,6 +873,17 @@ int vsr_set_no_repeat_ngram(vsr_handle h, int32_t n) {
   VSR_REQUIRE(n >= 0 && n <= c->d.seq_len, VSR_EINVAL, "vsr_set_no_repeat_ngram: n=%d not in [0, seq_len=%d] (0 = off)", n,
               c->d.seq_len);
   c->ngram = n;
+  return VSR_OK;
+}
+
+int vsr_set_beam_diversity(vsr_handle h, int32_t groups, float penalty) {
+  if (!h) { vsr::set_error("vsr_set_beam_diversity: null handle"); return VSR_EINVAL; }
+  Ctx* c = (Ctx*)h;
+  VSR_REQUIRE(groups >= 1 && groups <= VSR_MAX_BEAM, VSR_EINVAL, "vsr_set_beam_diversity: groups=%d not in [1, %d] (1 = off)",
+              groups, VSR_MAX_BEAM);
+  VSR_REQUIRE(isfinite(penalty) && penalty >= 0.f, VSR_EINVAL, "vsr_set_beam_diversity: penalty=%g is not finite and >= 0",
+              (double)penalty);
+  c->beam_groups = groups; c->beam_penalty = penalty;
   return VSR_OK;
 }
 

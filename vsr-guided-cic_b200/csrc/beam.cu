@@ -38,6 +38,7 @@ struct BeamArgs {
   int32_t *hist_parent, *hist_word, *hist_gate;    // [T][b][k] slices for step t
   float *hist_score, *hist_lpw, *hist_lpg;
   const int32_t *f_beam, *f_word, *f_gate;        // forced selections for step t or null
+  int groups; float penalty;                       // diverse beam search (k_beam_step<true> only): G > 1 groups, lambda
 };
 
 constexpr int MAXC = 2 * VSR_MAX_BEAM * VSR_MAX_BEAM;  // 128 candidates per caption
@@ -47,7 +48,12 @@ struct BeamSmem {
   int full[VSR_MAX_BEAM], pb[VSR_MAX_BEAM], pw[VSR_MAX_BEAM], pg[VSR_MAX_BEAM];
 };
 
-// selection for caption c by one warp; leaves the picks (parent, word, gate) in sh.pb / pw / pg
+// selection for caption c by one warp; leaves the picks (parent, word, gate) in sh.pb / pw / pg.
+// DIVERSE (vsr_set_beam_diversity, G = a.groups > 1): groups g = 0 .. G-1 in turn fill slots [g*B, (g+1)*B), B = k / G,
+// from the candidates of their own parents (all of them at t = 0), by key = sc - lambda * (number of earlier groups'
+// picks of this step with the same word and a live parent); forced rows and frozen beams are not penalised.  The
+// stored score stays sc.  The top-k word candidates per row are enough for every group (DESIGN.md §2).
+template <bool DIVERSE>
 __device__ __forceinline__ void beam_select_warp(const BeamArgs& a, BeamSmem& sh, int c, int lane, bool write) {
   const int k = a.k, cur = a.cur;
   float* s_seq = sh.seq; float* s_m0 = sh.m0; float* s_m1 = sh.m1; float* s_ps = sh.ps;
@@ -69,11 +75,13 @@ __device__ __forceinline__ void beam_select_warp(const BeamArgs& a, BeamSmem& sh
   if (a.f_beam == nullptr) {
     // candidates: idx = (parent j, i-th word candidate, gate g); lane owns idx = lane + 32*q
     float cs[MAXC / 32]; int cf[MAXC / 32]; bool used[MAXC / 32];
+    bool pen[MAXC / 32];                                  // DIVERSE: a live, unforced row's candidate (penalised)
     const int ncand = cur * k * 2;
 #pragma unroll
     for (int q = 0; q < MAXC / 32; ++q) {
       const int idx = lane + 32 * q;
       cs[q] = -INFINITY; cf[q] = 0x7fffffff; used[q] = true;
+      if constexpr (DIVERSE) pen[q] = false;
       if (idx < ncand) {
         const int j = idx / (2 * k), i = (idx >> 1) % k, g = idx & 1;
         const int row = c * cur + j;
@@ -82,6 +90,7 @@ __device__ __forceinline__ void beam_select_warp(const BeamArgs& a, BeamSmem& sh
           word = a.cand[row * VSR_MAX_BEAM + i];
           const float wl = row_logp(a.logits, a.ld, a.row_max, a.row_lsum, a.forced, row, word);
           sc = __fadd_rn(s_seq[j], __fadd_rn(wl, a.gate_lp[row * 2 + g]));   // seq + (word + gate), :139
+          if constexpr (DIVERSE) pen[q] = a.forced[row] < 0;
         } else {
           // frozen beam: old score at word 0 (both gates), -999 elsewhere (:146-150)
           word = i;
@@ -90,25 +99,61 @@ __device__ __forceinline__ void beam_select_warp(const BeamArgs& a, BeamSmem& sh
         cs[q] = sc; cf[q] = j * 2 * a.V + word * 2 + g; used[q] = false;
       }
     }
-    for (int sel = 0; sel < k; ++sel) {
-      float bv = -INFINITY; int bf = 0x7fffffff;
+    if constexpr (DIVERSE) {
+      const int B = k / a.groups;
+      for (int grp = 0; grp < a.groups; ++grp) {
+        float key[MAXC / 32];
 #pragma unroll
-      for (int q = 0; q < MAXC / 32; ++q)
-        if (!used[q] && before(cs[q], cf[q], bv, bf)) { bv = cs[q]; bf = cf[q]; }
-      {   // warp arg-best in (score desc, flat index asc) order: two redux.sync + one broadcast
-        const unsigned u = __float_as_uint(bv);
-        const unsigned key = (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-        const unsigned kbest = __reduce_max_sync(0xffffffffu, key);
-        const int fbest = (int)__reduce_min_sync(0xffffffffu, key == kbest ? (unsigned)bf : 0xffffffffu);
-        const unsigned owner = __ballot_sync(0xffffffffu, key == kbest && bf == fbest);
-        bv = __shfl_sync(0xffffffffu, bv, __ffs(owner) - 1);
-        bf = fbest;
+        for (int q = 0; q < MAXC / 32; ++q) {
+          const int idx = lane + 32 * q, j = idx / (2 * k);
+          used[q] = !(idx < ncand && (a.t == 0 || j / B == grp));      // own parents only; fresh flags per group
+          key[q] = cs[q];
+          if (!used[q] && pen[q]) {
+            const int w = (cf[q] - j * 2 * a.V) >> 1;
+            int cnt = 0;
+            for (int s = 0; s < grp * B; ++s) cnt += (s_pw[s] == w && s_full[s_pb[s]]) ? 1 : 0;
+            key[q] = __fsub_rn(cs[q], __fmul_rn(a.penalty, (float)cnt));
+          }
+        }
+        for (int sel = grp * B; sel < (grp + 1) * B; ++sel) {
+          float bv = -INFINITY, bs = -INFINITY; int bf = 0x7fffffff;
+#pragma unroll
+          for (int q = 0; q < MAXC / 32; ++q)
+            if (!used[q] && before(key[q], cf[q], bv, bf)) { bv = key[q]; bf = cf[q]; bs = cs[q]; }
+          unsigned kbest; int fbest;
+          warp_argbest_redux(bv, bf, kbest, fbest);
+          const unsigned owner = __ballot_sync(0xffffffffu, orderable(bv) == kbest && bf == fbest);
+          bs = __shfl_sync(0xffffffffu, bs, __ffs(owner) - 1);     // the model's score of the pick, not its key
+#pragma unroll
+          for (int q = 0; q < MAXC / 32; ++q) if (cf[q] == fbest) used[q] = true;
+          if (lane == 0) {
+            const int j = fbest / (2 * a.V), rem = fbest - j * 2 * a.V;
+            s_pb[sel] = j; s_pw[sel] = rem >> 1; s_pg[sel] = rem & 1; s_ps[sel] = bs;
+          }
+        }
+        __syncwarp();                                                  // the next group counts these picks
       }
+    } else {
+      for (int sel = 0; sel < k; ++sel) {
+        float bv = -INFINITY; int bf = 0x7fffffff;
 #pragma unroll
-      for (int q = 0; q < MAXC / 32; ++q) if (cf[q] == bf) used[q] = true;
-      if (lane == 0) {
-        const int j = bf / (2 * a.V), rem = bf - j * 2 * a.V;
-        s_pb[sel] = j; s_pw[sel] = rem >> 1; s_pg[sel] = rem & 1; s_ps[sel] = bv;
+        for (int q = 0; q < MAXC / 32; ++q)
+          if (!used[q] && before(cs[q], cf[q], bv, bf)) { bv = cs[q]; bf = cf[q]; }
+        {   // warp arg-best in (score desc, flat index asc) order: two redux.sync + one broadcast
+          const unsigned u = __float_as_uint(bv);
+          const unsigned key = (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+          const unsigned kbest = __reduce_max_sync(0xffffffffu, key);
+          const int fbest = (int)__reduce_min_sync(0xffffffffu, key == kbest ? (unsigned)bf : 0xffffffffu);
+          const unsigned owner = __ballot_sync(0xffffffffu, key == kbest && bf == fbest);
+          bv = __shfl_sync(0xffffffffu, bv, __ffs(owner) - 1);
+          bf = fbest;
+        }
+#pragma unroll
+        for (int q = 0; q < MAXC / 32; ++q) if (cf[q] == bf) used[q] = true;
+        if (lane == 0) {
+          const int j = bf / (2 * a.V), rem = bf - j * 2 * a.V;
+          s_pb[sel] = j; s_pw[sel] = rem >> 1; s_pg[sel] = rem & 1; s_ps[sel] = bv;
+        }
       }
     }
   } else if (lane < k) {
@@ -210,12 +255,14 @@ __global__ void __launch_bounds__(256) k_advance(const AdvanceArgs a) {
 // beam selection fused with the reorder of the beam states.  Grid (captions, k): every CTA of a caption
 // repeats the (cheap, deterministic) selection with its warp 0 — only CTA y = 0 records it — and then
 // moves ONE new beam row, so the copy keeps captions x k CTAs of parallelism without a second launch.
+// DIVERSE: the grouped selection of diverse beam search (only launched with groups > 1).
+template <bool DIVERSE>
 __global__ void __launch_bounds__(256) k_beam_step(const BeamArgs b, const AdvanceArgs a, int do_advance) {
   __shared__ BeamSmem sh;
   const int c = blockIdx.x, i = blockIdx.y;
   pdl_trigger();
   pdl_wait();
-  if (threadIdx.x < 32) beam_select_warp(b, sh, c, threadIdx.x, i == 0);
+  if (threadIdx.x < 32) beam_select_warp<DIVERSE>(b, sh, c, threadIdx.x, i == 0);
   __syncthreads();
   if (!do_advance) return;
   advance_row(a, c * b.k + i, c * b.cur + sh.pb[i], (int64_t)sh.pw[i], sh.pg[i]);
@@ -665,7 +712,12 @@ int launch_beam_step(Ctx* c, int t, int b, int cur, int k, int64_t eos0, int64_t
   ad.rows_new = b * k; ad.cur = cur; ad.k = k; ad.fixed_slot = -1;
   fill_advance(c, ad);
   if (c->ngram > 0) { ad.whist = c->whist; ad.whist_n = c->whist_n; ad.whist_ld = c->d.seq_len; ad.hist_t = t; }
-  k_beam_step<<<dim3(b, advance ? k : 1), 256, 0, st>>>(a, ad, advance ? 1 : 0);
+  if (c->beam_groups > 1) {
+    a.groups = c->beam_groups; a.penalty = c->beam_penalty;
+    k_beam_step<true><<<dim3(b, advance ? k : 1), 256, 0, st>>>(a, ad, advance ? 1 : 0);
+  } else {
+    k_beam_step<false><<<dim3(b, advance ? k : 1), 256, 0, st>>>(a, ad, advance ? 1 : 0);
+  }
   VSR_CHECK_CUDA(cudaGetLastError()); c->launches++;
   std::swap(c->sel_beam, c->sel_beam_n);
   std::swap(c->sel_word, c->sel_word_n);

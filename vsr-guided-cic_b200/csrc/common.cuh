@@ -368,6 +368,9 @@ struct Ctx {
   int ngram = 0;
   int32_t *whist = nullptr, *whist_n = nullptr;
   int cap_whist = 0;
+  // diverse beam search (vsr_set_beam_diversity): beam groups (1 = off) and the Hamming diversity penalty lambda
+  int beam_groups = 1;
+  float beam_penalty = 0.f;
   // attention capture (vsr_set_attention_capture): per step t, rows t * attn_step_rows .. of [R+1] weights and the
   // slot each row read; attn_path = the back-tracked rows of the returned beams [b][out_size][T]
   bool attn_capture = false;
@@ -393,6 +396,7 @@ struct Ctx {
     const void *det, *det_seqs, *slot_index, *verbs;
     int64_t det_stride, eos0, eos1;
     int32_t b, D, L, R, n_img, verbs_dtype, k, use_verbs, gt, T, attn, feat_dtype, ngram;
+    int32_t beam_groups; uint32_t beam_penalty;   // 0 unless groups > 1; the penalty by its bits
   };
   struct GraphEntry { GraphKey key; cudaGraphExec_t exec; int64_t launches; uint64_t last_use; };
   std::vector<GraphEntry> graphs;

@@ -24,6 +24,14 @@ banned, greedy takes the best of them, sampling drops banned words before temper
 log-probs stay the model's own; verb-forced words are never blocked.  0 = off, bit-identical to a call without the
 keyword.  The semantics and limits (n <= seq_len; vocab_size >= beam_size + seq_len - 1, or >= seq_len for greedy and
 sampling) are spelled out in include/vsrdec.h, vsr_set_no_repeat_ngram.
+
+The beam-search drivers (`beam_search`, `beam_search_v`, `beam_search_v_indexed`) take `num_beam_groups=1,
+diversity_penalty=0.0`: diverse beam search (Vijayakumar et al., AAAI 2018).  With G = num_beam_groups > 1 the beam is
+split into G groups of beam_size / G beams that choose in turn at every step; a group's candidate loses
+diversity_penalty per pick of the same word by an earlier group at that step.  The penalty only steers the selection:
+the beam scores and log-probs stay the model's, and the final ranking is over all beams (out_size = beam_size returns
+every group's).  1 = off, bit-identical to a call without the keywords.  Semantics and limits (G in [1, 8] dividing
+beam_size, a finite penalty >= 0): include/vsrdec.h, vsr_set_beam_diversity.
 """
 import torch
 from torch import nn
@@ -53,13 +61,22 @@ class CaptioningModel(nn.Module):
         check_no_repeat_ngram(no_repeat_ngram_size, self.seq_len, self.vocab_size, beam_size)
 
     @staticmethod
-    def _run(eng, decode, return_attention, no_repeat_ngram_size=0):
+    def _check_diversity(num_beam_groups, diversity_penalty, beam_size):
+        """VsrError unless the diverse beam search setting is valid for a beam search of beam_size."""
+        from vsrdec.engine import check_beam_diversity
+        check_beam_diversity(num_beam_groups, diversity_penalty, beam_size)
+
+    @staticmethod
+    def _run(eng, decode, return_attention, no_repeat_ngram_size=0, diversity=(1, 0.0)):
         """decode() alone, or with the engine's attention capture on around it: (result, attention dict or None).  The
-        engine's n-gram blocking is no_repeat_ngram_size for the duration of the call and restored afterwards."""
-        prev = eng.no_repeat_ngram
+        engine's n-gram blocking is no_repeat_ngram_size and its beam diversity (groups, penalty) is `diversity` for the
+        duration of the call; both are restored afterwards."""
+        prev, prev_div = eng.no_repeat_ngram, eng.beam_diversity
         if no_repeat_ngram_size != prev:
             eng.set_no_repeat_ngram(no_repeat_ngram_size)
         try:
+            if tuple(diversity) != prev_div:
+                eng.set_beam_diversity(*diversity)
             if not return_attention:
                 return decode(), None
             eng.set_attention_capture(True)
@@ -72,6 +89,8 @@ class CaptioningModel(nn.Module):
         finally:
             if eng.no_repeat_ngram != prev:
                 eng.set_no_repeat_ngram(prev)
+            if eng.beam_diversity != prev_div:
+                eng.set_beam_diversity(*prev_div)
 
     # ---- drivers
     def forward(self, statics, seqs, *args, return_attention=False):
@@ -149,10 +168,10 @@ class CaptioningModel(nn.Module):
         return out.reshape((b_s * beam_size,) + tail) if reduced else out
 
     def _beam_run(self, eng, eos_idxs, beam_size, out_size, use_verbs, gt, return_attention, slot_index=None,
-                  no_repeat_ngram_size=0):
+                  no_repeat_ngram_size=0, diversity=(1, 0.0)):
         def decode():
             return eng.beam_search(beam_size, out_size, eos_idxs, use_verbs=use_verbs, gt=gt)
-        ((words, gates), (lpw, lpg), _), att = self._run(eng, decode, return_attention, no_repeat_ngram_size)
+        ((words, gates), (lpw, lpg), _), att = self._run(eng, decode, return_attention, no_repeat_ngram_size, diversity)
         outputs, log_probs = [words, gates], [lpw, lpg]
         if att is not None and slot_index is not None:      # detection row of every region of the slot read
             b, R = slot_index.size(0), slot_index.size(2)
@@ -165,37 +184,47 @@ class CaptioningModel(nn.Module):
                 att = {k: v.squeeze(1) for k, v in att.items()}
         return (outputs, log_probs) if att is None else (outputs, log_probs, att)
 
-    def _beam(self, statics, eos_idxs, beam_size, out_size, use_verbs, gt, return_attention=False, no_repeat_ngram_size=0):
+    def _beam(self, statics, eos_idxs, beam_size, out_size, use_verbs, gt, return_attention=False, no_repeat_ngram_size=0,
+              num_beam_groups=1, diversity_penalty=0.0):
         self._check_ngram(no_repeat_ngram_size, beam_size)
+        self._check_diversity(num_beam_groups, diversity_penalty, beam_size)
         eng = self._engine_for(statics)
         return self._beam_run(eng, eos_idxs, beam_size, out_size, use_verbs, gt, return_attention,
-                              no_repeat_ngram_size=no_repeat_ngram_size)
+                              no_repeat_ngram_size=no_repeat_ngram_size, diversity=(num_beam_groups, diversity_penalty))
 
     def beam_search_v_indexed(self, statics, eos_idxs, beam_size, out_size=1, *args, gt=False, return_attention=False,
-                              no_repeat_ngram_size=0):
+                              no_repeat_ngram_size=0, num_beam_groups=1, diversity_penalty=0.0):
         """Extension (SURVEY §8 f3): beam_search_v with the slots given as INDICES into the detections instead
         of materialised feature tiles: statics = (detections (b,D,F), slot_index (b,L,R) int, verbs (b,L) or None);
         slot_index >= 0 picks a detection row, -2 the mean of the image's valid detections, -1 is padding.
         Same return structure as beam_search_v; 10x fewer input bytes.  With return_attention the attention dict also
         holds det_index (..., R) int64 = slot_index[caption, slot, :]: the detection row each alpha[..., 1:] column
-        weighs (-2 the image's mean row, -1 padding).  no_repeat_ngram_size as in beam_search."""
+        weighs (-2 the image's mean row, -1 padding).  no_repeat_ngram_size, num_beam_groups and diversity_penalty as in
+        beam_search."""
         self._check_ngram(no_repeat_ngram_size, beam_size)
+        self._check_diversity(num_beam_groups, diversity_penalty, beam_size)
         eng = self._engine()
         verbs = statics[2] if len(statics) > 2 else None
         eng.prologue_indexed(statics[0], statics[1], verbs)
         self._prologue_key = None
         return self._beam_run(eng, eos_idxs, beam_size, out_size, verbs is not None, gt, return_attention,
-                              slot_index=statics[1], no_repeat_ngram_size=no_repeat_ngram_size)
+                              slot_index=statics[1], no_repeat_ngram_size=no_repeat_ngram_size,
+                              diversity=(num_beam_groups, diversity_penalty))
 
-    def beam_search(self, statics, eos_idxs, beam_size, out_size=1, *args, return_attention=False, no_repeat_ngram_size=0):
+    def beam_search(self, statics, eos_idxs, beam_size, out_size=1, *args, return_attention=False, no_repeat_ngram_size=0,
+                    num_beam_groups=1, diversity_penalty=0.0):
         """Joint (word, gate) beam search (reference CaptioningModel.py:116-195).  beam_size <= 8, out_size <= beam_size,
         <= 64 regions per slot (see the limits in models/controllable_captioning.py).  With no_repeat_ngram_size = n >= 1
-        no beam picks a word that would repeat an n-gram of its own word path (the scores stay the model's)."""
-        return self._beam(statics[:2], eos_idxs, beam_size, out_size, False, False, return_attention, no_repeat_ngram_size)
+        no beam picks a word that would repeat an n-gram of its own word path (the scores stay the model's).  With
+        num_beam_groups = G > 1 the search is a diverse beam search of G groups, diversity_penalty per earlier group's
+        pick of the same word (see the module docstring)."""
+        return self._beam(statics[:2], eos_idxs, beam_size, out_size, False, False, return_attention, no_repeat_ngram_size,
+                          num_beam_groups, diversity_penalty)
 
     def beam_search_v(self, statics, eos_idxs, beam_size, out_size=1, *args, gt=False, return_attention=False,
-                      no_repeat_ngram_size=0):
+                      no_repeat_ngram_size=0, num_beam_groups=1, diversity_penalty=0.0):
         """Beam search with verb forcing (reference CaptioningModel.py:197-294).  beam_size <= 8, out_size <= beam_size,
-        <= 64 regions per slot (see the limits in models/controllable_captioning.py).  no_repeat_ngram_size as in
-        beam_search; a verb-forced word is never blocked."""
-        return self._beam(statics, eos_idxs, beam_size, out_size, True, gt, return_attention, no_repeat_ngram_size)
+        <= 64 regions per slot (see the limits in models/controllable_captioning.py).  no_repeat_ngram_size,
+        num_beam_groups and diversity_penalty as in beam_search; a verb-forced word is never blocked or penalised."""
+        return self._beam(statics, eos_idxs, beam_size, out_size, True, gt, return_attention, no_repeat_ngram_size,
+                          num_beam_groups, diversity_penalty)

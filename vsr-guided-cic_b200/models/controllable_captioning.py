@@ -26,6 +26,8 @@ LIMITS the reference does not have (each raises VsrError with a message, never a
     any other dtype raises); half precision is refused under VSRDEC_GEMM=simt (the fp32 FFMA verification twin).
   * no-repeat n-gram blocking (`no_repeat_ngram_size` of every word-choosing driver): an int in [0, seq_len]; when on,
     vocab_size >= beam_size + seq_len - 1 (beam search) or >= seq_len (greedy, sampling);
+  * diverse beam search (`num_beam_groups`, `diversity_penalty` of the beam-search drivers): groups an int in [1, 8]
+    that divides beam_size, the penalty a finite float32 >= 0;
   * sampling (`sample_rl`, `sample_v`): captions x n draws <= 2^30 rows per call; temperature a finite float32 > 0 and
     top_p in (0, 1] as float32 values (where logits / temperature overflows float32 it is clamped to +-FLT_MAX: the
     overflowing words tie and the lowest index among them wins).

@@ -58,6 +58,7 @@ EXPORTED_SYMBOLS = {
     "vsr_set_attention_capture": (ctypes.c_int, [c_vp, c_i32]),
     "vsr_get_attention": (ctypes.c_int, [c_vp, c_vp, c_vp, c_vp]),
     "vsr_set_no_repeat_ngram": (ctypes.c_int, [c_vp, c_i32]),
+    "vsr_set_beam_diversity": (ctypes.c_int, [c_vp, c_i32, c_f]),
     "vsr_launch_count": (c_i64, [c_vp]),
     "vsr_gemm_kind": (ctypes.c_char_p, [c_vp]),
     "vsr_set_profiling": (ctypes.c_int, [c_vp, c_i32]),

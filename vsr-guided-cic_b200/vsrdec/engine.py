@@ -78,6 +78,24 @@ def check_no_repeat_ngram(n, seq_len, vocab_size=None, beam_size=1):
                        f"got {vocab_size}")
 
 
+MAX_BEAM = 8                    # VSR_MAX_BEAM
+
+
+def check_beam_diversity(groups, penalty, beam_size=None):
+    """Raise VsrError unless (groups, penalty) is a valid diverse beam search setting (vsr_set_beam_diversity): groups an
+    int in [1, 8] (1 = off), penalty a real number, finite and >= 0 as a float32.  With beam_size, also for a beam search
+    of that size: beam_size must be a multiple of groups."""
+    if isinstance(groups, bool) or not isinstance(groups, numbers.Integral) or not 1 <= groups <= MAX_BEAM:
+        raise VsrError(f"num_beam_groups must be an int in [1, {MAX_BEAM}] (1 = off), got {groups!r}")
+    if isinstance(penalty, bool) or not isinstance(penalty, numbers.Real):
+        raise VsrError(f"diversity_penalty must be a real number >= 0, got {penalty!r}")
+    p32 = c_f(float(penalty)).value
+    if not math.isfinite(p32) or not p32 >= 0.0:
+        raise VsrError(f"diversity_penalty must be finite and >= 0 in float32, got {penalty!r}")
+    if beam_size is not None and beam_size % groups != 0:
+        raise VsrError(f"beam_size={beam_size} is not a multiple of num_beam_groups={groups}")
+
+
 def _req_cuda(t: torch.Tensor, name: str, dtype=None):
     if not isinstance(t, torch.Tensor) or not t.is_cuda:
         raise VsrError(f"{name} must be a CUDA tensor (no CPU fallback on this path)")
@@ -95,6 +113,7 @@ class DecoderEngine:
         self._weights = None
         self._attn_shape = None
         self.no_repeat_ngram = 0
+        self.beam_diversity = (1, 0.0)
         self.handle = c_vp()
         d = VsrDims(*(int(self.dims[k]) for k in ("seq_len", "vocab_size", "bos_idx", "det_feat_size",
                                                    "input_encoding_size", "rnn_size", "att_size",
@@ -367,6 +386,15 @@ class DecoderEngine:
         check_no_repeat_ngram(n, self.dims["seq_len"])
         _lib.check(self.lib, self.lib.vsr_set_no_repeat_ngram(self.handle, int(n)))
         self.no_repeat_ngram = int(n)
+
+    # ------------------------------------------------------------------ diverse beam search
+    def set_beam_diversity(self, groups: int, penalty: float):
+        """Split the following beam searches into `groups` groups of beam_size / groups beams, each penalised by
+        `penalty` per earlier group's pick of the same word at the step (vsr_set_beam_diversity); groups = 1 is off,
+        the default.  The beam scores stay the model's."""
+        check_beam_diversity(groups, penalty)
+        _lib.check(self.lib, self.lib.vsr_set_beam_diversity(self.handle, int(groups), float(penalty)))
+        self.beam_diversity = (int(groups), float(penalty))
 
     # ------------------------------------------------------------------ instrumentation
     def launch_count(self) -> int:

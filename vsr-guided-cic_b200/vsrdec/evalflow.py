@@ -20,10 +20,13 @@ from .preorder import RoleOrderer, permute_slot_index
 
 class EvalFlow:
     def __init__(self, model, orderer: RoleOrderer, eos_idxs, beam_size: int = 5, out_size: int = 1, gt: bool = True,
-                 overlap: bool = True, no_repeat_ngram_size: int = 0):
-        """no_repeat_ngram_size: n-gram blocking of every decode (see CaptioningModel.beam_search; 0 = off)."""
+                 overlap: bool = True, no_repeat_ngram_size: int = 0, num_beam_groups: int = 1,
+                 diversity_penalty: float = 0.0):
+        """no_repeat_ngram_size: n-gram blocking of every decode (see CaptioningModel.beam_search; 0 = off).
+        num_beam_groups, diversity_penalty: diverse beam search of every decode (see beam_search; 1 group = off)."""
         self.model, self.orderer = model, orderer
         self.no_repeat_ngram_size = no_repeat_ngram_size
+        self.num_beam_groups, self.diversity_penalty = num_beam_groups, diversity_penalty
         self.eos_idxs, self.beam_size, self.out_size, self.gt = eos_idxs, beam_size, out_size, gt
         self.overlap = bool(overlap)
         self._side = None
@@ -38,7 +41,9 @@ class EvalFlow:
         dev = b["slot_index"].device
         statics = (b["detections"], permute_slot_index(b["slot_index"], src), verbs.to(dev).double())
         return self.model.beam_search_v_indexed(statics, self.eos_idxs, self.beam_size, self.out_size, gt=self.gt,
-                                                no_repeat_ngram_size=self.no_repeat_ngram_size)
+                                                no_repeat_ngram_size=self.no_repeat_ngram_size,
+                                                num_beam_groups=self.num_beam_groups,
+                                                diversity_penalty=self.diversity_penalty)
 
     def run(self, batches: Iterable[dict]) -> Iterator:
         it = iter(batches)

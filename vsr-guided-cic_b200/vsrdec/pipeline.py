@@ -22,12 +22,14 @@ import torch
 class DecodePipeline:
     def __init__(self, models: Sequence, eos_idxs, beam_size: int, out_size: int = 1, gt: bool = False,
                  indexed: bool = False, buffers: Optional[int] = None, stack: int = 1, ramp: bool = True,
-                 post: Optional[Callable[[torch.Tensor], torch.Tensor]] = None, no_repeat_ngram_size: int = 0):
+                 post: Optional[Callable[[torch.Tensor], torch.Tensor]] = None, no_repeat_ngram_size: int = 0,
+                 num_beam_groups: int = 1, diversity_penalty: float = 0.0):
         """models: one drop-in model per lane (same weights, same device).  `stack` host batches (of equal shapes) are
         decoded per call; with `ramp` the first group of a run holds a single batch, so that the first decode starts after
         one batch's host->device copy instead of `stack` of them (the un-overlapped pipeline fill of a short run).  `post` is
         applied to each batch's words tensor on the lane's stream (e.g. the all-gather of a caption-sharded job).
-        `no_repeat_ngram_size` is passed to every decode (n-gram blocking, see beam_search; 0 = off)."""
+        `no_repeat_ngram_size` is passed to every decode (n-gram blocking, see beam_search; 0 = off), and so are
+        `num_beam_groups` and `diversity_penalty` (diverse beam search, see beam_search; 1 group = off)."""
         if not models:
             raise ValueError("DecodePipeline needs at least one model")
         self.models = list(models)
@@ -37,6 +39,7 @@ class DecodePipeline:
         self.eos_idxs, self.beam_size, self.out_size, self.gt, self.indexed = eos_idxs, beam_size, out_size, gt, indexed
         self.post = post
         self.no_repeat_ngram_size = no_repeat_ngram_size
+        self.num_beam_groups, self.diversity_penalty = num_beam_groups, diversity_penalty
         self.stack = max(1, int(stack))
         self.ramp = bool(ramp)
         self.n_lanes = len(self.models)
@@ -89,7 +92,8 @@ class DecodePipeline:
             fn = model.beam_search_v_indexed if self.indexed else model.beam_search_v
             statics = tuple(t[:n * b] for t in self._bufs[slot])
             (words, gates), (lpw, lpg) = fn(statics, self.eos_idxs, self.beam_size, self.out_size, gt=self.gt,
-                                            no_repeat_ngram_size=self.no_repeat_ngram_size)
+                                            no_repeat_ngram_size=self.no_repeat_ngram_size,
+                                            num_beam_groups=self.num_beam_groups, diversity_penalty=self.diversity_penalty)
             self._freed[slot].record(lane)
             if self.post is not None:
                 words = torch.cat([self.post(words[i * b:(i + 1) * b]) for i in range(n)], 0)

@@ -79,9 +79,12 @@ constexpr int MPAD = 128;   // UMMA M tile
 
 // An fp32 matrix carried as an error-compensated fp16 pair (x = hi + lo + O(2^-22 x)) with the TMA
 // tensor maps (64 x box_rows boxes, 128-byte swizzle) the tcgen05 GEMM loads it through.
-// Activation twins of the f16+f8x2 GEMM mode are stored scaled by ACT_SCALE_F8 (a power of two, exact): their
-// residuals x*s - fp16(x*s) then sit in the normal range of e4m3 for the |x| ~ 1e-2..1 of the decoder's states.
-constexpr float ACT_SCALE_F8 = 256.f;
+// Activation twins of the f16+f8x2 GEMM mode are stored scaled by ACT_SCALE_F8 (a power of two, exact, undone by the
+// GEMM epilogue).  32 keeps |hi| = |32 x| <= 2^13 for |x| <= 256, the supported range of the attended feature vector
+// att (DESIGN.md §4): hi8 = e4m3(hi / 32) saturates only above |x| = 448 and the fp16 hi above 2047.  Residuals of
+// |x| < 1/32 fall into the e4m3 subnormals, so an activation carries an absolute error of at most
+// max(2^-15 |x|, 2^-20): small against the output scale of the GEMMs, whose activations are O(1).
+constexpr float ACT_SCALE_F8 = 32.f;
 
 struct F16Pair {
   void* hi = nullptr;   // __half [rows][ld]

@@ -18,10 +18,6 @@ LIMITS the reference does not have (each raises VsrError with a message, never a
   * <= 64 regions per slot (the slot validity mask is one 64-bit word);
   * det_feat_size % 4 == 0 and att_size % 4 == 0 (128-bit loads); vocab_size <= 49152; vocab_size >= beam_size;
   * seq_len <= 256 for beam search (back-track kernel's shared-memory history);
-  * tensor-core operands are carried as fp16 (+ fp16 / e4m3 residuals): weights are rescaled per tensor by a power of
-    two, activations are not — hidden states are in [-1, 1] by construction, region features must stay below 255 in
-    magnitude in the default "f16+f8x2" GEMM mode (65504 with VSRDEC_GEMM=f16x3); larger values saturate.  The bound is
-    on the activation scale, not the input format: it is the same for float32, float16 and bfloat16 features;
   * region features are float32, float16 or bfloat16, one dtype for the detections and the slot tiles (a mismatch or
     any other dtype raises); half precision is refused under VSRDEC_GEMM=simt (the fp32 FFMA verification twin).
   * no-repeat n-gram blocking (`no_repeat_ngram_size` of every word-choosing driver): an int in [0, seq_len]; when on,
@@ -32,6 +28,14 @@ LIMITS the reference does not have (each raises VsrError with a message, never a
     top_p in (0, 1] as float32 values (where logits / temperature overflows float32 it is clamped to +-FLT_MAX: the
     overflowing words tie and the lowest index among them wins).
 Among candidates whose fp32 scores tie EXACTLY the order is (score desc, flat index asc); torch.sort leaves it unspecified.
+
+A RANGE that is NOT checked (nothing raises; results lose precision silently above it): tensor-core operands are carried
+as fp16 (+ fp16 / e4m3 residuals); weights are rescaled per tensor by a power of two, activations by a constant.  Hidden
+states are in [-1, 1] by construction; the attended features att (the attention-weighted mean of the slot's region
+features and the sentinel s_fc(s_t)) must stay within +-256 in the default "f16+f8x2" GEMM mode, i.e. region features
+and sentinel within +-256 (65504 with VSRDEC_GEMM=f16x3).  Above 448 an e4m3 residual operand saturates (an error up to
+2^-11 of att's share of the LSTM-2 pre-activation), above 2047 the fp16 operand.  The range is on the activation scale,
+not the input format: it is the same for float32, float16 and bfloat16 features.
 """
 import json
 import os
